@@ -21,6 +21,7 @@ only for the barrier and the max-over-ranks of the measured time.
 
 `--impl reference` times that CPU implementation alone (rank 0 only), same metric/config.
 `--config 5` runs BASELINE config 5 (one 24 h stream) on one GPU and prints its own line.
+`--dump-outputs DIR` writes the events of the last timed step (rank 0) as .npy files, see dump_outputs().
 """
 import argparse
 import json
@@ -62,7 +63,14 @@ def parse_args():
     ap.add_argument("--config4-chunk-seconds", type=float, default=5.0)
     ap.add_argument("--kernel", type=int, default=0, help="diagnostic: engine option 'kernel' (0 = measured policy)")
     ap.add_argument("--lanes-per-warp", type=int, default=0, help="diagnostic: engine option 'lanes_per_warp'")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the events the last timed step drained (rank 0) to DIR/*.npy, for comparing two builds")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.config == 5:
+        ap.error("--dump-outputs covers the config-3 step; --config 5 has no step to dump")
+    return args
 
 
 def workload_name(streams, seconds):
@@ -253,6 +261,44 @@ def profiled_traffic(ns, seconds):
     return tj.get("dram_bytes_per_launch"), f"ncu --set full capture of {tj.get('captured', '?')} ({tj.get('report', '')})"
 
 
+DUMP_MAX_BYTES = 64 * 10 ** 6
+
+
+def canonical_events(evs, pay):
+    """One drain's same_event records and payload, with every event's payload bytes laid out in event order and
+    `data_offset` pointing there.  Where a device drain places a payload in its arena depends on which warp wrote
+    first, so only this form is comparable from run to run.  link.Burst (kind 3) payloads are stored up to
+    SAME_BURST_CAP = 1024 bytes; `data_len` keeps the true length."""
+    e = np.array(evs, copy=True)
+    stored = np.where(e["kind"] == 3, np.minimum(e["data_len"], 1024), e["data_len"]).astype(np.int64)
+    start = np.cumsum(stored) - stored
+    idx = np.repeat(e["data_offset"].astype(np.int64) - start, stored) + np.arange(int(stored.sum()))
+    e["data_offset"] = start
+    return e, np.asarray(pay)[idx]
+
+
+def dump_outputs(dirname, evs, pay, n_streams, max_bytes=DUMP_MAX_BYTES):
+    """Write one drain in canonical_events form: DIR/event_<field>.npy for each same_event field (float64: every value
+    is an integer below 2^53) and DIR/payload.npy (the payload bytes, float32), plus DIR/streams.npy, the streams
+    included.  When all streams do not fit in `max_bytes`, the longest prefix that fits of a fixed seeded permutation
+    of the streams is written, in stream order, so the same events always give the same files.  Returns
+    (streams written, events written)."""
+    evs, pay = canonical_events(evs, pay)
+    fields = evs.dtype.names
+    stored = np.diff(np.append(evs["data_offset"].astype(np.int64), pay.size))
+    per_stream = np.bincount(evs["stream"], weights=8 * len(fields) + 4 * stored, minlength=n_streams) + 8
+    order = np.random.default_rng(0x5A3E).permutation(n_streams)
+    budget = max_bytes - 4096 * (len(fields) + 2)                 # room for the .npy headers
+    keep = np.sort(order[:int((np.cumsum(per_stream[order]) <= budget).sum())])
+    evs, pay = canonical_events(evs[np.isin(evs["stream"], keep)], pay)
+    os.makedirs(dirname, exist_ok=True)
+    for f in fields:
+        np.save(os.path.join(dirname, f"event_{f}.npy"), evs[f].astype(np.float64))
+    np.save(os.path.join(dirname, "payload.npy"), pay.astype(np.float32))
+    np.save(os.path.join(dirname, "streams.npy"), keep.astype(np.float64))
+    return int(keep.size), int(evs.size)
+
+
 def main():
     args = parse_args()
     rank = int(os.environ.get("RANK", "0"))
@@ -337,10 +383,10 @@ def main():
         return rx.drain_raw(reuse=True)
 
     # correctness guard inside the bench: every step must decode the corpus (no skipped work)
+    n_headers = None
     for _ in range(args.warmup):
         evs, _pay = step_device()
-    n_headers = int((evs["kind"] == 18).sum())
-    n_events = int(evs.size)
+        n_headers, n_events = int((evs["kind"] == 18).sum()), int(evs.size)
 
     sampler = ClockSampler(device)
     launches0 = rx.launch_count()
@@ -359,7 +405,11 @@ def main():
     launches = rx.launch_count() - launches0
     dev_ms = max_over_ranks(dev_ms)
     value = audio_per_step * args.steps * world / (dev_ms * 1e-3)
+    if n_headers is None:       # no warm-up: the last timed step sets the reference counts
+        n_headers, n_events = int((evs["kind"] == 18).sum()), int(evs.size)
     assert int((evs["kind"] == 18).sum()) == n_headers and (n_headers > 0 or args.no_bursts), "bench step lost its work"
+    # drain_raw(reuse=True) hands out views that the e2e leg's drains overwrite
+    last_step = (evs.copy(), _pay.copy()) if args.dump_outputs and rank == 0 else None
     if args.seconds >= 60.0 and not args.no_bursts:
         assert n_headers >= int(0.9 * ns), "corpus not decoded"
 
@@ -476,6 +526,9 @@ def main():
             "headers_decoded_per_step": n_headers, "realtime_factor_per_gpu": round(value / world, 1),
             "config4": config4,
         }
+        if last_step is not None:
+            k, nev = dump_outputs(args.dump_outputs, *last_step, ns)
+            print(f"dumped {nev} events of {k} streams to {args.dump_outputs}", file=sys.stderr)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -668,6 +721,9 @@ def run_reference(args, cfgname, n_samples):
         secs_total += secs
         n_som = int((ev["kind"] == 18).sum())
     wall = time.perf_counter() - t0
+    if args.dump_outputs:
+        k_dumped, nev = dump_outputs(args.dump_outputs, ev, _pay, k)
+        print(f"dumped {nev} events of {k_dumped} streams to {args.dump_outputs}", file=sys.stderr)
     assert args.seconds < 60.0 or n_som >= int(0.9 * k), "reference arm did not decode its corpus"
     value = audio * args.steps / secs_total
     line = {
@@ -688,4 +744,5 @@ def run_reference(args, cfgname, n_samples):
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True      # the tree may be read-only: the benchmark writes nothing into it
     sys.exit(main())

@@ -1,5 +1,5 @@
-import time, numpy as np, torch, sys
-sys.path.insert(0, "/root/repo")
+import time, numpy as np, torch, sys, os
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
 import sameold_b200 as sb
 from sameold_b200 import synth
 RATE=22050; ns=4096; secs=60.0
