@@ -14,6 +14,7 @@ use std::ptr;
 pub struct SameBatchReceiver {
     multi: *mut same_multi,
     n_streams: u32,
+    devices: Vec<i32>,
 }
 
 /// One event of one stream, in order of occurrence per stream (== what `iter_events` yields on that stream).
@@ -55,13 +56,49 @@ impl SameBatchReceiver {
             frame_prefix_max_errors: builder.frame_prefix_max_errors(),
             frame_max_invalid_bytes: builder.frame_max_invalid(),
         };
+        Self::create(&cfg, n_streams, devices)
+    }
+
+    fn create(cfg: &same_config, n_streams: u32, devices: &[i32]) -> Result<Self, String> {
         let mut multi = ptr::null_mut();
-        let rc = unsafe { same_multi_create(&cfg, devices.as_ptr(), devices.len() as u32, n_streams, &mut multi) };
+        let rc = unsafe { same_multi_create(cfg, devices.as_ptr(), devices.len() as u32, n_streams, &mut multi) };
         if rc != 0 {
             let msg = unsafe { std::ffi::CStr::from_ptr(same_multi_last_error(ptr::null())) };
             return Err(format!("same_multi_create: {} ({})", rc, msg.to_string_lossy()));
         }
-        Ok(Self { multi, n_streams })
+        Ok(Self { multi, n_streams, devices: devices.to_vec() })
+    }
+
+    /// The complete receiver state of streams `ids` (`None`: every stream, in order) as a portable buffer (format in
+    /// same_engine.h) that any engine with the same configuration can import, on any device or in another process.
+    pub fn export_streams(&mut self, ids: Option<&[u32]>) -> Result<Vec<u8>, String> {
+        let n = ids.map(|v| v.len() as u32).unwrap_or(self.n_streams);
+        let ids_ptr = ids.map(|v| v.as_ptr()).unwrap_or(ptr::null());
+        let mut buf = vec![0u8; unsafe { same_multi_state_bytes(self.multi, n) }];
+        let mut written = 0usize;
+        unsafe {
+            check(self.multi, same_multi_export_streams(self.multi, ids_ptr, n, buf.as_mut_ptr() as *mut _, buf.len(), &mut written))?;
+        }
+        Ok(buf)
+    }
+
+    /// Record i -> stream `ids[i]` (`None`: record i -> stream i): like `reset` of those streams followed by writing the
+    /// recorded state; all or nothing.
+    pub fn import_streams(&mut self, data: &[u8], ids: Option<&[u32]>) -> Result<(), String> {
+        let n = match ids {
+            Some(v) => v.len() as u32,
+            None => state_info(data)?.1,
+        };
+        let ids_ptr = ids.map(|v| v.as_ptr()).unwrap_or(ptr::null());
+        unsafe { check(self.multi, same_multi_import_streams(self.multi, ids_ptr, n, data.as_ptr() as *const _, data.len())) }
+    }
+
+    /// A new receiver batch on `devices`, built from the configuration embedded in `data` and holding every record.
+    pub fn from_state(data: &[u8], devices: &[i32]) -> Result<Self, String> {
+        let (cfg, n) = state_info(data)?;
+        let mut rx = Self::create(&cfg, n, devices)?;
+        rx.import_streams(data, None)?;
+        Ok(rx)
     }
 
     /// == `iter_events(chunk)` driven to exhaustion on every stream.  `chunks[i]` is stream i's next s16 samples
@@ -154,6 +191,29 @@ impl SameBatchReceiver {
             })
             .collect())
     }
+}
+
+/// == `SameReceiver: Clone` (receiver.rs:70): an independent batch on the same devices in the same state.
+impl Clone for SameBatchReceiver {
+    fn clone(&self) -> Self {
+        let mut me = Self { multi: self.multi, n_streams: self.n_streams, devices: Vec::new() };
+        let data = me.export_streams(None);
+        std::mem::forget(me);   // borrowed handle: not ours to destroy
+        Self::from_state(&data.expect("exporting the receiver state failed"), &self.devices)
+            .expect("importing the receiver state failed")
+    }
+}
+
+/// (configuration, number of records) of an export buffer: header checks only.
+pub fn state_info(data: &[u8]) -> Result<(same_config, u32), String> {
+    let mut cfg = std::mem::MaybeUninit::<same_config>::zeroed();
+    let mut n = 0u32;
+    let rc = unsafe { same_state_info(data.as_ptr() as *const _, data.len(), cfg.as_mut_ptr(), &mut n) };
+    if rc != 0 {
+        let msg = unsafe { std::ffi::CStr::from_ptr(same_last_error()) };
+        return Err(format!("same_state_info: {} ({})", rc, msg.to_string_lossy()));
+    }
+    Ok((unsafe { cfg.assume_init() }, n))
 }
 
 impl Drop for SameBatchReceiver {

@@ -133,6 +133,12 @@ extern "C" {
     pub fn same_engine_snapshot(e: *mut same_engine, out: *mut *mut same_snapshot) -> c_int;
     pub fn same_engine_restore(e: *mut same_engine, snap: *const same_snapshot) -> c_int;
     pub fn same_snapshot_free(snap: *mut same_snapshot);
+    // portable stream state (format in same_engine.h): SameReceiver: Clone for single streams, across engines/devices/processes
+    pub fn same_engine_state_bytes(e: *const same_engine, n: u32) -> usize;
+    pub fn same_engine_export_streams(e: *mut same_engine, ids: *const u32, n: u32, buf: *mut c_void, cap: usize,
+                                      written: *mut usize) -> c_int;
+    pub fn same_engine_import_streams(e: *mut same_engine, ids: *const u32, n: u32, buf: *const c_void, len: usize) -> c_int;
+    pub fn same_state_info(buf: *const c_void, len: usize, cfg: *mut same_config, n_records: *mut u32) -> c_int;
     pub fn same_engine_set_event_capacity(e: *mut same_engine, max_events: usize, max_payload_bytes: usize) -> c_int;
     // diagnostics
     pub fn same_engine_enable_soft_trace(e: *mut same_engine, cap_per_stream: u32) -> c_int;
@@ -166,4 +172,8 @@ extern "C" {
     pub fn same_multi_pending(m: *mut same_multi, n_events: *mut usize, n_payload: *mut usize) -> c_int;
     pub fn same_multi_drain_events(m: *mut same_multi, events: *mut same_event, events_cap: usize, n_events: *mut usize,
                                    payload: *mut u8, payload_cap: usize, n_payload: *mut usize) -> c_int;
+    pub fn same_multi_state_bytes(m: *const same_multi, n: u32) -> usize;
+    pub fn same_multi_export_streams(m: *mut same_multi, ids: *const u32, n: u32, buf: *mut c_void, cap: usize,
+                                     written: *mut usize) -> c_int;
+    pub fn same_multi_import_streams(m: *mut same_multi, ids: *const u32, n: u32, buf: *const c_void, len: usize) -> c_int;
 }

@@ -132,11 +132,55 @@ int same_engine_reset(same_engine* e, const uint32_t* stream_ids, uint32_t n);
 
 /* == `SameReceiver: Clone` (receiver.rs:70): a device-resident copy of every stream's complete state.  restore puts the
  * engine back exactly where snapshot was taken (pending undrained events are dropped).  Used by the host layer to make
- * flush() stop at the sample the reference stops at (receiver.rs:220-222), and as checkpoint/resume.  Both imply sync. */
+ * flush() stop at the sample the reference stops at (receiver.rs:220-222).  The snapshot also keeps the engine's f32 flag
+ * (see same_engine_submit_f32).  Copies that leave the engine: the portable stream state below.  Both imply sync. */
 typedef struct same_snapshot same_snapshot;
 int same_engine_snapshot(same_engine* e, same_snapshot** out);
 int same_engine_restore(same_engine* e, const same_snapshot* snap);
 void same_snapshot_free(same_snapshot* snap);
+
+/* ---- Portable stream state: `SameReceiver: Clone` (receiver.rs:70) for single streams, across engines, devices and
+ * processes (checkpoint / resume, moving a stream to another slot, engine or GPU).
+ *
+ * An export buffer is one header followed by n records.  All fields little-endian; offsets in bytes.
+ *   Header (2224 bytes):
+ *     0  u32 magic 0x54534D53 ("SMST")          4  u32 format version (1; readers accept only their own)
+ *     8  u32 byte-order mark 0x01020304         12 u32 header size (2224)
+ *     16 u32 n_records                          20 u32 n_words (state words per stream)
+ *     24 u32 sizeof(StreamBlob) (3240)          28 u32 SAME_BURST_CAP
+ *     32 u32 record size R                      36 u32 reserved (0)
+ *     40    same_config the state was produced under (sanitized; 19 x 4 bytes)
+ *     116   same_derived of that engine (12 x 4 bytes)
+ *     164   mark filter taps, raw f32 bits, (re, im) x 128, unused taps 0
+ *     1188  space filter taps, same layout
+ *     2212  8 bytes reserved (0)
+ *     2220  u32 CRC-32 (zlib polynomial, as zlib.crc32) of bytes 0..2219
+ *   Record (R = W + B bytes, W = round_up(8 + 4 * n_words, 16), B = round_up(sizeof(StreamBlob) + 4, 16)):
+ *     0      u32 source stream id
+ *     4      u32 flags: bit 0 = the DC-blocker state may be non-integer (the engine had an f32 submit since
+ *            create / reset(all)); other bits 0
+ *     8      the n_words state words in word order (independent of the engine size: a record fits any engine)
+ *     W      the raw StreamBlob; zero padding in between and after
+ *     R - 4  u32 CRC-32 (zlib) of record bytes 0 .. R-5
+ *   At 22050 Hz (6/4 equalizer) n_words = 192 and R = 4032.
+ *
+ * same_engine_state_bytes: exact size of an export of n streams.
+ * same_engine_export_streams: records of streams ids[0..n) in that order (ids == NULL: every stream in order, n is
+ *   ignored).  Changes nothing: pending events stay pending and a stream that keeps running is bit-identical to one
+ *   that was never exported.  cap too small: SAME_ERR_INVALID_ARG with *written = the size needed.  Implies sync.
+ * same_engine_import_streams: record i -> stream ids[i] (ids == NULL: record i -> stream i, n == number of streams).
+ *   Behaves as same_engine_reset(ids) followed by writing the records' state: undrained events of those streams are
+ *   dropped, their next events continue the source's input_sample_counter and seq, their soft trace starts empty.  A
+ *   record with flag bit 0 puts the engine on the rate-generic kernel until reset(all) (same results).  All or nothing:
+ *   on any error no stream changes.  SAME_ERR_INVALID_ARG: bad magic, version or byte order, len not the announced
+ *   size, n != n_records, an id out of range, a duplicate target id, a CRC mismatch, or a record field the receiver
+ *   kernels use as an index or a length out of its range.  SAME_ERR_INVALID_CONFIG: configuration, derived constants,
+ *   filter taps or words per stream differ from this engine's (the message names the first).  Implies sync.
+ * same_state_info: header checks only (no engine, no GPU): the configuration and record count of a buffer. */
+size_t same_engine_state_bytes(const same_engine* e, uint32_t n);
+int same_engine_export_streams(same_engine* e, const uint32_t* ids, uint32_t n, void* buf, size_t cap, size_t* written);
+int same_engine_import_streams(same_engine* e, const uint32_t* ids, uint32_t n, const void* buf, size_t len);
+int same_state_info(const void* buf, size_t len, same_config* cfg, uint32_t* n_records);
 
 /* Capacity of the device event arena (events) and payload arena (bytes).  The arenas fill from one same_engine_sync
  * (or any call that implies it) to the next — NOT per submit: a long run of unsynced submits accumulates.  Defaults:
@@ -281,6 +325,12 @@ int same_multi_input_sample_counters(same_multi* m, uint64_t* out);
 int same_multi_pending(same_multi* m, size_t* n_events, size_t* n_payload_bytes);
 int same_multi_drain_events(same_multi* m, same_event* events, size_t events_cap, size_t* n_events, uint8_t* payload,
                             size_t payload_cap, size_t* n_payload);
+/* Portable stream state with GLOBAL stream ids (format and semantics as same_engine_*_streams above), routed to the
+ * owning shards and run on the shards' threads in parallel; records come out in the order of `ids` and carry global
+ * source ids.  An import validates on every shard before any shard changes. */
+size_t same_multi_state_bytes(const same_multi* m, uint32_t n);
+int same_multi_export_streams(same_multi* m, const uint32_t* ids, uint32_t n, void* buf, size_t cap, size_t* written);
+int same_multi_import_streams(same_multi* m, const uint32_t* ids, uint32_t n, const void* buf, size_t len);
 
 #ifdef __cplusplus
 }

@@ -128,11 +128,11 @@ class SameReceiverBuilder {   // builder.rs:14-357
 
 class SameBatchReceiver {
  public:
-  SameBatchReceiver(const same_config& cfg, uint32_t n_streams, int device = 0) : n_(n_streams) {
+  SameBatchReceiver(const same_config& cfg, uint32_t n_streams, int device = 0) : n_(n_streams), device_(device) {
     int rc = same_engine_create(&cfg, device, n_streams, &e_);
     if (rc) throw EngineError(rc, same_last_error());
   }
-  SameBatchReceiver(SameBatchReceiver&& o) noexcept : e_(o.e_), n_(o.n_) { o.e_ = nullptr; }
+  SameBatchReceiver(SameBatchReceiver&& o) noexcept : e_(o.e_), n_(o.n_), device_(o.device_) { o.e_ = nullptr; }
   SameBatchReceiver(const SameBatchReceiver&) = delete;
   ~SameBatchReceiver() { if (e_) same_engine_destroy(e_); }
 
@@ -204,6 +204,31 @@ class SameBatchReceiver {
     return out;
   }
   same_engine* handle() { return e_; }
+  int device() const { return device_; }
+
+  // Portable stream state (format: same_engine.h): the complete receiver state of `ids` (empty: every stream, in order)
+  std::vector<uint8_t> export_streams(const std::vector<uint32_t>& ids = {}) {
+    const uint32_t n = ids.empty() ? n_ : (uint32_t)ids.size();
+    std::vector<uint8_t> buf(same_engine_state_bytes(e_, n));
+    size_t written = 0;
+    ck(same_engine_export_streams(e_, ids.empty() ? nullptr : ids.data(), n, buf.data(), buf.size(), &written));
+    return buf;
+  }
+  // record i -> stream ids[i] (empty: record i -> stream i); == reset(ids) + the recorded state, all or nothing
+  void import_streams(const std::vector<uint8_t>& data, const std::vector<uint32_t>& ids = {}) {
+    const uint32_t n = ids.empty() ? n_ : (uint32_t)ids.size();
+    ck(same_engine_import_streams(e_, ids.empty() ? nullptr : ids.data(), n, data.data(), data.size()));
+  }
+  // a new engine built from the configuration embedded in `data`, holding every record of it
+  static SameBatchReceiver from_state(const std::vector<uint8_t>& data, int device = 0) {
+    same_config cfg;
+    uint32_t n = 0;
+    int rc = same_state_info(data.data(), data.size(), &cfg, &n);
+    if (rc) throw EngineError(rc, same_last_error());
+    SameBatchReceiver rx(cfg, n, device);
+    rx.import_streams(data);
+    return rx;
+  }
 
  private:
   void ck(int rc) { if (rc) throw EngineError(rc, same_engine_last_error(e_)); }
@@ -225,6 +250,7 @@ class SameBatchReceiver {
   }
   same_engine* e_ = nullptr;
   uint32_t n_;
+  int device_ = 0;
   friend class SameReceiver;
 };
 
@@ -235,6 +261,12 @@ class SameReceiver {
   uint32_t input_rate() const { return b_.input_rate(); }
   uint64_t input_sample_counter() { return b_.input_sample_counters()[0]; }
   void reset() { b_.reset(); }
+  // this receiver's complete state as a portable buffer
+  std::vector<uint8_t> export_state() { return b_.export_streams(); }
+  // == `SameReceiver: Clone` (receiver.rs:70): a new receiver on `device` (-1: this one's) in the same state
+  SameReceiver clone(int device = -1) {
+    return SameReceiver(SameBatchReceiver::from_state(export_state(), device < 0 ? b_.device() : device));
+  }
   std::vector<SameReceiverEvent> iter_events(const std::vector<int16_t>& samples) {                                               // receiver.rs:119-130
     auto evs = b_.process(std::vector<std::vector<int16_t>>{samples});
     return std::move(evs[0]);

@@ -13,6 +13,7 @@ from .receiver import (  # noqa: F401
     SameReceiver,
     SameReceiverBuilder,
     SameReceiverEvent,
+    state_info,
 )
 from .build import build_native  # noqa: F401
 

@@ -72,6 +72,10 @@ API = {
     "same_engine_snapshot": (C.c_int, [_P, C.POINTER(_P)]),
     "same_engine_restore": (C.c_int, [_P, _P]),
     "same_snapshot_free": (None, [_P]),
+    "same_engine_state_bytes": (C.c_size_t, [_P, C.c_uint32]),
+    "same_engine_export_streams": (C.c_int, [_P, _P, C.c_uint32, _P, C.c_size_t, C.POINTER(C.c_size_t)]),
+    "same_engine_import_streams": (C.c_int, [_P, _P, C.c_uint32, _P, C.c_size_t]),
+    "same_state_info": (C.c_int, [_P, C.c_size_t, C.POINTER(SameConfig), C.POINTER(C.c_uint32)]),
     "same_engine_set_event_capacity": (C.c_int, [_P, C.c_size_t, C.c_size_t]),
     "same_engine_submit_s16": (C.c_int, [_P, _P, C.c_uint64, _P, _P]),
     "same_engine_submit_s16_2d": (C.c_int, [_P, _P, C.c_uint64, C.c_uint64, C.c_uint32]),
@@ -114,6 +118,9 @@ API = {
     "same_multi_input_sample_counters": (C.c_int, [_P, _P]),
     "same_multi_pending": (C.c_int, [_P, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
     "same_multi_drain_events": (C.c_int, [_P, _P, C.c_size_t, C.POINTER(C.c_size_t), _P, C.c_size_t, C.POINTER(C.c_size_t)]),
+    "same_multi_state_bytes": (C.c_size_t, [_P, C.c_uint32]),
+    "same_multi_export_streams": (C.c_int, [_P, _P, C.c_uint32, _P, C.c_size_t, C.POINTER(C.c_size_t)]),
+    "same_multi_import_streams": (C.c_int, [_P, _P, C.c_uint32, _P, C.c_size_t]),
     # synthetic corpus generator (bench / test tooling, same library)
     "same_synth_generate": (C.c_int, [C.c_int, _P, C.c_uint32, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint32, _P, _P, C.c_uint32,
                                       _P, C.c_uint64, _P, _P, C.c_float, C.c_float, _P]),

@@ -35,6 +35,15 @@ extern "C" cudaError_t same_launch_evsort(const same_event* d_events, uint32_t n
                                           cudaStream_t stream);
 extern "C" cudaError_t same_launch_init(const SameParams* p, const uint32_t* d_ids, uint32_t n, int after_reset,
                                         cudaStream_t stream);
+// same_state.cu
+extern "C" uint32_t same_state_record_bytes(uint32_t n_words);
+extern "C" uint32_t same_state_crc32(const void* data, size_t n);
+extern "C" cudaError_t same_state_launch_gather(const SameParams* p, const uint32_t* d_ids, uint32_t first, uint32_t n,
+                                                uint32_t id_base, uint32_t rec_flags, uint8_t* d_out, cudaStream_t stream);
+extern "C" cudaError_t same_state_launch_validate(const uint8_t* d_in, uint32_t n, uint32_t n_words, unsigned long long* d_result,
+                                                  cudaStream_t stream);
+extern "C" cudaError_t same_state_launch_scatter(const SameParams* p, const uint32_t* d_ids, uint32_t first, uint32_t n,
+                                                 const uint8_t* d_in, cudaStream_t stream);
 
 namespace {
 
@@ -128,6 +137,12 @@ struct same_engine {
   std::vector<uint8_t> pend_payload;
   cudaEvent_t t_h2d0 = nullptr, t_h2d1 = nullptr, t_k0 = nullptr, t_k1 = nullptr, t_sw0 = nullptr, t_sw1 = nullptr;
   bool timed_h2d = false, timed_kernel = false;
+  // portable stream state (same_state.cu): device staging of records, ids, validation result, timing of the last call
+  uint8_t* d_xfer = nullptr; size_t xfer_cap = 0;
+  uint32_t* d_xids = nullptr; size_t xids_cap = 0;
+  unsigned long long* d_xres = nullptr;
+  cudaEvent_t t_st[3] = {nullptr, nullptr, nullptr};
+  float st_kernel_ms = 0.0f, st_copy_ms = 0.0f;
   uint64_t launches = 0;
   std::string last_error;
 };
@@ -616,6 +631,7 @@ int same_engine_create(const same_config* cfg_in, int device, uint32_t n_streams
   CKC(cudaEventCreate(&e->t_h2d0)); CKC(cudaEventCreate(&e->t_h2d1));
   CKC(cudaEventCreate(&e->t_k0)); CKC(cudaEventCreate(&e->t_k1));
   CKC(cudaEventCreate(&e->t_sw0)); CKC(cudaEventCreate(&e->t_sw1));
+  for (auto& ev : e->t_st) CKC(cudaEventCreate(&ev));
   p.state32 = e->d_state; p.blobs = e->d_blobs; p.counters = e->d_counters;
   {
     size_t nev = std::max<size_t>(65536, (size_t)n_streams * 64);
@@ -660,6 +676,10 @@ void same_engine_destroy(same_engine* e) {
   if (e->tiles.d) cudaFree(e->tiles.d);
   if (e->tiles.dc_next) cudaFree(e->tiles.dc_next);
   for (cudaEvent_t ev : {e->t_h2d0, e->t_h2d1, e->t_k0, e->t_k1, e->t_sw0, e->t_sw1}) if (ev) cudaEventDestroy(ev);
+  for (cudaEvent_t ev : e->t_st) if (ev) cudaEventDestroy(ev);
+  if (e->d_xfer) cudaFree(e->d_xfer);
+  if (e->d_xids) cudaFree(e->d_xids);
+  if (e->d_xres) cudaFree(e->d_xres);
   if (e->compute) cudaStreamDestroy(e->compute);
   if (e->copy) cudaStreamDestroy(e->copy);
   delete e;
@@ -728,6 +748,7 @@ int same_engine_reset(same_engine* e, const uint32_t* ids, uint32_t n) {
 struct same_snapshot {
   int device; uint32_t n_streams; size_t state_bytes, blob_bytes;
   uint32_t* d_state; StreamBlob* d_blobs;
+  bool saw_f32;   // the DC-blocker state may be non-integer: restore must keep the engine on the generic kernel
 };
 
 int same_engine_snapshot(same_engine* e, same_snapshot** out) {
@@ -739,6 +760,7 @@ int same_engine_snapshot(same_engine* e, same_snapshot** out) {
   s->state_bytes = (size_t)e->p.layout.n_words * e->p.layout.n_pad * sizeof(uint32_t);
   s->blob_bytes = (size_t)e->n_streams * sizeof(StreamBlob);
   s->d_state = nullptr; s->d_blobs = nullptr;
+  s->saw_f32 = e->saw_f32;
   cudaError_t err = cudaMalloc(&s->d_state, s->state_bytes);
   if (err == cudaSuccess) err = cudaMalloc(&s->d_blobs, s->blob_bytes);
   if (err == cudaSuccess) err = cudaMemcpyAsync(s->d_state, e->d_state, s->state_bytes, cudaMemcpyDeviceToDevice, e->compute);
@@ -763,6 +785,7 @@ int same_engine_restore(same_engine* e, const same_snapshot* s) {
   CK(e, cudaMemcpyAsync(e->d_blobs, s->d_blobs, s->blob_bytes, cudaMemcpyDeviceToDevice, e->compute));
   CK(e, cudaStreamSynchronize(e->compute));
   e->pend_events.clear(); e->pend_payload.clear();
+  e->saw_f32 = s->saw_f32;
   return SAME_OK;
 }
 
@@ -926,6 +949,8 @@ int same_engine_get_option(same_engine* e, const char* key, int* value) {
   if (strcmp(key, "long_stream_passes") == 0) { *value = (int)std::min<uint64_t>(e->ls_spec_launches, 0x7fffffff); return SAME_OK; }
   if (strcmp(key, "long_stream_fallback_spans") == 0) { *value = (int)std::min<uint64_t>(e->ls_fallback_launches, 0x7fffffff); return SAME_OK; }
   if (strcmp(key, "lanes_per_warp") == 0) { *value = (int)e->lanes_per_warp; return SAME_OK; }
+  if (strcmp(key, "state_kernel_us") == 0) { *value = (int)std::min(e->st_kernel_ms * 1000.0f, 2.0e9f); return SAME_OK; }
+  if (strcmp(key, "state_copy_us") == 0) { *value = (int)std::min(e->st_copy_ms * 1000.0f, 2.0e9f); return SAME_OK; }
   if (strcmp(key, "kernel_selected") == 0) {
     const bool fast_geometry = e->p.ntaps == 42 && e->p.dc_len == 16;
     *value = (e->saw_f32 || !fast_geometry) ? 1 : (e->force_generic ? e->force_generic : e->kernel_auto);
@@ -998,6 +1023,350 @@ int same_engine_get_derived(const same_engine* e, same_derived* d, float* mark_r
     if (mark_re_im) { mark_re_im[2 * i] = e->taps.mark_re[i]; mark_re_im[2 * i + 1] = e->taps.mark_im[i]; }
     if (space_re_im) { space_re_im[2 * i] = e->taps.space_re[i]; space_re_im[2 * i + 1] = e->taps.space_im[i]; }
   }
+  return SAME_OK;
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Portable stream state (format in include/same_engine.h).  The header is parsed and compared with an engine here only;
+// same_multi.cu reuses these helpers (same_state_* below, C++ linkage, not part of the C ABI).
+// ---------------------------------------------------------------------------------------------------------------------
+namespace {
+
+constexpr uint32_t kStMagic = 0x54534D53u;   // "SMST"
+constexpr uint32_t kStVersion = 1u;
+constexpr uint32_t kStBom = 0x01020304u;
+constexpr size_t kStHeaderBytes = 2224;
+constexpr size_t kStOffConfig = 40, kStOffDerived = 116, kStOffMark = 164, kStOffSpace = 1188, kStOffCrc = 2220;
+static_assert(sizeof(same_config) == 19 * 4 && sizeof(same_derived) == 12 * 4, "4-byte fields only");
+static_assert(kStOffDerived == kStOffConfig + sizeof(same_config) && kStOffMark == kStOffDerived + sizeof(same_derived) &&
+              kStOffSpace == kStOffMark + 8 * SAME_MAX_TAPS && kStOffCrc + 4 == kStHeaderBytes, "header layout");
+
+void put32(uint8_t* p, uint32_t v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); p[2] = (uint8_t)(v >> 16); p[3] = (uint8_t)(v >> 24); }
+uint32_t get32(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24); }
+// a struct of 4-byte fields <-> little-endian words
+void put_words(uint8_t* p, const void* src, size_t bytes) {
+  for (size_t i = 0; i < bytes; i += 4) { uint32_t v; memcpy(&v, static_cast<const uint8_t*>(src) + i, 4); put32(p + i, v); }
+}
+void get_words(void* dst, const uint8_t* p, size_t bytes) {
+  for (size_t i = 0; i < bytes; i += 4) { const uint32_t v = get32(p + i); memcpy(static_cast<uint8_t*>(dst) + i, &v, 4); }
+}
+
+const char* const kConfigFields[19] = {
+    "input_rate", "dc_blocker_len", "agc_bandwidth", "agc_gain_min", "agc_gain_max", "timing_bw_unlocked",
+    "timing_bw_locked", "timing_max_deviation", "squelch_power_open", "squelch_power_close", "squelch_bandwidth",
+    "preamble_max_errors", "eq_enabled", "eq_nff", "eq_nfb", "eq_relaxation", "eq_regularization",
+    "frame_prefix_max_errors", "frame_max_invalid_bytes"};
+const char* const kDerivedFields[12] = {"sps", "agc_bw", "agc_gain0", "samples_per_ted", "period_min", "period_max",
+                                        "alpha_unlocked", "beta_unlocked", "alpha_locked", "beta_locked", "dc_len", "ntaps"};
+// same_state.cu: enum Check
+const char* const kCheckNames[] = {
+    "valid", "CRC mismatch", "record flags (only bit 0 is defined)", "F_FLAGS (undefined bits)", "framer state > 2",
+    "transport state > 2", "F_CLOCK > 2^22", "F_TEDCNT not in {0, 1}", "F_SQ_BYTECLK not in -1..7", "F_SQ_HEAD >= 64",
+    "F_HIST_N > 3", "burst history length > 268", "pending length > 268", "pending kind > 2", "pending error > 3",
+    "pending_offset beyond the pending text", "previous-message length > 268"};
+
+struct StateHeader {
+  same_config cfg;
+  same_derived derived;
+  uint8_t taps[2 * 8 * SAME_MAX_TAPS];   // raw little-endian bits: mark (re, im) x 128, then space
+  uint32_t n_records, n_words, record_bytes;
+};
+
+void write_header(const same_engine* e, uint32_t n, uint8_t* h) {
+  memset(h, 0, kStHeaderBytes);
+  put32(h + 0, kStMagic); put32(h + 4, kStVersion); put32(h + 8, kStBom); put32(h + 12, (uint32_t)kStHeaderBytes);
+  put32(h + 16, n); put32(h + 20, e->p.layout.n_words); put32(h + 24, (uint32_t)sizeof(StreamBlob));
+  put32(h + 28, SAME_BURST_CAP); put32(h + 32, same_state_record_bytes(e->p.layout.n_words));
+  put_words(h + kStOffConfig, &e->cfg, sizeof(same_config));
+  put_words(h + kStOffDerived, &e->derived, sizeof(same_derived));
+  for (uint32_t i = 0; i < e->p.ntaps; ++i) {
+    const float v[4] = {e->taps.mark_re[i], e->taps.mark_im[i], e->taps.space_re[i], e->taps.space_im[i]};
+    put_words(h + kStOffMark + 8 * i, v, 8);
+    put_words(h + kStOffSpace + 8 * i, v + 2, 8);
+  }
+  put32(h + kStOffCrc, same_state_crc32(h, kStOffCrc));
+}
+
+// Format checks only (no engine): SAME_ERR_INVALID_ARG on any failure
+int parse_header(const void* buf, size_t len, StateHeader* out, std::string* why) {
+  const uint8_t* h = static_cast<const uint8_t*>(buf);
+  auto bad = [&](const std::string& m) { *why = "state buffer: " + m; return (int)SAME_ERR_INVALID_ARG; };
+  if (!h) return bad("null pointer");
+  if (len < 16) return bad("truncated header");
+  if (get32(h) != kStMagic) return bad("bad magic");
+  if (get32(h + 8) != kStBom) return bad("wrong byte order");
+  if (get32(h + 4) != kStVersion) return bad("format version " + std::to_string(get32(h + 4)) + ", this library reads version " + std::to_string(kStVersion));
+  if (get32(h + 12) != kStHeaderBytes) return bad("bad header size");
+  if (len < kStHeaderBytes) return bad("truncated header");
+  if (get32(h + kStOffCrc) != same_state_crc32(h, kStOffCrc)) return bad("header CRC mismatch");
+  StateHeader s;
+  s.n_records = get32(h + 16); s.n_words = get32(h + 20); s.record_bytes = get32(h + 32);
+  if (get32(h + 24) != sizeof(StreamBlob) || get32(h + 28) != SAME_BURST_CAP) return bad("stream blob layout differs from this library's");
+  if (s.n_words < F_NUM_SCALARS || s.n_words > (1u << 16) || s.record_bytes != same_state_record_bytes(s.n_words))
+    return bad("inconsistent record size");
+  const size_t need = kStHeaderBytes + (size_t)s.n_records * s.record_bytes;
+  if (len < need) return bad("truncated: " + std::to_string(len) + " bytes, the header announces " + std::to_string(need));
+  if (len > need) return bad("trailing bytes after the last record");
+  get_words(&s.cfg, h + kStOffConfig, sizeof(same_config));
+  get_words(&s.derived, h + kStOffDerived, sizeof(same_derived));
+  memcpy(s.taps, h + kStOffMark, sizeof s.taps);
+  *out = s;
+  return SAME_OK;
+}
+
+// The state must have been produced under exactly this engine's configuration: SAME_ERR_INVALID_CONFIG names the first
+// field that differs (derived values and taps are compared bit for bit: they are libm results of the exporting host)
+int compare_header(const same_engine* e, const StateHeader& s, std::string* why) {
+  uint32_t a[19], b[19];
+  memcpy(a, &e->cfg, sizeof a); memcpy(b, &s.cfg, sizeof b);
+  for (int i = 0; i < 19; ++i)
+    if (a[i] != b[i]) { *why = std::string("state was produced under another configuration: ") + kConfigFields[i] + " differs"; return SAME_ERR_INVALID_CONFIG; }
+  uint32_t c[12], d[12];
+  memcpy(c, &e->derived, sizeof c); memcpy(d, &s.derived, sizeof d);
+  for (int i = 0; i < 12; ++i)
+    if (c[i] != d[i]) { *why = std::string("derived constant ") + kDerivedFields[i] + " differs from this engine's (another host's libm?)"; return SAME_ERR_INVALID_CONFIG; }
+  StateHeader mine;
+  {
+    uint8_t h[kStHeaderBytes];
+    write_header(e, 0, h);
+    memcpy(mine.taps, h + kStOffMark, sizeof mine.taps);
+  }
+  if (memcmp(mine.taps, s.taps, 8 * SAME_MAX_TAPS) != 0) { *why = "mark filter taps differ from this engine's"; return SAME_ERR_INVALID_CONFIG; }
+  if (memcmp(mine.taps + 8 * SAME_MAX_TAPS, s.taps + 8 * SAME_MAX_TAPS, 8 * SAME_MAX_TAPS) != 0) {
+    *why = "space filter taps differ from this engine's"; return SAME_ERR_INVALID_CONFIG;
+  }
+  if (s.n_words != e->p.layout.n_words) { *why = "state words per stream differ from this engine's"; return SAME_ERR_INVALID_CONFIG; }
+  return SAME_OK;
+}
+
+bool is_pinned(const void* p) {
+  cudaPointerAttributes a;
+  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
+  return a.type == cudaMemoryTypeHost;
+}
+
+int ensure_xfer(same_engine* e, size_t bytes, uint32_t n_ids) {
+  if (bytes > e->xfer_cap) {
+    if (e->d_xfer) CK(e, cudaFree(e->d_xfer));
+    e->d_xfer = nullptr; e->xfer_cap = 0;
+    CK(e, cudaMalloc(&e->d_xfer, bytes));
+    e->xfer_cap = bytes;
+  }
+  if (n_ids > e->xids_cap) {
+    if (e->d_xids) CK(e, cudaFree(e->d_xids));
+    e->d_xids = nullptr; e->xids_cap = 0;
+    CK(e, cudaMalloc(&e->d_xids, (size_t)n_ids * sizeof(uint32_t)));
+    e->xids_cap = n_ids;
+  }
+  if (!e->d_xres) CK(e, cudaMalloc(&e->d_xres, 2 * sizeof(unsigned long long)));
+  return SAME_OK;
+}
+
+// ids -> (device id list, or nullptr + first for a contiguous run)
+int upload_ids(same_engine* e, const uint32_t* ids, uint32_t n, const uint32_t** d_ids, uint32_t* first) {
+  *d_ids = nullptr; *first = 0;
+  if (!ids || n == 0) return SAME_OK;
+  bool run = true;
+  for (uint32_t i = 1; i < n && run; ++i) run = ids[i] == ids[0] + i;
+  if (run) { *first = ids[0]; return SAME_OK; }
+  CK(e, cudaMemcpyAsync(e->d_xids, ids, (size_t)n * sizeof(uint32_t), cudaMemcpyHostToDevice, e->compute));
+  *d_ids = e->d_xids;
+  return SAME_OK;
+}
+
+// device -> host (pinned: one copy; pageable: through the pinned staging area, two pieces in flight)
+int copy_out(same_engine* e, uint8_t* dst, const uint8_t* src, size_t bytes) {
+  if (is_pinned(dst)) {
+    if (bytes) CK(e, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, e->compute));
+    return SAME_OK;
+  }
+  const size_t half = STAGE_BYTES / 2;
+  size_t done = 0, queued = 0, qn[2] = {0, 0};
+  int qslot = 0, pslot = 0, inflight = 0;
+  while (done < bytes) {
+    while (inflight < 2 && queued < bytes) {
+      const size_t n = std::min(half, bytes - queued);
+      CK(e, cudaMemcpyAsync(e->h_stage + qslot * half, src + queued, n, cudaMemcpyDeviceToHost, e->compute));
+      CK(e, cudaEventRecord(e->stage_done[qslot], e->compute));
+      qn[qslot] = n; queued += n; qslot ^= 1; ++inflight;
+    }
+    CK(e, cudaEventSynchronize(e->stage_done[pslot]));
+    memcpy(dst + done, e->h_stage + pslot * half, qn[pslot]);
+    done += qn[pslot]; pslot ^= 1; --inflight;
+  }
+  return SAME_OK;
+}
+
+// host -> device, the same way round
+int copy_in(same_engine* e, uint8_t* dst, const uint8_t* src, size_t bytes) {
+  if (is_pinned(src)) {
+    if (bytes) CK(e, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, e->compute));
+    return SAME_OK;
+  }
+  const size_t half = STAGE_BYTES / 2;
+  int slot = 0;
+  for (size_t off = 0; off < bytes; off += half, slot ^= 1) {
+    const size_t n = std::min(half, bytes - off);
+    CK(e, cudaEventSynchronize(e->stage_done[slot]));   // the copy that last read this half has finished
+    memcpy(e->h_stage + slot * half, src + off, n);
+    CK(e, cudaMemcpyAsync(dst + off, e->h_stage + slot * half, n, cudaMemcpyHostToDevice, e->compute));
+    CK(e, cudaEventRecord(e->stage_done[slot], e->compute));
+  }
+  return SAME_OK;
+}
+
+int check_ids(same_engine* e, const uint32_t* ids, uint32_t n, uint32_t limit, bool unique) {
+  if (!ids) return SAME_OK;
+  std::vector<char> seen(unique ? limit : 0, 0);
+  for (uint32_t i = 0; i < n; ++i) {
+    if (ids[i] >= limit) return fail(e, SAME_ERR_INVALID_ARG, "stream id " + std::to_string(ids[i]) + " out of range");
+    if (unique) {
+      if (seen[ids[i]]) return fail(e, SAME_ERR_INVALID_ARG, "duplicate target stream id " + std::to_string(ids[i]));
+      seen[ids[i]] = 1;
+    }
+  }
+  return SAME_OK;
+}
+
+}  // namespace
+
+// ---- helpers shared with same_multi.cu (C++ linkage; the engine must be synced and the arguments checked) ----
+size_t same_state_header_bytes() { return kStHeaderBytes; }
+size_t same_state_engine_record_bytes(const same_engine* e) { return same_state_record_bytes(e->p.layout.n_words); }
+void same_state_write_header(const same_engine* e, uint32_t n, void* dst) { write_header(e, n, static_cast<uint8_t*>(dst)); }
+
+// header format + comparison with `e`; on failure the reason is the engine's last error
+int same_state_check_header(same_engine* e, const void* buf, size_t len, uint32_t* n_records) {
+  StateHeader s;
+  std::string why;
+  int rc = parse_header(buf, len, &s, &why);
+  if (rc == SAME_OK) rc = compare_header(e, s, &why);
+  if (rc != SAME_OK) return fail(e, rc, why);
+  *n_records = s.n_records;
+  return SAME_OK;
+}
+
+// n records of `ids` (nullptr: streams 0..n-1) -> host dst (n * record bytes); source ids are written as id + id_base
+int same_state_export_records(same_engine* e, const uint32_t* ids, uint32_t n, uint32_t id_base, void* dst) {
+  int rc = same_engine_sync(e);
+  if (rc) return rc;
+  CK(e, cudaSetDevice(e->device));
+  const size_t bytes = (size_t)n * same_state_engine_record_bytes(e);
+  rc = ensure_xfer(e, bytes, n);
+  if (rc) return rc;
+  const uint32_t* d_ids; uint32_t first;
+  rc = upload_ids(e, ids, n, &d_ids, &first);
+  if (rc) return rc;
+  CK(e, cudaEventRecord(e->t_st[0], e->compute));
+  CK(e, same_state_launch_gather(&e->p, d_ids, first, n, id_base, e->saw_f32 ? 1u : 0u, e->d_xfer, e->compute));
+  e->launches += n ? 1 : 0;
+  CK(e, cudaEventRecord(e->t_st[1], e->compute));
+  rc = copy_out(e, static_cast<uint8_t*>(dst), e->d_xfer, bytes);
+  if (rc) return rc;
+  CK(e, cudaEventRecord(e->t_st[2], e->compute));
+  CK(e, cudaStreamSynchronize(e->compute));
+  CK(e, cudaEventElapsedTime(&e->st_kernel_ms, e->t_st[0], e->t_st[1]));
+  CK(e, cudaEventElapsedTime(&e->st_copy_ms, e->t_st[1], e->t_st[2]));
+  return SAME_OK;
+}
+
+// phase 1 of an import: records -> device staging, validated there.  Changes no stream.
+int same_state_import_stage(same_engine* e, uint32_t n, const void* recs, uint32_t* rec_flags) {
+  int rc = same_engine_sync(e);
+  if (rc) return rc;
+  CK(e, cudaSetDevice(e->device));
+  const size_t bytes = (size_t)n * same_state_engine_record_bytes(e);
+  rc = ensure_xfer(e, bytes, n);
+  if (rc) return rc;
+  const unsigned long long init[2] = {~0ull, 0ull};
+  CK(e, cudaMemcpyAsync(e->d_xres, init, sizeof init, cudaMemcpyHostToDevice, e->compute));
+  CK(e, cudaEventRecord(e->t_st[0], e->compute));
+  rc = copy_in(e, e->d_xfer, static_cast<const uint8_t*>(recs), bytes);
+  if (rc) return rc;
+  CK(e, cudaEventRecord(e->t_st[1], e->compute));
+  CK(e, same_state_launch_validate(e->d_xfer, n, e->p.layout.n_words, e->d_xres, e->compute));
+  e->launches += n ? 1 : 0;
+  CK(e, cudaEventRecord(e->t_st[2], e->compute));
+  unsigned long long res[2];
+  CK(e, cudaMemcpyAsync(res, e->d_xres, sizeof res, cudaMemcpyDeviceToHost, e->compute));
+  CK(e, cudaStreamSynchronize(e->compute));
+  CK(e, cudaEventElapsedTime(&e->st_copy_ms, e->t_st[0], e->t_st[1]));
+  CK(e, cudaEventElapsedTime(&e->st_kernel_ms, e->t_st[1], e->t_st[2]));
+  if (res[0] != ~0ull) {
+    const uint32_t code = (uint32_t)res[0], rec = (uint32_t)(res[0] >> 32);
+    const size_t nc = sizeof kCheckNames / sizeof kCheckNames[0];
+    return fail(e, SAME_ERR_INVALID_ARG, "state record " + std::to_string(rec) + ": " + (code < nc ? kCheckNames[code] : "invalid"));
+  }
+  *rec_flags = (uint32_t)res[1];
+  return SAME_OK;
+}
+
+// phase 2: the staged records -> streams ids[i] (nullptr: 0..n-1); == reset(ids) + the records' state
+int same_state_import_commit(same_engine* e, const uint32_t* ids, uint32_t n, uint32_t rec_flags) {
+  CK(e, cudaSetDevice(e->device));
+  const uint32_t* d_ids; uint32_t first;
+  int rc = upload_ids(e, ids, n, &d_ids, &first);
+  if (rc) return rc;
+  CK(e, cudaEventRecord(e->t_st[0], e->compute));
+  CK(e, same_state_launch_scatter(&e->p, d_ids, first, n, e->d_xfer, e->compute));
+  e->launches += n ? 1 : 0;
+  CK(e, cudaEventRecord(e->t_st[1], e->compute));
+  CK(e, cudaStreamSynchronize(e->compute));
+  float ms = 0.0f;
+  CK(e, cudaEventElapsedTime(&ms, e->t_st[0], e->t_st[1]));
+  e->st_kernel_ms += ms;
+  // undrained events of the target streams belong to the state that was replaced
+  std::vector<char> hit(e->n_streams, 0);
+  for (uint32_t i = 0; i < n; ++i) hit[ids ? ids[i] : i] = 1;
+  e->pend_events.erase(std::remove_if(e->pend_events.begin(), e->pend_events.end(),
+                                      [&](const same_event& ev) { return hit[ev.stream] != 0; }),
+                       e->pend_events.end());
+  if (rec_flags & 1u) e->saw_f32 = true;
+  return SAME_OK;
+}
+
+extern "C" {
+
+size_t same_engine_state_bytes(const same_engine* e, uint32_t n) {
+  return e ? kStHeaderBytes + (size_t)n * same_state_engine_record_bytes(e) : 0;
+}
+
+int same_engine_export_streams(same_engine* e, const uint32_t* ids, uint32_t n, void* buf, size_t cap, size_t* written) {
+  if (!e) return fail(nullptr, SAME_ERR_INVALID_ARG, "null engine");
+  if (!ids) n = e->n_streams;
+  int rc = check_ids(e, ids, n, e->n_streams, false);
+  if (rc) return rc;
+  const size_t need = same_engine_state_bytes(e, n);
+  if (written) *written = need;
+  if (!buf || cap < need) return fail(e, SAME_ERR_INVALID_ARG, "export buffer too small: " + std::to_string(need) + " bytes needed");
+  write_header(e, n, static_cast<uint8_t*>(buf));
+  return same_state_export_records(e, ids, n, 0, static_cast<uint8_t*>(buf) + kStHeaderBytes);
+}
+
+int same_engine_import_streams(same_engine* e, const uint32_t* ids, uint32_t n, const void* buf, size_t len) {
+  if (!e) return fail(nullptr, SAME_ERR_INVALID_ARG, "null engine");
+  uint32_t n_records = 0;
+  int rc = same_state_check_header(e, buf, len, &n_records);
+  if (rc) return rc;
+  if (!ids && n != e->n_streams) return fail(e, SAME_ERR_INVALID_ARG, "ids == NULL imports into every stream: n must equal the number of streams");
+  if (n != n_records) return fail(e, SAME_ERR_INVALID_ARG, "n = " + std::to_string(n) + " but the buffer holds " + std::to_string(n_records) + " records");
+  rc = check_ids(e, ids, n, e->n_streams, true);
+  if (rc) return rc;
+  uint32_t flags = 0;
+  rc = same_state_import_stage(e, n, static_cast<const uint8_t*>(buf) + kStHeaderBytes, &flags);
+  if (rc) return rc;
+  return same_state_import_commit(e, ids, n, flags);
+}
+
+int same_state_info(const void* buf, size_t len, same_config* cfg, uint32_t* n_records) {
+  StateHeader s;
+  std::string why;
+  const int rc = parse_header(buf, len, &s, &why);
+  if (rc) return fail(nullptr, rc, why);
+  if (cfg) *cfg = s.cfg;
+  if (n_records) *n_records = s.n_records;
   return SAME_OK;
 }
 

@@ -5,7 +5,8 @@
 // Streams are independent (SameReceiver owns all of its state, receiver.rs:71-90), so there is no collective and no
 // device-to-device traffic: shard i owns the contiguous stream range [first_i, first_i + count_i), every call fans out
 // to the shards' worker threads, and drain concatenates the per-device event lists re-tagged with global stream ids
-// (the "host-side gather of decoded messages").  Built on the public single-device C ABI only.
+// (the "host-side gather of decoded messages").  Built on the public single-device C ABI, plus the engine's internal
+// stream-state helpers (same_engine.cu) so that an import can validate on every shard before any shard changes.
 #include <algorithm>
 #include <condition_variable>
 #include <cstring>
@@ -16,6 +17,15 @@
 #include <vector>
 
 #include "../../include/same_engine.h"
+
+// same_engine.cu: portable stream state, one engine
+size_t same_state_header_bytes();
+size_t same_state_engine_record_bytes(const same_engine* e);
+void same_state_write_header(const same_engine* e, uint32_t n, void* dst);
+int same_state_check_header(same_engine* e, const void* buf, size_t len, uint32_t* n_records);
+int same_state_export_records(same_engine* e, const uint32_t* ids, uint32_t n, uint32_t id_base, void* dst);
+int same_state_import_stage(same_engine* e, uint32_t n, const void* recs, uint32_t* rec_flags);
+int same_state_import_commit(same_engine* e, const uint32_t* ids, uint32_t n, uint32_t rec_flags);
 
 namespace {
 
@@ -33,6 +43,10 @@ struct Shard {
   // scratch reused across submits
   std::vector<uint64_t> off;
   size_t pend_ev = 0, pend_pay = 0;
+  // stream-state export / import: this shard's share of a call
+  std::vector<uint32_t> st_ids, st_pos;
+  std::vector<uint8_t> st_buf;
+  uint32_t st_flags = 0;
   std::string err;   // text of a failed create (the library's last-error string is per thread)
 };
 
@@ -260,6 +274,84 @@ int same_multi_drain_events(same_multi* m, same_event* events, size_t events_cap
     if (r != SAME_OK) return r;
     for (size_t k = 0; k < a; ++k) { dst[k].stream += s.first; dst[k].data_offset += (uint32_t)pay_base[i]; }
     return (int)SAME_OK;
+  });
+}
+
+// ---- portable stream state with global ids ----
+size_t same_multi_state_bytes(const same_multi* m, uint32_t n) {
+  return m ? same_state_header_bytes() + (size_t)n * same_state_engine_record_bytes(m->shards[0]->eng) : 0;
+}
+
+// ids -> each shard's local ids and positions in `ids`; false on an id out of range (or a duplicate, if unique)
+static bool split_ids(same_multi* m, const uint32_t* ids, uint32_t n, bool unique) {
+  for (Shard* s : m->shards) { s->st_ids.clear(); s->st_pos.clear(); }
+  std::vector<char> seen(unique ? m->n_streams : 0, 0);
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint32_t g = ids ? ids[i] : i;
+    if (g >= m->n_streams) { mfail(m, SAME_ERR_INVALID_ARG, "stream id " + std::to_string(g) + " out of range"); return false; }
+    if (unique) {
+      if (seen[g]) { mfail(m, SAME_ERR_INVALID_ARG, "duplicate target stream id " + std::to_string(g)); return false; }
+      seen[g] = 1;
+    }
+    size_t k = 0;
+    while (g >= m->shards[k]->first + m->shards[k]->count) ++k;
+    m->shards[k]->st_ids.push_back(g - m->shards[k]->first);
+    m->shards[k]->st_pos.push_back(i);
+  }
+  return true;
+}
+
+int same_multi_export_streams(same_multi* m, const uint32_t* ids, uint32_t n, void* buf, size_t cap, size_t* written) {
+  if (!m) return mfail(nullptr, SAME_ERR_INVALID_ARG, "null handle");
+  if (!ids) n = m->n_streams;
+  if (!split_ids(m, ids, n, false)) return SAME_ERR_INVALID_ARG;
+  const size_t need = same_multi_state_bytes(m, n);
+  if (written) *written = need;
+  if (!buf || cap < need) return mfail(m, SAME_ERR_INVALID_ARG, "export buffer too small: " + std::to_string(need) + " bytes needed");
+  const size_t hdr = same_state_header_bytes(), rec = same_state_engine_record_bytes(m->shards[0]->eng);
+  same_state_write_header(m->shards[0]->eng, n, buf);
+  uint8_t* out = static_cast<uint8_t*>(buf) + hdr;
+  return run_all(m, [=](Shard& s) {
+    const uint32_t k = (uint32_t)s.st_ids.size();
+    if (k == 0) return (int)SAME_OK;
+    // records of a run of consecutive positions go straight to their place in the caller's buffer
+    const bool in_place = s.st_pos.back() - s.st_pos.front() + 1u == k;
+    uint8_t* dst = out + (size_t)s.st_pos.front() * rec;
+    if (!in_place) { s.st_buf.resize((size_t)k * rec); dst = s.st_buf.data(); }
+    const int r = same_state_export_records(s.eng, s.st_ids.data(), k, s.first, dst);
+    if (r != SAME_OK || in_place) return r;
+    for (uint32_t j = 0; j < k; ++j) memcpy(out + (size_t)s.st_pos[j] * rec, s.st_buf.data() + (size_t)j * rec, rec);
+    return (int)SAME_OK;
+  });
+}
+
+int same_multi_import_streams(same_multi* m, const uint32_t* ids, uint32_t n, const void* buf, size_t len) {
+  if (!m) return mfail(nullptr, SAME_ERR_INVALID_ARG, "null handle");
+  uint32_t n_records = 0;
+  same_engine* e0 = m->shards[0]->eng;
+  int rc = same_state_check_header(e0, buf, len, &n_records);   // every shard has the same configuration
+  if (rc != SAME_OK) return mfail(m, rc, same_engine_last_error(e0));
+  if (!ids && n != m->n_streams) return mfail(m, SAME_ERR_INVALID_ARG, "ids == NULL imports into every stream: n must equal the number of streams");
+  if (n != n_records) return mfail(m, SAME_ERR_INVALID_ARG, "n = " + std::to_string(n) + " but the buffer holds " + std::to_string(n_records) + " records");
+  if (!split_ids(m, ids, n, true)) return SAME_ERR_INVALID_ARG;
+  const size_t hdr = same_state_header_bytes(), rec = same_state_engine_record_bytes(e0);
+  const uint8_t* in = static_cast<const uint8_t*>(buf) + hdr;
+  // every shard stages and validates its records; only if all of them passed does any shard write its streams
+  rc = run_all(m, [=](Shard& s) {
+    const uint32_t k = (uint32_t)s.st_ids.size();
+    if (k == 0) return (int)SAME_OK;
+    const uint8_t* src = in + (size_t)s.st_pos.front() * rec;
+    if (s.st_pos.back() - s.st_pos.front() + 1u != k) {
+      s.st_buf.resize((size_t)k * rec);
+      for (uint32_t j = 0; j < k; ++j) memcpy(s.st_buf.data() + (size_t)j * rec, in + (size_t)s.st_pos[j] * rec, rec);
+      src = s.st_buf.data();
+    }
+    return same_state_import_stage(s.eng, k, src, &s.st_flags);
+  });
+  if (rc != SAME_OK) return rc;
+  return run_all(m, [](Shard& s) {
+    const uint32_t k = (uint32_t)s.st_ids.size();
+    return k ? same_state_import_commit(s.eng, s.st_ids.data(), k, s.st_flags) : (int)SAME_OK;
   });
 }
 

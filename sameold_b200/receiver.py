@@ -572,6 +572,67 @@ class SameBatchReceiver:
     def free_snapshot(self, snap):
         self._lib.same_snapshot_free(snap)
 
+    # -- portable stream state (format: include/same_engine.h) --
+    def export_streams(self, ids: Optional[Sequence[int]] = None) -> bytes:
+        """The complete receiver state of streams `ids` (None: all, in order) as a self-describing buffer that any
+        engine with the same configuration can import, on any device or in another process.  Changes nothing."""
+        return _export(self._lib, self._lib.same_engine_state_bytes, self._lib.same_engine_export_streams, self._h, ids,
+                       self.n_streams, self._ck)
+
+    def import_streams(self, data, ids: Optional[Sequence[int]] = None):
+        """Record i -> stream ids[i] (None: record i -> stream i).  Like reset(ids) followed by writing the recorded
+        state; all or nothing."""
+        _import(self._lib.same_engine_import_streams, self._h, data, ids, self._ck)
+
+    @classmethod
+    def from_state(cls, data, device: int = 0) -> "SameBatchReceiver":
+        """A new engine built from the configuration embedded in `data`, holding every record of it."""
+        cfg, n = state_info(data)
+        rx = cls(cfg, n, device)
+        rx.import_streams(data)
+        return rx
+
+
+def _buffer(data) -> np.ndarray:
+    """bytes / bytearray / memoryview / uint8 array -> a uint8 view (no copy)."""
+    return np.frombuffer(data, dtype=np.uint8) if not isinstance(data, np.ndarray) else data.reshape(-1).view(np.uint8)
+
+
+def _ids(ids):
+    if ids is None:
+        return None, None
+    a = np.ascontiguousarray(ids, dtype=np.uint32).reshape(-1)
+    return a, a.ctypes.data
+
+
+def _export(lib, state_bytes, export, h, ids, n_streams, ck) -> bytes:
+    a, p = _ids(ids)
+    n = n_streams if a is None else a.size
+    out = bytearray(state_bytes(h, n))
+    written = C.c_size_t()
+    cbuf = (C.c_char * len(out)).from_buffer(out)
+    ck(export(h, p, n, C.addressof(cbuf), len(out), C.byref(written)))
+    del cbuf
+    return bytes(out)
+
+
+def _import(imp, h, data, ids, ck):
+    buf = _buffer(data)
+    a, p = _ids(ids)
+    n = state_info(buf)[1] if a is None else a.size
+    ck(imp(h, p, n, buf.ctypes.data, buf.size))
+
+
+def state_info(data) -> "tuple[_lib.SameConfig, int]":
+    """(configuration, number of records) of an export buffer: header checks only, no GPU needed."""
+    lib = _lib.load()
+    buf = _buffer(data)
+    cfg, n = _lib.SameConfig(), C.c_uint32()
+    rc = lib.same_state_info(buf.ctypes.data if buf.size else None, buf.size, C.byref(cfg), C.byref(n))
+    if rc != 0:
+        raise SameEngineError(rc, lib.same_last_error().decode())
+    return cfg, n.value
+
 
 # ---------------------------------------------------------------------------------------------------------------------
 # One batch over several GPUs of a box, inside one process (same_multi_* in include/same_engine.h)
@@ -670,6 +731,15 @@ class SameMultiReceiver:
         self.sync()
         return self.drain_by_stream()
 
+    def export_streams(self, ids: Optional[Sequence[int]] = None) -> bytes:
+        """SameBatchReceiver.export_streams with global stream ids; records come out in the order of `ids`."""
+        return _export(self._lib, self._lib.same_multi_state_bytes, self._lib.same_multi_export_streams, self._h, ids,
+                       self.n_streams, self._ck)
+
+    def import_streams(self, data, ids: Optional[Sequence[int]] = None):
+        """SameBatchReceiver.import_streams with global stream ids: validated on every shard before any shard changes."""
+        _import(self._lib.same_multi_import_streams, self._h, data, ids, self._ck)
+
     def iter_messages_batched(self, chunks) -> Iterator["tuple[int, Message]"]:
         """== iter_messages (receiver.rs:155-161) for every stream of the whole box: yields (stream, Message)."""
         for evs in self.process(chunks):
@@ -702,6 +772,15 @@ class SameReceiver:
 
     def reset(self):
         self._b.reset()
+
+    def export_state(self) -> bytes:
+        """This receiver's complete state as a portable buffer (SameBatchReceiver.export_streams)."""
+        return self._b.export_streams()
+
+    def clone(self, device: Optional[int] = None) -> "SameReceiver":
+        """== `SameReceiver: Clone` (receiver.rs:70): a new receiver on `device` (default: this one's) in the same
+        state; the two share nothing afterwards."""
+        return SameReceiver(SameBatchReceiver.from_state(self.export_state(), self._b.device if device is None else device))
 
     def _blocks(self, source) -> Iterator[np.ndarray]:
         """int16 arrays (and iterables of Python ints) go in as s16 PCM — what samedec feeds (`sa as f32`, app.rs:112);
