@@ -13,7 +13,7 @@ CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_build")
 LIB = os.path.join(OUT_DIR, "libsame_b200.so")
 SOURCES = ["same_kernels.cu", "same_long.cu", "same_engine.cu", "same_multi.cu", "same_synth.cu", "same_state.cu"]
-HEADERS = ["same_params.h", "same_transport.cuh", "same_lane.cuh", "same_fast.cuh", os.path.join("..", "..", "include", "same_engine.h"),
+HEADERS = ["same_params.h", "same_internal.h", "same_transport.cuh", "same_lane.cuh", "same_fast.cuh", os.path.join("..", "..", "include", "same_engine.h"),
            os.path.join("..", "..", "include", "same_synth.h")]
 
 NVCC_FLAGS = [

@@ -11,39 +11,12 @@
 #include <cstdio>
 #include <cstring>
 #include <cstdlib>
+#include <memory>
 #include <string>
+#include <utility>
 #include <vector>
 
-#include "same_params.h"
-
-extern "C" cudaError_t same_launch_rx(const SameParams* p, const SameTaps* taps, const SameTaps2* taps2, int force_generic,
-                                      uint32_t lanes_per_warp, const void* d_samples, int sample_fmt,
-                                      const unsigned long long* d_offsets, const uint32_t* d_lengths,
-                                      const SameTiles* tiles, cudaStream_t stream);
-extern "C" cudaError_t same_launch_frontend(const SameParams* p, const int16_t* d_samples, const unsigned long long* d_offsets,
-                                            const uint32_t* d_lengths, const SameTiles* tiles, cudaStream_t stream);
-extern "C" cudaError_t same_launch_rx_tilefed(const SameParams* p, const SameTaps2* taps2, const uint32_t* d_lengths,
-                                              const SameTiles* tiles, cudaStream_t stream);
-extern "C" cudaError_t same_long_launch_dc(const SameParams* p, const int16_t* d_src, uint32_t len, float* d, uint32_t* dc_next,
-                                           cudaStream_t stream);
-extern "C" cudaError_t same_long_launch_commit_dc(const SameParams* p, const uint32_t* dc_next, cudaStream_t stream);
-extern "C" cudaError_t same_long_launch_speculative(const SameParams* p, const SameTaps2* taps2, const float* d, uint32_t pos0,
-                                                    uint32_t end, float* yfull, float* gspec, float* g_in, float* soft,
-                                                    uint32_t* ctrl, cudaStream_t stream);
-extern "C" cudaError_t same_launch_evsort(const same_event* d_events, uint32_t n, uint32_t n_streams, uint32_t* d_cnt,
-                                          uint32_t* d_minseq, uint32_t* d_start, same_event* d_sorted, uint32_t* d_bad,
-                                          cudaStream_t stream);
-extern "C" cudaError_t same_launch_init(const SameParams* p, const uint32_t* d_ids, uint32_t n, int after_reset,
-                                        cudaStream_t stream);
-// same_state.cu
-extern "C" uint32_t same_state_record_bytes(uint32_t n_words);
-extern "C" uint32_t same_state_crc32(const void* data, size_t n);
-extern "C" cudaError_t same_state_launch_gather(const SameParams* p, const uint32_t* d_ids, uint32_t first, uint32_t n,
-                                                uint32_t id_base, uint32_t rec_flags, uint8_t* d_out, cudaStream_t stream);
-extern "C" cudaError_t same_state_launch_validate(const uint8_t* d_in, uint32_t n, uint32_t n_words, unsigned long long* d_result,
-                                                  cudaStream_t stream);
-extern "C" cudaError_t same_state_launch_scatter(const SameParams* p, const uint32_t* d_ids, uint32_t first, uint32_t n,
-                                                 const uint8_t* d_in, cudaStream_t stream);
+#include "same_internal.h"
 
 namespace {
 
@@ -82,66 +55,124 @@ size_t f32_as_usize(float x) {  // `as usize`: truncating, saturating, NaN -> 0
   return (size_t)x;
 }
 
+// ---- owned CUDA resources: released when their owner goes, on the device that is current then ----
+
+// An array of T from Alloc, released with Free.  grow() allocates before it releases: a failed allocation leaves the
+// old array in place and clears the runtime's last error, so that the next launcher does not report it as its own.
+template <class T, cudaError_t (*Alloc)(void**, size_t), cudaError_t (*Free)(void*)>
+class Buf {
+ public:
+  Buf() = default;
+  Buf(const Buf&) = delete;
+  Buf& operator=(const Buf&) = delete;
+  ~Buf() { if (p_) Free(p_); }
+  operator T*() const { return p_; }
+  size_t size() const { return n_; }   // elements
+  // room for at least n elements (when it has to grow: n + slack); the contents are not kept
+  cudaError_t grow(size_t n, size_t slack = 0) {
+    if (n <= n_) return cudaSuccess;
+    void* q = nullptr;
+    const cudaError_t err = Alloc(&q, (n + slack) * sizeof(T));
+    if (err != cudaSuccess) { cudaGetLastError(); return err; }
+    if (p_) Free(p_);
+    p_ = static_cast<T*>(q); n_ = n + slack;
+    return cudaSuccess;
+  }
+  void swap(Buf& o) { std::swap(p_, o.p_); std::swap(n_, o.n_); }
+
+ private:
+  T* p_ = nullptr;
+  size_t n_ = 0;
+};
+template <class T> using DevBuf = Buf<T, cudaMalloc, cudaFree>;
+template <class T> using PinnedBuf = Buf<T, cudaMallocHost, cudaFreeHost>;
+
+class Event {
+ public:
+  Event() = default;
+  Event(const Event&) = delete;
+  Event& operator=(const Event&) = delete;
+  ~Event() { if (ev_) cudaEventDestroy(ev_); }
+  cudaError_t create(unsigned flags = cudaEventDefault) { return cudaEventCreateWithFlags(&ev_, flags); }
+  operator cudaEvent_t() const { return ev_; }
+
+ private:
+  cudaEvent_t ev_ = nullptr;
+};
+
+class Stream {
+ public:
+  Stream() = default;
+  Stream(const Stream&) = delete;
+  Stream& operator=(const Stream&) = delete;
+  ~Stream() { if (st_) cudaStreamDestroy(st_); }
+  cudaError_t create() { return cudaStreamCreateWithFlags(&st_, cudaStreamNonBlocking); }
+  operator cudaStream_t() const { return st_; }
+
+ private:
+  cudaStream_t st_ = nullptr;
+};
+
 struct InputBuf {
-  uint8_t* d = nullptr; size_t cap = 0;          // device samples (s16 or f32), capacity in bytes
-  unsigned long long* d_off = nullptr; uint32_t* d_len = nullptr;
-  cudaEvent_t copied = nullptr, consumed = nullptr;
+  DevBuf<uint8_t> d;                     // device samples (s16 or f32)
+  DevBuf<unsigned long long> d_off;
+  DevBuf<uint32_t> d_len;
+  Event copied, consumed;
   bool used = false;
 };
 
 }  // namespace
 
 struct same_engine {
+  Stream compute, copy;   // declared first, so destroyed last
   same_config cfg;
   int device = 0;
   uint32_t n_streams = 0;
-  SameParams p;
+  SameParams p;           // its pointers into the buffers below are set by bind()
   SameTaps taps;
   SameTaps2 taps2;
-  int force_generic = 0;
+  Kernel kernel_override = POLICY;   // option "kernel"
   uint32_t lanes_per_warp = 32;   // streams per warp in the fast kernel (lane-sparse warps for small batches)
   int sm_count = 148;
-  int kernel_auto = 0;            // fast-kernel flavour when force_generic == 0: 3 pipelined, 4 three-warp, 2 single-warp, 6 look-ahead
-  SameTiles tiles{nullptr, nullptr, 0u, 32u, 1u};   // split pipeline (kernel 5): front-end output, allocated on first use
-  size_t tiles_cap = 0;           // floats
+  // split pipeline (kernel 5): front-end output, allocated on first use
+  SameTiles tiles{nullptr, nullptr, 0u, 32u, 1u};
+  DevBuf<float> tiles_d;
+  DevBuf<uint32_t> tiles_dc_next;
   // long-stream path (same_long.cu): one stream, long chunks
   int long_stream = 1;            // option "long_stream"
-  float *ls_d = nullptr, *ls_y = nullptr, *ls_g = nullptr, *ls_soft = nullptr, *ls_gin = nullptr;
-  uint32_t* ls_ctrl = nullptr;    // device: {verified end, position reached, reason, -}
-  uint32_t* ls_hctrl = nullptr;   // pinned mirror + scratch
-  size_t ls_cap = 0;              // samples
+  DevBuf<float> ls_d, ls_y, ls_g, ls_soft, ls_gin;
+  DevBuf<uint32_t> ls_ctrl;       // {verified end, position reached, reason, -}
+  PinnedBuf<uint32_t> ls_hctrl;   // mirror + scratch
   uint64_t ls_spec_launches = 0, ls_fallback_launches = 0;
   bool saw_f32 = false;           // an f32 submit happened since create / reset(all): DC state may be non-integer -> generic kernel
   uint64_t lost_events = 0, lost_payloads = 0;
   same_derived derived;
-  cudaStream_t compute = nullptr, copy = nullptr;
-  uint32_t* d_state = nullptr;
-  StreamBlob* d_blobs = nullptr;
-  same_event* d_events = nullptr;
-  same_event* d_sorted = nullptr;        // arena events counting-sorted by (stream, seq) before read-back
-  uint32_t* d_sort_ws = nullptr;         // cnt[n+1] | start[n+1] | minseq[n] | bad[1]
+  DevBuf<uint32_t> d_state;
+  DevBuf<StreamBlob> d_blobs;
+  DevBuf<same_event> d_events;
+  DevBuf<same_event> d_sorted;           // arena events counting-sorted by (stream, seq) before read-back
+  DevBuf<uint32_t> d_sort_ws;            // cnt[n+1] | start[n+1] | minseq[n] | bad[1]
   bool pend_sorted = false;              // pend_events is one device-sorted batch: drain copies it as it is
   int device_sort = 1;                   // option "device_sort": 0 = always sort on the host (diagnostic)
-  uint8_t* d_payload = nullptr;
-  unsigned int* d_counters = nullptr;
-  unsigned int* h_counters = nullptr;   // pinned
-  uint8_t* h_stage = nullptr;           // pinned staging for event / payload read-back (STAGE_BYTES, used as two halves)
-  cudaEvent_t stage_done[2] = {nullptr, nullptr};
-  same_soft_symbol* d_trace = nullptr;
-  uint32_t* d_ids = nullptr; size_t ids_cap = 0;
+  DevBuf<uint8_t> d_payload;
+  DevBuf<unsigned int> d_counters;
+  PinnedBuf<unsigned int> h_counters;
+  PinnedBuf<uint8_t> h_stage;            // staging for device <-> pageable host copies (STAGE_BYTES, used as two halves)
+  Event stage_done[2];
+  DevBuf<same_soft_symbol> d_trace;      // n_streams x trace_cap symbols
+  DevBuf<uint32_t> d_ids;
   InputBuf in[2];
   int cur = 0;
   bool in_flight = false;
-  size_t events_cap = 0, payload_cap = 0;
   std::vector<same_event> pend_events;
   std::vector<uint8_t> pend_payload;
-  cudaEvent_t t_h2d0 = nullptr, t_h2d1 = nullptr, t_k0 = nullptr, t_k1 = nullptr, t_sw0 = nullptr, t_sw1 = nullptr;
+  Event t_h2d0, t_h2d1, t_k0, t_k1, t_sw0, t_sw1;
   bool timed_h2d = false, timed_kernel = false;
   // portable stream state (same_state.cu): device staging of records, ids, validation result, timing of the last call
-  uint8_t* d_xfer = nullptr; size_t xfer_cap = 0;
-  uint32_t* d_xids = nullptr; size_t xids_cap = 0;
-  unsigned long long* d_xres = nullptr;
-  cudaEvent_t t_st[3] = {nullptr, nullptr, nullptr};
+  DevBuf<uint8_t> d_xfer;
+  DevBuf<uint32_t> d_xids;
+  DevBuf<unsigned long long> d_xres;
+  Event t_st[3];
   float st_kernel_ms = 0.0f, st_copy_ms = 0.0f;
   uint64_t launches = 0;
   std::string last_error;
@@ -162,43 +193,72 @@ int fail(same_engine* e, int code, const std::string& msg) {
       return fail((e), SAME_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(_err));            \
   } while (0)
 
+// The kernel parameters that point into the engine's buffers, set from their owners after any of them changed
+void bind(same_engine* e) {
+  SameParams& p = e->p;
+  p.state32 = e->d_state; p.blobs = e->d_blobs; p.counters = e->d_counters;
+  p.events = e->d_events; p.payload = e->d_payload;
+  p.events_cap = (uint32_t)std::min<size_t>(e->d_events.size(), 0xffffffffu);
+  p.payload_cap = (uint32_t)std::min<size_t>(e->d_payload.size(), 0xffffffffu);
+  p.trace = e->d_trace; p.trace_cap = (uint32_t)(e->d_trace.size() / e->n_streams);
+  e->tiles.d = e->tiles_d; e->tiles.dc_next = e->tiles_dc_next;
+}
+
+// Event arenas of exactly these sizes; the old ones stay in use unless all of the new ones could be allocated
 int alloc_arenas(same_engine* e, size_t max_events, size_t max_payload) {
-  if (e->d_events) cudaFree(e->d_events);
-  if (e->d_sorted) cudaFree(e->d_sorted);
-  if (e->d_payload) cudaFree(e->d_payload);
-  e->d_events = nullptr; e->d_sorted = nullptr; e->d_payload = nullptr;
-  CK(e, cudaMalloc(&e->d_events, max_events * sizeof(same_event)));
-  CK(e, cudaMalloc(&e->d_sorted, max_events * sizeof(same_event)));
-  if (!e->d_sort_ws) CK(e, cudaMalloc(&e->d_sort_ws, (3 * (size_t)e->n_streams + 3) * sizeof(uint32_t)));
-  CK(e, cudaMalloc(&e->d_payload, max_payload));
-  e->events_cap = max_events; e->payload_cap = max_payload;
-  e->p.events = e->d_events; e->p.payload = e->d_payload;
-  e->p.events_cap = (uint32_t)std::min<size_t>(max_events, 0xffffffffu);
-  e->p.payload_cap = (uint32_t)std::min<size_t>(max_payload, 0xffffffffu);
+  DevBuf<same_event> events, sorted;
+  DevBuf<uint8_t> payload;
+  CK(e, events.grow(max_events));
+  CK(e, sorted.grow(max_events));
+  CK(e, payload.grow(max_payload));
+  e->d_events.swap(events); e->d_sorted.swap(sorted); e->d_payload.swap(payload);
+  bind(e);
   return SAME_OK;
 }
 
 static const size_t STAGE_BYTES = 2 * 48 * 32768;   // two halves of 32768 events (1.5 MiB each)
+
+// device -> pinned staging -> take(slice, n) for each slice in order: two halves, so that the copy of one slice overlaps
+// the host's use of the other
+template <class Take>
+int stage_out(same_engine* e, const uint8_t* src, size_t bytes, Take&& take) {
+  const size_t half = STAGE_BYTES / 2;
+  size_t done = 0, queued = 0, qn[2] = {0, 0};
+  int qslot = 0, pslot = 0, inflight = 0;
+  while (done < bytes) {
+    while (inflight < 2 && queued < bytes) {   // keep both halves in flight
+      const size_t n = std::min(half, bytes - queued);
+      CK(e, cudaMemcpyAsync(e->h_stage + qslot * half, src + queued, n, cudaMemcpyDeviceToHost, e->compute));
+      CK(e, cudaEventRecord(e->stage_done[qslot], e->compute));
+      qn[qslot] = n; queued += n; qslot ^= 1; ++inflight;
+    }
+    CK(e, cudaEventSynchronize(e->stage_done[pslot]));
+    take(e->h_stage + pslot * half, qn[pslot]);
+    done += qn[pslot]; pslot ^= 1; --inflight;
+  }
+  return SAME_OK;
+}
 
 // Pull the events produced since the last collect from the device arenas into the host pending lists.
 int collect(same_engine* e) {
   CK(e, cudaMemcpyAsync(e->h_counters, e->d_counters, 4 * sizeof(unsigned int), cudaMemcpyDeviceToHost, e->compute));
   CK(e, cudaStreamSynchronize(e->compute));
   const size_t nev = e->h_counters[0], npay = e->h_counters[1];
+  const size_t events_cap = e->d_events.size(), payload_cap = e->d_payload.size();
   int rc = SAME_OK;
-  if (nev > e->events_cap || e->h_counters[2] != 0) {
+  if (nev > events_cap || e->h_counters[2] != 0) {
     // Events beyond the arena were dropped by the device; events whose payload did not fit were stored with
     // data_len 0 + SAME_EV_FLAG_PAYLOAD_LOST (same_transport.cuh:emit_event_impl), so everything handed to the caller
     // below stays self-consistent.  The stream state has advanced: what was dropped is lost, and counted.
-    const uint64_t ev_lost = nev > e->events_cap ? nev - e->events_cap : 0;
+    const uint64_t ev_lost = nev > events_cap ? nev - events_cap : 0;
     e->lost_events += ev_lost;
     e->lost_payloads += e->h_counters[2];
     char buf[256];
     snprintf(buf, sizeof buf, "event arena overflow since the last sync: %llu events dropped (capacity %zu), %u payloads dropped "
-             "(capacity %zu bytes)", (unsigned long long)ev_lost, e->events_cap, e->h_counters[2], e->payload_cap);
+             "(capacity %zu bytes)", (unsigned long long)ev_lost, events_cap, e->h_counters[2], payload_cap);
     rc = fail(e, SAME_ERR_EVENT_OVERFLOW, buf);
   }
-  const size_t cev = std::min(nev, e->events_cap), cpay = std::min(npay, e->payload_cap);
+  const size_t cev = std::min(nev, events_cap), cpay = std::min(npay, payload_cap);
   // big single batches are put into (stream, occurrence) order on the device; the host sort in drain is the fallback
   const same_event* ev_src = e->d_events;
   bool dev_sorted = false;
@@ -215,34 +275,17 @@ int collect(same_engine* e) {
   }
   e->pend_sorted = dev_sorted || (cev == 0 && e->pend_sorted);
   if (cev) {
-    // device -> pinned staging (two halves, so the copy of one slice overlaps the append of the other) -> pending lists
+    // appended slice by slice: the staging halves hold whole events
     const size_t base_ev = e->pend_events.size(), base_pay = e->pend_payload.size();
     e->pend_events.reserve(base_ev + cev);
     e->pend_payload.reserve(base_pay + cpay);
-    const size_t half = STAGE_BYTES / 2;
-    const uint8_t* src[2] = {reinterpret_cast<const uint8_t*>(ev_src), e->d_payload};
-    const size_t bytes[2] = {cev * sizeof(same_event), cpay};
-    for (int part = 0; part < 2; ++part) {
-      size_t done = 0, queued = 0, qn[2] = {0, 0};
-      int qslot = 0, pslot = 0, inflight = 0;
-      while (done < bytes[part]) {
-        while (inflight < 2 && queued < bytes[part]) {   // keep both halves in flight
-          const size_t n = std::min(half, bytes[part] - queued);
-          CK(e, cudaMemcpyAsync(e->h_stage + qslot * half, src[part] + queued, n, cudaMemcpyDeviceToHost, e->compute));
-          CK(e, cudaEventRecord(e->stage_done[qslot], e->compute));
-          qn[qslot] = n; queued += n; qslot ^= 1; ++inflight;
-        }
-        CK(e, cudaEventSynchronize(e->stage_done[pslot]));
-        const uint8_t* h = e->h_stage + pslot * half;
-        if (part == 0) {
-          const same_event* ev = reinterpret_cast<const same_event*>(h);
-          e->pend_events.insert(e->pend_events.end(), ev, ev + qn[pslot] / sizeof(same_event));
-        } else {
-          e->pend_payload.insert(e->pend_payload.end(), h, h + qn[pslot]);
-        }
-        done += qn[pslot]; pslot ^= 1; --inflight;
-      }
-    }
+    int r = stage_out(e, reinterpret_cast<const uint8_t*>(ev_src), cev * sizeof(same_event), [e](const uint8_t* h, size_t n) {
+      const same_event* ev = reinterpret_cast<const same_event*>(h);
+      e->pend_events.insert(e->pend_events.end(), ev, ev + n / sizeof(same_event));
+    });
+    if (r) return r;
+    r = stage_out(e, e->d_payload, cpay, [e](const uint8_t* h, size_t n) { e->pend_payload.insert(e->pend_payload.end(), h, h + n); });
+    if (r) return r;
     for (size_t i = base_ev; i < base_ev + cev; ++i) {
       same_event& ev = e->pend_events[i];
       const uint32_t stored = ev.kind == SAME_EV_LINK_BURST ? std::min<uint32_t>(ev.data_len, SAME_BURST_CAP) : ev.data_len;
@@ -256,29 +299,22 @@ int collect(same_engine* e) {
   return rc;
 }
 
-int ensure_input(same_engine* e, InputBuf& b, size_t bytes) {
-  if (bytes > b.cap) {
-    if (b.d) CK(e, cudaFree(b.d));
-    b.d = nullptr; b.cap = 0;
-    size_t cap = bytes + bytes / 8 + 8192;
-    CK(e, cudaMalloc(&b.d, cap));
-    b.cap = cap;
-  }
-  return SAME_OK;
+// Drop the undrained events of streams ids[0..n) (nullptr: 0..n-1); their payload bytes stay until the next drain
+void forget_events(same_engine* e, const uint32_t* ids, uint32_t n) {
+  std::vector<char> hit(e->n_streams, 0);
+  for (uint32_t i = 0; i < n; ++i) hit[ids ? ids[i] : i] = 1;
+  e->pend_events.erase(std::remove_if(e->pend_events.begin(), e->pend_events.end(),
+                                      [&](const same_event& ev) { return hit[ev.stream] != 0; }),
+                       e->pend_events.end());
 }
 
 // Tile buffer of the split pipeline: n_pad streams x n_max samples of f32 (+ the 34-word DC state per stream).
 int ensure_tiles(same_engine* e, uint32_t max_len) {
   const uint32_t n_max = (max_len + 31u) & ~31u;
-  const size_t need = (size_t)e->p.layout.n_pad * n_max;
-  if (need > e->tiles_cap) {
-    if (e->tiles.d) CK(e, cudaFree(e->tiles.d));
-    e->tiles.d = nullptr; e->tiles_cap = 0;
-    CK(e, cudaMalloc(&e->tiles.d, need * sizeof(float)));
-    e->tiles_cap = need;
-  }
-  if (!e->tiles.dc_next) CK(e, cudaMalloc(&e->tiles.dc_next, (size_t)34 * e->p.layout.n_pad * sizeof(uint32_t)));
+  CK(e, e->tiles_d.grow((size_t)e->p.layout.n_pad * n_max));
+  CK(e, e->tiles_dc_next.grow((size_t)34 * e->p.layout.n_pad));
   e->tiles.n_max = n_max;
+  bind(e);
   return SAME_OK;
 }
 
@@ -288,19 +324,15 @@ constexpr uint32_t kLongChunk = 1u << 24;       // samples per internal pass (bo
 constexpr uint32_t kLongSpan = 8192;            // samples per fallback launch while the AGC is locked (inside a burst)
 
 int ensure_long(same_engine* e, size_t n) {
-  if (n > e->ls_cap) {
-    for (float** q : {&e->ls_d, &e->ls_y, &e->ls_g, &e->ls_soft, &e->ls_gin}) { if (*q) CK(e, cudaFree(*q)); *q = nullptr; }
-    e->ls_cap = 0;
-    CK(e, cudaMalloc(&e->ls_d, (n + 64) * sizeof(float)));
-    CK(e, cudaMalloc(&e->ls_y, (n + 128) * sizeof(float)));
-    CK(e, cudaMalloc(&e->ls_g, (n + 64) * sizeof(float)));
-    CK(e, cudaMalloc(&e->ls_soft, (n + 2 * 4096 + 64) * sizeof(float)));   // + two tiles: the sequential kernel stages ahead
-    CK(e, cudaMalloc(&e->ls_gin, (n / 2048 + 8) * sizeof(float)));
-    e->ls_cap = n;
-  }
-  if (!e->ls_ctrl) CK(e, cudaMalloc(&e->ls_ctrl, 4 * sizeof(uint32_t)));
-  if (!e->ls_hctrl) CK(e, cudaHostAlloc(&e->ls_hctrl, 8 * sizeof(uint32_t), cudaHostAllocDefault));
-  if (!e->tiles.dc_next) CK(e, cudaMalloc(&e->tiles.dc_next, (size_t)34 * e->p.layout.n_pad * sizeof(uint32_t)));
+  CK(e, e->ls_d.grow(n + 64));
+  CK(e, e->ls_y.grow(n + 128));
+  CK(e, e->ls_g.grow(n + 64));
+  CK(e, e->ls_soft.grow(n + 2 * 4096 + 64));   // + two tiles: the sequential kernel stages ahead
+  CK(e, e->ls_gin.grow(n / 2048 + 8));
+  CK(e, e->ls_ctrl.grow(4));
+  CK(e, e->ls_hctrl.grow(8));
+  CK(e, e->tiles_dc_next.grow((size_t)34 * e->p.layout.n_pad));
+  bind(e);
   return SAME_OK;
 }
 
@@ -311,7 +343,7 @@ int run_long(same_engine* e, const int16_t* d_src, uint32_t len) {
     const uint32_t n = std::min(kLongChunk, len - base);
     int rc = ensure_long(e, n);
     if (rc) return rc;
-    CK(e, same_long_launch_dc(&e->p, d_src + base, n, e->ls_d, e->tiles.dc_next, e->compute));
+    CK(e, same_long_launch_dc(&e->p, d_src + base, n, e->ls_d, e->tiles_dc_next, e->compute));
     e->launches += 1;
     uint32_t pos = 0;
     while (pos < n) {
@@ -322,7 +354,7 @@ int run_long(same_engine* e, const int16_t* d_src, uint32_t len) {
         const uint32_t span = std::min(kLongSpan, n - pos);
         e->ls_hctrl[5] = span;
         CK(e, cudaMemcpyAsync(e->ls_ctrl + 3, e->ls_hctrl + 5, sizeof(uint32_t), cudaMemcpyHostToDevice, e->compute));
-        SameTiles t{e->ls_d + pos, e->tiles.dc_next, span, 1u, 0u};
+        SameTiles t{e->ls_d + pos, e->tiles_dc_next, span, 1u, 0u};
         CK(e, same_launch_rx_tilefed(&e->p, &e->taps2, e->ls_ctrl + 3, &t, e->compute));
         e->launches += 1; e->ls_fallback_launches += 1;
         pos += span;
@@ -338,10 +370,34 @@ int run_long(same_engine* e, const int16_t* d_src, uint32_t len) {
       if (reached == pos && e->ls_hctrl[2] == 0u) return fail(e, SAME_ERR_CUDA, "long-stream pass made no progress");
       pos = reached;
     }
-    CK(e, same_long_launch_commit_dc(&e->p, e->tiles.dc_next, e->compute));
+    CK(e, same_long_launch_commit_dc(&e->p, e->tiles_dc_next, e->compute));
     e->launches += 1;
   }
   return SAME_OK;
+}
+
+// The receiver kernel an s16 submit launches:
+//  * the generic kernel once f32 input reached the state (saw_f32): the DC-blocker state may hold non-integers, and
+//    the fast kernels' DC blocker is an integer recursion;
+//  * the generic kernel for any geometry but the 22050 Hz class (42 taps, DC length 16), the fast kernels' only one;
+//  * option "kernel";
+//  * else the policy for the 22050 Hz class (measured on B200, tables in profiles/README.md), by 32-stream blocks per SM:
+//    * <= 1: four-warp pipelined kernel (producer / AGC / space filter / consumer), every warp on its own scheduler:
+//      the per-stream dependent chain is what bounds the run time, so it is cut into stages.
+//    * <= 4: three-warp kernel (producer / look-ahead AGC / consumer): fewer instructions in total, still
+//      latency-hiding across the co-resident blocks.
+//    * <= 8: single-warp fast kernel (8 resident blocks per SM: the whole batch is one wave; fewest instructions).
+//    * more: single-warp look-ahead kernel (16 resident warps per SM, no d ring): the issue-bound regime.
+//    20 s streams, ms per launch, pipelined / three-warp / single-warp / look-ahead: 4096 streams 24.0 / 24.9 / 41.6 / -;
+//    8192: 36.8 / 29.1 / 43.3 / 66; 16384: 74.6 / 40.0 / 43.9 / 70; 32768: - / - / 57.7 / 81; 49152: - / - / 109 / 83;
+//    65536: 228 / 158 / 116 / 97.
+// Option "lanes_per_warp" spreads streams over more, lane-sparse warps (diagnostic).  No environment variable is read
+// here: same_engine_set_option is the only override.
+Kernel rx_kernel(const same_engine* e) {
+  if (e->saw_f32 || e->p.ntaps != 42 || e->p.dc_len != 16) return GENERIC;
+  if (e->kernel_override != POLICY) return e->kernel_override;
+  const uint32_t blocks32 = (e->n_streams + 31u) / 32u, sms = (uint32_t)e->sm_count;
+  return blocks32 <= sms ? PIPE : blocks32 <= 4u * sms ? THREE : blocks32 <= 8u * sms ? SINGLE : LOOKAHEAD;
 }
 
 struct Submit2D { uint64_t row_stride = 0, col_start = 0, dpitch = 0; uint32_t n_cols = 0; bool on = false; };
@@ -388,8 +444,7 @@ int submit_common(same_engine* e, const void* host_samples, const void* dev_samp
   }
   CK(e, cudaMemcpyAsync(b.d_len, lengths, e->n_streams * sizeof(uint32_t), cudaMemcpyHostToDevice, e->copy));
   if (!zeros && host_samples) {
-    int rc = ensure_input(e, b, total * ssz);
-    if (rc) return rc;
+    CK(e, b.d.grow(total * ssz, total * ssz / 8 + 8192));
     CK(e, cudaEventRecord(e->t_h2d0, e->copy));
     if (total && two_d.on)
       CK(e, cudaMemcpy2DAsync(b.d, (size_t)two_d.dpitch * ssz, static_cast<const uint8_t*>(host_samples) + two_d.col_start * ssz,
@@ -406,39 +461,32 @@ int submit_common(same_engine* e, const void* host_samples, const void* dev_samp
   CK(e, cudaEventRecord(b.copied, e->copy));
   CK(e, cudaStreamWaitEvent(e->compute, b.copied, 0));
   CK(e, cudaEventRecord(e->t_k0, e->compute));
-  // f32 input (now or earlier: the DC-blocker state may hold non-integers) needs the literal f32 recursion
-  int kernel = e->saw_f32 ? 1 : (e->force_generic ? e->force_generic : e->kernel_auto);
+  Kernel kernel = rx_kernel(e);
   // one stream, a long chunk: the long-stream path (time-parallel DC / AGC / matched filters, sequential timing loop)
-  if (e->long_stream && e->n_streams == 1 && !zeros && d_src && sample_fmt == 0 && !e->saw_f32 && e->force_generic == 0 &&
-      e->p.ntaps == 42 && e->p.dc_len == 16 && lengths[0] >= kLongMinSamples) {
+  const bool long_path = e->long_stream && e->n_streams == 1 && d_src && e->kernel_override == POLICY && kernel != GENERIC &&
+                         lengths[0] >= kLongMinSamples;
+  // the split pipeline's front end needs real samples: a zeros submit has none and takes the fused single-warp kernel
+  // (the resident state is the same)
+  if (kernel == SPLIT && !d_src) kernel = SINGLE;
+  if (long_path) {
     int rc = run_long(e, static_cast<const int16_t*>(d_src) + offsets[0], lengths[0]);
     if (rc) return rc;
-    CK(e, cudaEventRecord(e->t_k1, e->compute));
-    CK(e, cudaEventRecord(b.consumed, e->compute));
-    b.used = true;
-    e->timed_kernel = true;
-    e->in_flight = true;
-    return SAME_OK;
-  }
-  if (kernel == 5) {
-    // split pipeline: the front end needs real samples (a zeros submit has none: the fused single-warp kernel takes it,
-    // the resident state is the same) and a tile buffer for the longest chunk
-    if (zeros || !d_src) kernel = 2;
-    else {
+  } else {
+    if (kernel == SPLIT) {   // a tile buffer for the longest chunk
       uint32_t max_len = 0;
       for (uint32_t i = 0; i < e->n_streams; ++i) max_len = std::max(max_len, lengths[i]);
       int rc = ensure_tiles(e, max_len);
       if (rc) return rc;
       e->launches += 1;   // the front-end kernel
     }
+    CK(e, same_launch_rx(&e->p, &e->taps, &e->taps2, kernel, e->lanes_per_warp, d_src, sample_fmt, b.d_off, b.d_len,
+                         &e->tiles, e->compute));
+    e->launches += 1;
   }
-  CK(e, same_launch_rx(&e->p, &e->taps, &e->taps2, kernel, e->lanes_per_warp, d_src, sample_fmt, b.d_off, b.d_len, &e->tiles,
-                       e->compute));
   CK(e, cudaEventRecord(e->t_k1, e->compute));
   CK(e, cudaEventRecord(b.consumed, e->compute));
   b.used = true;
   e->timed_kernel = true;
-  e->launches += 1;
   e->in_flight = true;
   return SAME_OK;
 }
@@ -521,7 +569,7 @@ int same_engine_create(const same_config* cfg_in, int device, uint32_t n_streams
   float regul = cfg.eq_enabled ? cfg.eq_regularization : 1.0e-6f;
   if (nff > SAME_MAX_EQ || nfb > SAME_MAX_EQ) return fail(nullptr, SAME_ERR_INVALID_CONFIG, "equalizer order beyond the engine limit of 16 taps per arm");
 
-  same_engine* e = new same_engine();
+  std::unique_ptr<same_engine, void (*)(same_engine*)> e(new same_engine(), same_engine_destroy);
   e->cfg = cfg; e->device = device; e->n_streams = n_streams;
   SameParams& p = e->p;
   memset(&p, 0, sizeof p);
@@ -543,25 +591,9 @@ int same_engine_create(const same_config* cfg_in, int device, uint32_t n_streams
   }
   p.f_one = 1.0f; p.f_negzero = -0.0f;
   {
-    // Kernel / mapping policy for the 22050 Hz class (measured on B200, tables in profiles/README.md), by 32-stream
-    // blocks per SM:
-    //  * <= 1: four-warp pipelined kernel (producer / AGC / space filter / consumer), every warp on its own scheduler:
-    //    the per-stream dependent chain is what bounds the run time, so it is cut into stages.
-    //  * <= 4: three-warp kernel (producer / look-ahead AGC / consumer): fewer instructions in total, still
-    //    latency-hiding across the co-resident blocks.
-    //  * <= 8: single-warp fast kernel (8 resident blocks per SM: the whole batch is one wave; fewest instructions).
-    //  * more: single-warp look-ahead kernel (16 resident warps per SM, no d ring): the issue-bound regime.
-    //  20 s streams, ms per launch, pipelined / three-warp / single-warp / look-ahead: 4096 streams 24.0 / 24.9 / 41.6 / -;
-    //  8192: 36.8 / 29.1 / 43.3 / 66; 16384: 74.6 / 40.0 / 43.9 / 70; 32768: - / - / 57.7 / 81; 49152: - / - / 109 / 83;
-    //  65536: 228 / 158 / 116 / 97.
-    // Option "lanes_per_warp" spreads streams over more, lane-sparse warps (diagnostic).  No environment variable is
-    // read here: same_engine_set_option is the only override.
     int sms = 148;
     if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || sms <= 0) sms = 148;
-    e->sm_count = sms;
-    e->lanes_per_warp = 32;
-    const uint32_t blocks32 = (n_streams + 31u) / 32u;
-    e->kernel_auto = (blocks32 <= (uint32_t)sms) ? 3 : (blocks32 <= 4u * (uint32_t)sms) ? 4 : (blocks32 <= 8u * (uint32_t)sms) ? 2 : 6;
+    e->sm_count = sms;   // for the kernel policy (rx_kernel)
   }
   p.spt = sps / 2.0f;                                                         // symsync.rs:146
   {
@@ -602,86 +634,41 @@ int same_engine_create(const same_config* cfg_in, int device, uint32_t n_streams
   e->derived.alpha_locked = p.alpha_l; e->derived.beta_locked = p.beta_l;
   e->derived.dc_len = p.dc_len; e->derived.ntaps = p.ntaps;
 
-#define CKC(call)                                                                            \
-  do {                                                                                       \
-    cudaError_t _err = (call);                                                               \
-    if (_err != cudaSuccess) {                                                               \
-      int rc = fail(nullptr, SAME_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(_err)); \
-      same_engine_destroy(e);                                                                \
-      return rc;                                                                             \
-    }                                                                                        \
-  } while (0)
-  CKC(cudaSetDevice(device));
-  CKC(cudaStreamCreateWithFlags(&e->compute, cudaStreamNonBlocking));
-  CKC(cudaStreamCreateWithFlags(&e->copy, cudaStreamNonBlocking));
-  CKC(cudaMalloc(&e->d_state, (size_t)L.n_words * L.n_pad * sizeof(uint32_t)));
-  CKC(cudaMalloc(&e->d_blobs, (size_t)n_streams * sizeof(StreamBlob)));
-  CKC(cudaMemsetAsync(e->d_blobs, 0, (size_t)n_streams * sizeof(StreamBlob), e->compute));
-  CKC(cudaMalloc(&e->d_counters, 4 * sizeof(unsigned int)));
-  CKC(cudaMemsetAsync(e->d_counters, 0, 4 * sizeof(unsigned int), e->compute));
-  CKC(cudaHostAlloc(&e->h_counters, 4 * sizeof(unsigned int), cudaHostAllocDefault));
-  CKC(cudaHostAlloc(&e->h_stage, STAGE_BYTES, cudaHostAllocDefault));
-  for (auto& ev : e->stage_done) CKC(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-  for (auto& b : e->in) {
-    CKC(cudaMalloc(&b.d_off, (size_t)n_streams * sizeof(unsigned long long)));
-    CKC(cudaMalloc(&b.d_len, (size_t)n_streams * sizeof(uint32_t)));
-    CKC(cudaEventCreateWithFlags(&b.copied, cudaEventDisableTiming));
-    CKC(cudaEventCreateWithFlags(&b.consumed, cudaEventDisableTiming));
+  CK(nullptr, cudaSetDevice(device));
+  CK(nullptr, e->compute.create());
+  CK(nullptr, e->copy.create());
+  CK(nullptr, e->d_state.grow((size_t)L.n_words * L.n_pad));
+  CK(nullptr, e->d_blobs.grow(n_streams));
+  CK(nullptr, cudaMemsetAsync(e->d_blobs, 0, (size_t)n_streams * sizeof(StreamBlob), e->compute));
+  CK(nullptr, e->d_counters.grow(4));
+  CK(nullptr, cudaMemsetAsync(e->d_counters, 0, 4 * sizeof(unsigned int), e->compute));
+  CK(nullptr, e->d_sort_ws.grow(3 * (size_t)n_streams + 3));
+  CK(nullptr, e->h_counters.grow(4));
+  CK(nullptr, e->h_stage.grow(STAGE_BYTES));
+  for (Event& ev : e->stage_done) CK(nullptr, ev.create(cudaEventDisableTiming));
+  for (InputBuf& b : e->in) {
+    CK(nullptr, b.d_off.grow(n_streams));
+    CK(nullptr, b.d_len.grow(n_streams));
+    CK(nullptr, b.copied.create(cudaEventDisableTiming));
+    CK(nullptr, b.consumed.create(cudaEventDisableTiming));
   }
-  CKC(cudaEventCreate(&e->t_h2d0)); CKC(cudaEventCreate(&e->t_h2d1));
-  CKC(cudaEventCreate(&e->t_k0)); CKC(cudaEventCreate(&e->t_k1));
-  CKC(cudaEventCreate(&e->t_sw0)); CKC(cudaEventCreate(&e->t_sw1));
-  for (auto& ev : e->t_st) CKC(cudaEventCreate(&ev));
-  p.state32 = e->d_state; p.blobs = e->d_blobs; p.counters = e->d_counters;
-  {
-    size_t nev = std::max<size_t>(65536, (size_t)n_streams * 64);
-    size_t npay = std::max<size_t>(4u << 20, (size_t)n_streams * 4096);
-    int rc = alloc_arenas(e, nev, npay);
-    if (rc) { same_engine_destroy(e); return rc; }
-  }
-  CKC(same_launch_init(&e->p, nullptr, n_streams, 0, e->compute));
-  CKC(cudaStreamSynchronize(e->compute));
-#undef CKC
-  *out = e;
+  for (Event* ev : {&e->t_h2d0, &e->t_h2d1, &e->t_k0, &e->t_k1, &e->t_sw0, &e->t_sw1}) CK(nullptr, ev->create());
+  for (Event& ev : e->t_st) CK(nullptr, ev.create());
+  const int rc = alloc_arenas(e.get(), std::max<size_t>(65536, (size_t)n_streams * 64),
+                              std::max<size_t>(4u << 20, (size_t)n_streams * 4096));   // binds the kernel parameters
+  if (rc) return rc;
+  CK(nullptr, same_launch_init(&e->p, nullptr, n_streams, 0, e->compute));
+  CK(nullptr, cudaStreamSynchronize(e->compute));
+  *out = e.release();
   return SAME_OK;
 }
 
+// Everything the engine owns is released by its members' destructors, once the work queued on its streams is done.
 void same_engine_destroy(same_engine* e) {
   if (!e) return;
   cudaSetDevice(e->device);
   if (e->compute) cudaStreamSynchronize(e->compute);
   if (e->copy) cudaStreamSynchronize(e->copy);
-  for (auto& b : e->in) {
-    if (b.d) cudaFree(b.d);
-    if (b.d_off) cudaFree(b.d_off);
-    if (b.d_len) cudaFree(b.d_len);
-    if (b.copied) cudaEventDestroy(b.copied);
-    if (b.consumed) cudaEventDestroy(b.consumed);
-  }
-  if (e->d_state) cudaFree(e->d_state);
-  if (e->d_blobs) cudaFree(e->d_blobs);
-  if (e->d_events) cudaFree(e->d_events);
-  if (e->d_sorted) cudaFree(e->d_sorted);
-  if (e->d_sort_ws) cudaFree(e->d_sort_ws);
-  if (e->d_payload) cudaFree(e->d_payload);
-  if (e->d_counters) cudaFree(e->d_counters);
-  if (e->h_counters) cudaFreeHost(e->h_counters);
-  if (e->h_stage) cudaFreeHost(e->h_stage);
-  for (auto& ev : e->stage_done) if (ev) cudaEventDestroy(ev);
-  if (e->d_trace) cudaFree(e->d_trace);
-  if (e->d_ids) cudaFree(e->d_ids);
-  for (float* q : {e->ls_d, e->ls_y, e->ls_g, e->ls_soft, e->ls_gin}) if (q) cudaFree(q);
-  if (e->ls_ctrl) cudaFree(e->ls_ctrl);
-  if (e->ls_hctrl) cudaFreeHost(e->ls_hctrl);
-  if (e->tiles.d) cudaFree(e->tiles.d);
-  if (e->tiles.dc_next) cudaFree(e->tiles.dc_next);
-  for (cudaEvent_t ev : {e->t_h2d0, e->t_h2d1, e->t_k0, e->t_k1, e->t_sw0, e->t_sw1}) if (ev) cudaEventDestroy(ev);
-  for (cudaEvent_t ev : e->t_st) if (ev) cudaEventDestroy(ev);
-  if (e->d_xfer) cudaFree(e->d_xfer);
-  if (e->d_xids) cudaFree(e->d_xids);
-  if (e->d_xres) cudaFree(e->d_xres);
-  if (e->compute) cudaStreamDestroy(e->compute);
-  if (e->copy) cudaStreamDestroy(e->copy);
   delete e;
 }
 
@@ -725,64 +712,51 @@ int same_engine_reset(same_engine* e, const uint32_t* ids, uint32_t n) {
   } else {
     for (uint32_t i = 0; i < n; ++i)
       if (ids[i] >= e->n_streams) return fail(e, SAME_ERR_INVALID_ARG, "stream id out of range");
-    if (n > e->ids_cap) {
-      if (e->d_ids) CK(e, cudaFree(e->d_ids));
-      e->d_ids = nullptr;
-      CK(e, cudaMalloc(&e->d_ids, (size_t)n * sizeof(uint32_t)));
-      e->ids_cap = n;
-    }
+    CK(e, e->d_ids.grow(n));
     CK(e, cudaMemcpyAsync(e->d_ids, ids, (size_t)n * sizeof(uint32_t), cudaMemcpyHostToDevice, e->compute));
     CK(e, same_launch_init(&e->p, e->d_ids, n, 1, e->compute));
     e->launches += 1;
-    // drop queued events of the reset streams
-    std::vector<char> is_reset(e->n_streams, 0);
-    for (uint32_t i = 0; i < n; ++i) is_reset[ids[i]] = 1;
-    e->pend_events.erase(std::remove_if(e->pend_events.begin(), e->pend_events.end(),
-                                        [&](const same_event& ev) { return is_reset[ev.stream] != 0; }),
-                         e->pend_events.end());
+    forget_events(e, ids, n);
   }
   CK(e, cudaStreamSynchronize(e->compute));
   return SAME_OK;
 }
 
 struct same_snapshot {
-  int device; uint32_t n_streams; size_t state_bytes, blob_bytes;
-  uint32_t* d_state; StreamBlob* d_blobs;
-  bool saw_f32;   // the DC-blocker state may be non-integer: restore must keep the engine on the generic kernel
+  int device = 0;
+  uint32_t n_streams = 0;
+  bool saw_f32 = false;   // the DC-blocker state may be non-integer: restore must keep the engine on the generic kernel
+  DevBuf<uint32_t> d_state;
+  DevBuf<StreamBlob> d_blobs;
 };
 
 int same_engine_snapshot(same_engine* e, same_snapshot** out) {
   if (!e || !out) return fail(e, SAME_ERR_INVALID_ARG, "null argument");
   int rc = same_engine_sync(e);
   if (rc) return rc;
-  same_snapshot* s = new same_snapshot();
+  std::unique_ptr<same_snapshot> s(new same_snapshot());
   s->device = e->device; s->n_streams = e->n_streams;
-  s->state_bytes = (size_t)e->p.layout.n_words * e->p.layout.n_pad * sizeof(uint32_t);
-  s->blob_bytes = (size_t)e->n_streams * sizeof(StreamBlob);
-  s->d_state = nullptr; s->d_blobs = nullptr;
   s->saw_f32 = e->saw_f32;
-  cudaError_t err = cudaMalloc(&s->d_state, s->state_bytes);
-  if (err == cudaSuccess) err = cudaMalloc(&s->d_blobs, s->blob_bytes);
-  if (err == cudaSuccess) err = cudaMemcpyAsync(s->d_state, e->d_state, s->state_bytes, cudaMemcpyDeviceToDevice, e->compute);
-  if (err == cudaSuccess) err = cudaMemcpyAsync(s->d_blobs, e->d_blobs, s->blob_bytes, cudaMemcpyDeviceToDevice, e->compute);
+  cudaError_t err = s->d_state.grow(e->d_state.size());
+  if (err == cudaSuccess) err = s->d_blobs.grow(e->d_blobs.size());
+  if (err == cudaSuccess)
+    err = cudaMemcpyAsync(s->d_state, e->d_state, e->d_state.size() * sizeof(uint32_t), cudaMemcpyDeviceToDevice, e->compute);
+  if (err == cudaSuccess)
+    err = cudaMemcpyAsync(s->d_blobs, e->d_blobs, e->d_blobs.size() * sizeof(StreamBlob), cudaMemcpyDeviceToDevice, e->compute);
   if (err == cudaSuccess) err = cudaStreamSynchronize(e->compute);
-  if (err != cudaSuccess) {
-    same_snapshot_free(s);
-    return fail(e, SAME_ERR_CUDA, std::string("snapshot: ") + cudaGetErrorString(err));
-  }
-  *out = s;
+  if (err != cudaSuccess) return fail(e, SAME_ERR_CUDA, std::string("snapshot: ") + cudaGetErrorString(err));
+  *out = s.release();
   return SAME_OK;
 }
 
 int same_engine_restore(same_engine* e, const same_snapshot* s) {
   if (!e || !s) return fail(e, SAME_ERR_INVALID_ARG, "null argument");
-  if (s->device != e->device || s->n_streams != e->n_streams ||
-      s->state_bytes != (size_t)e->p.layout.n_words * e->p.layout.n_pad * sizeof(uint32_t))
+  if (s->device != e->device || s->n_streams != e->n_streams || s->d_state.size() != e->d_state.size())
     return fail(e, SAME_ERR_INVALID_ARG, "snapshot belongs to a different engine shape");
   int rc = same_engine_sync(e);
   if (rc) return rc;
-  CK(e, cudaMemcpyAsync(e->d_state, s->d_state, s->state_bytes, cudaMemcpyDeviceToDevice, e->compute));
-  CK(e, cudaMemcpyAsync(e->d_blobs, s->d_blobs, s->blob_bytes, cudaMemcpyDeviceToDevice, e->compute));
+  CK(e, cudaMemcpyAsync(e->d_state, s->d_state, e->d_state.size() * sizeof(uint32_t), cudaMemcpyDeviceToDevice, e->compute));
+  CK(e, cudaMemcpyAsync(e->d_blobs, s->d_blobs, e->d_blobs.size() * sizeof(StreamBlob), cudaMemcpyDeviceToDevice, e->compute));
   CK(e, cudaStreamSynchronize(e->compute));
   e->pend_events.clear(); e->pend_payload.clear();
   e->saw_f32 = s->saw_f32;
@@ -792,8 +766,6 @@ int same_engine_restore(same_engine* e, const same_snapshot* s) {
 void same_snapshot_free(same_snapshot* s) {
   if (!s) return;
   cudaSetDevice(s->device);
-  if (s->d_state) cudaFree(s->d_state);
-  if (s->d_blobs) cudaFree(s->d_blobs);
   delete s;
 }
 
@@ -890,14 +862,12 @@ int same_engine_enable_soft_trace(same_engine* e, uint32_t cap_per_stream) {
   if (!e) return fail(nullptr, SAME_ERR_INVALID_ARG, "null engine");
   int rc = same_engine_sync(e);
   if (rc) return rc;
-  if (e->d_trace) { CK(e, cudaFree(e->d_trace)); e->d_trace = nullptr; }
-  e->p.trace = nullptr; e->p.trace_cap = 0;
+  DevBuf<same_soft_symbol> trace;   // exactly cap_per_stream symbols per stream (none: tracing off)
+  CK(e, trace.grow((size_t)e->n_streams * cap_per_stream));
   const SameLayout& L = e->p.layout;
   CK(e, cudaMemset(e->d_state + (size_t)F_TRACE_N * L.n_pad, 0, (size_t)L.n_pad * 4));
-  if (cap_per_stream) {
-    CK(e, cudaMalloc(&e->d_trace, (size_t)e->n_streams * cap_per_stream * sizeof(same_soft_symbol)));
-    e->p.trace = e->d_trace; e->p.trace_cap = cap_per_stream;
-  }
+  e->d_trace.swap(trace);
+  bind(e);
   return SAME_OK;
 }
 
@@ -927,7 +897,7 @@ int same_engine_set_option(same_engine* e, const char* key, int value) {
   if (rc) return rc;
   if (strcmp(key, "kernel") == 0 || strcmp(key, "force_generic") == 0) {
     if (value < 0 || value > 6) return fail(e, SAME_ERR_INVALID_ARG, "kernel must be 0 (policy), 1 generic, 2 single-warp, 3 pipelined, 4 three-warp, 5 split (front end + tile-fed) or 6 look-ahead single-warp");
-    e->force_generic = value;
+    e->kernel_override = (Kernel)value;
     return SAME_OK;
   }
 
@@ -943,7 +913,7 @@ int same_engine_set_option(same_engine* e, const char* key, int value) {
 
 int same_engine_get_option(same_engine* e, const char* key, int* value) {
   if (!e || !key || !value) return fail(e, SAME_ERR_INVALID_ARG, "null argument");
-  if (strcmp(key, "kernel") == 0 || strcmp(key, "force_generic") == 0) { *value = e->force_generic; return SAME_OK; }
+  if (strcmp(key, "kernel") == 0 || strcmp(key, "force_generic") == 0) { *value = e->kernel_override; return SAME_OK; }
   if (strcmp(key, "device_sort") == 0) { *value = e->device_sort; return SAME_OK; }
   if (strcmp(key, "long_stream") == 0) { *value = e->long_stream; return SAME_OK; }
   if (strcmp(key, "long_stream_passes") == 0) { *value = (int)std::min<uint64_t>(e->ls_spec_launches, 0x7fffffff); return SAME_OK; }
@@ -951,11 +921,7 @@ int same_engine_get_option(same_engine* e, const char* key, int* value) {
   if (strcmp(key, "lanes_per_warp") == 0) { *value = (int)e->lanes_per_warp; return SAME_OK; }
   if (strcmp(key, "state_kernel_us") == 0) { *value = (int)std::min(e->st_kernel_ms * 1000.0f, 2.0e9f); return SAME_OK; }
   if (strcmp(key, "state_copy_us") == 0) { *value = (int)std::min(e->st_copy_ms * 1000.0f, 2.0e9f); return SAME_OK; }
-  if (strcmp(key, "kernel_selected") == 0) {
-    const bool fast_geometry = e->p.ntaps == 42 && e->p.dc_len == 16;
-    *value = (e->saw_f32 || !fast_geometry) ? 1 : (e->force_generic ? e->force_generic : e->kernel_auto);
-    return SAME_OK;
-  }
+  if (strcmp(key, "kernel_selected") == 0) { *value = rx_kernel(e); return SAME_OK; }
   return fail(e, SAME_ERR_INVALID_ARG, std::string("unknown option ") + key);
 }
 
@@ -1029,139 +995,20 @@ int same_engine_get_derived(const same_engine* e, same_derived* d, float* mark_r
 }  // extern "C"
 
 // ---------------------------------------------------------------------------------------------------------------------
-// Portable stream state (format in include/same_engine.h).  The header is parsed and compared with an engine here only;
+// Portable stream state (format in include/same_engine.h and same_state.cu): the parts that need the engine's buffers.
 // same_multi.cu reuses these helpers (same_state_* below, C++ linkage, not part of the C ABI).
 // ---------------------------------------------------------------------------------------------------------------------
 namespace {
 
-constexpr uint32_t kStMagic = 0x54534D53u;   // "SMST"
-constexpr uint32_t kStVersion = 1u;
-constexpr uint32_t kStBom = 0x01020304u;
-constexpr size_t kStHeaderBytes = 2224;
-constexpr size_t kStOffConfig = 40, kStOffDerived = 116, kStOffMark = 164, kStOffSpace = 1188, kStOffCrc = 2220;
-static_assert(sizeof(same_config) == 19 * 4 && sizeof(same_derived) == 12 * 4, "4-byte fields only");
-static_assert(kStOffDerived == kStOffConfig + sizeof(same_config) && kStOffMark == kStOffDerived + sizeof(same_derived) &&
-              kStOffSpace == kStOffMark + 8 * SAME_MAX_TAPS && kStOffCrc + 4 == kStHeaderBytes, "header layout");
-
-void put32(uint8_t* p, uint32_t v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); p[2] = (uint8_t)(v >> 16); p[3] = (uint8_t)(v >> 24); }
-uint32_t get32(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24); }
-// a struct of 4-byte fields <-> little-endian words
-void put_words(uint8_t* p, const void* src, size_t bytes) {
-  for (size_t i = 0; i < bytes; i += 4) { uint32_t v; memcpy(&v, static_cast<const uint8_t*>(src) + i, 4); put32(p + i, v); }
-}
-void get_words(void* dst, const uint8_t* p, size_t bytes) {
-  for (size_t i = 0; i < bytes; i += 4) { const uint32_t v = get32(p + i); memcpy(static_cast<uint8_t*>(dst) + i, &v, 4); }
-}
-
-const char* const kConfigFields[19] = {
-    "input_rate", "dc_blocker_len", "agc_bandwidth", "agc_gain_min", "agc_gain_max", "timing_bw_unlocked",
-    "timing_bw_locked", "timing_max_deviation", "squelch_power_open", "squelch_power_close", "squelch_bandwidth",
-    "preamble_max_errors", "eq_enabled", "eq_nff", "eq_nfb", "eq_relaxation", "eq_regularization",
-    "frame_prefix_max_errors", "frame_max_invalid_bytes"};
-const char* const kDerivedFields[12] = {"sps", "agc_bw", "agc_gain0", "samples_per_ted", "period_min", "period_max",
-                                        "alpha_unlocked", "beta_unlocked", "alpha_locked", "beta_locked", "dc_len", "ntaps"};
-// same_state.cu: enum Check
-const char* const kCheckNames[] = {
-    "valid", "CRC mismatch", "record flags (only bit 0 is defined)", "F_FLAGS (undefined bits)", "framer state > 2",
-    "transport state > 2", "F_CLOCK > 2^22", "F_TEDCNT not in {0, 1}", "F_SQ_BYTECLK not in -1..7", "F_SQ_HEAD >= 64",
-    "F_HIST_N > 3", "burst history length > 268", "pending length > 268", "pending kind > 2", "pending error > 3",
-    "pending_offset beyond the pending text", "previous-message length > 268"};
-
-struct StateHeader {
-  same_config cfg;
-  same_derived derived;
-  uint8_t taps[2 * 8 * SAME_MAX_TAPS];   // raw little-endian bits: mark (re, im) x 128, then space
-  uint32_t n_records, n_words, record_bytes;
-};
-
-void write_header(const same_engine* e, uint32_t n, uint8_t* h) {
-  memset(h, 0, kStHeaderBytes);
-  put32(h + 0, kStMagic); put32(h + 4, kStVersion); put32(h + 8, kStBom); put32(h + 12, (uint32_t)kStHeaderBytes);
-  put32(h + 16, n); put32(h + 20, e->p.layout.n_words); put32(h + 24, (uint32_t)sizeof(StreamBlob));
-  put32(h + 28, SAME_BURST_CAP); put32(h + 32, same_state_record_bytes(e->p.layout.n_words));
-  put_words(h + kStOffConfig, &e->cfg, sizeof(same_config));
-  put_words(h + kStOffDerived, &e->derived, sizeof(same_derived));
-  for (uint32_t i = 0; i < e->p.ntaps; ++i) {
-    const float v[4] = {e->taps.mark_re[i], e->taps.mark_im[i], e->taps.space_re[i], e->taps.space_im[i]};
-    put_words(h + kStOffMark + 8 * i, v, 8);
-    put_words(h + kStOffSpace + 8 * i, v + 2, 8);
-  }
-  put32(h + kStOffCrc, same_state_crc32(h, kStOffCrc));
-}
-
-// Format checks only (no engine): SAME_ERR_INVALID_ARG on any failure
-int parse_header(const void* buf, size_t len, StateHeader* out, std::string* why) {
-  const uint8_t* h = static_cast<const uint8_t*>(buf);
-  auto bad = [&](const std::string& m) { *why = "state buffer: " + m; return (int)SAME_ERR_INVALID_ARG; };
-  if (!h) return bad("null pointer");
-  if (len < 16) return bad("truncated header");
-  if (get32(h) != kStMagic) return bad("bad magic");
-  if (get32(h + 8) != kStBom) return bad("wrong byte order");
-  if (get32(h + 4) != kStVersion) return bad("format version " + std::to_string(get32(h + 4)) + ", this library reads version " + std::to_string(kStVersion));
-  if (get32(h + 12) != kStHeaderBytes) return bad("bad header size");
-  if (len < kStHeaderBytes) return bad("truncated header");
-  if (get32(h + kStOffCrc) != same_state_crc32(h, kStOffCrc)) return bad("header CRC mismatch");
-  StateHeader s;
-  s.n_records = get32(h + 16); s.n_words = get32(h + 20); s.record_bytes = get32(h + 32);
-  if (get32(h + 24) != sizeof(StreamBlob) || get32(h + 28) != SAME_BURST_CAP) return bad("stream blob layout differs from this library's");
-  if (s.n_words < F_NUM_SCALARS || s.n_words > (1u << 16) || s.record_bytes != same_state_record_bytes(s.n_words))
-    return bad("inconsistent record size");
-  const size_t need = kStHeaderBytes + (size_t)s.n_records * s.record_bytes;
-  if (len < need) return bad("truncated: " + std::to_string(len) + " bytes, the header announces " + std::to_string(need));
-  if (len > need) return bad("trailing bytes after the last record");
-  get_words(&s.cfg, h + kStOffConfig, sizeof(same_config));
-  get_words(&s.derived, h + kStOffDerived, sizeof(same_derived));
-  memcpy(s.taps, h + kStOffMark, sizeof s.taps);
-  *out = s;
-  return SAME_OK;
-}
-
-// The state must have been produced under exactly this engine's configuration: SAME_ERR_INVALID_CONFIG names the first
-// field that differs (derived values and taps are compared bit for bit: they are libm results of the exporting host)
-int compare_header(const same_engine* e, const StateHeader& s, std::string* why) {
-  uint32_t a[19], b[19];
-  memcpy(a, &e->cfg, sizeof a); memcpy(b, &s.cfg, sizeof b);
-  for (int i = 0; i < 19; ++i)
-    if (a[i] != b[i]) { *why = std::string("state was produced under another configuration: ") + kConfigFields[i] + " differs"; return SAME_ERR_INVALID_CONFIG; }
-  uint32_t c[12], d[12];
-  memcpy(c, &e->derived, sizeof c); memcpy(d, &s.derived, sizeof d);
-  for (int i = 0; i < 12; ++i)
-    if (c[i] != d[i]) { *why = std::string("derived constant ") + kDerivedFields[i] + " differs from this engine's (another host's libm?)"; return SAME_ERR_INVALID_CONFIG; }
-  StateHeader mine;
-  {
-    uint8_t h[kStHeaderBytes];
-    write_header(e, 0, h);
-    memcpy(mine.taps, h + kStOffMark, sizeof mine.taps);
-  }
-  if (memcmp(mine.taps, s.taps, 8 * SAME_MAX_TAPS) != 0) { *why = "mark filter taps differ from this engine's"; return SAME_ERR_INVALID_CONFIG; }
-  if (memcmp(mine.taps + 8 * SAME_MAX_TAPS, s.taps + 8 * SAME_MAX_TAPS, 8 * SAME_MAX_TAPS) != 0) {
-    *why = "space filter taps differ from this engine's"; return SAME_ERR_INVALID_CONFIG;
-  }
-  if (s.n_words != e->p.layout.n_words) { *why = "state words per stream differ from this engine's"; return SAME_ERR_INVALID_CONFIG; }
-  return SAME_OK;
+// the header of a state this engine exports, and that a state it imports must match
+same_state::Header state_header(const same_engine* e, uint32_t n) {
+  return same_state::make_header(e->cfg, e->derived, e->taps, e->p.ntaps, e->p.layout.n_words, n);
 }
 
 bool is_pinned(const void* p) {
   cudaPointerAttributes a;
   if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
   return a.type == cudaMemoryTypeHost;
-}
-
-int ensure_xfer(same_engine* e, size_t bytes, uint32_t n_ids) {
-  if (bytes > e->xfer_cap) {
-    if (e->d_xfer) CK(e, cudaFree(e->d_xfer));
-    e->d_xfer = nullptr; e->xfer_cap = 0;
-    CK(e, cudaMalloc(&e->d_xfer, bytes));
-    e->xfer_cap = bytes;
-  }
-  if (n_ids > e->xids_cap) {
-    if (e->d_xids) CK(e, cudaFree(e->d_xids));
-    e->d_xids = nullptr; e->xids_cap = 0;
-    CK(e, cudaMalloc(&e->d_xids, (size_t)n_ids * sizeof(uint32_t)));
-    e->xids_cap = n_ids;
-  }
-  if (!e->d_xres) CK(e, cudaMalloc(&e->d_xres, 2 * sizeof(unsigned long long)));
-  return SAME_OK;
 }
 
 // ids -> (device id list, or nullptr + first for a contiguous run)
@@ -1176,27 +1023,13 @@ int upload_ids(same_engine* e, const uint32_t* ids, uint32_t n, const uint32_t**
   return SAME_OK;
 }
 
-// device -> host (pinned: one copy; pageable: through the pinned staging area, two pieces in flight)
+// device -> host (pinned: one copy; pageable: through the pinned staging area)
 int copy_out(same_engine* e, uint8_t* dst, const uint8_t* src, size_t bytes) {
   if (is_pinned(dst)) {
     if (bytes) CK(e, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, e->compute));
     return SAME_OK;
   }
-  const size_t half = STAGE_BYTES / 2;
-  size_t done = 0, queued = 0, qn[2] = {0, 0};
-  int qslot = 0, pslot = 0, inflight = 0;
-  while (done < bytes) {
-    while (inflight < 2 && queued < bytes) {
-      const size_t n = std::min(half, bytes - queued);
-      CK(e, cudaMemcpyAsync(e->h_stage + qslot * half, src + queued, n, cudaMemcpyDeviceToHost, e->compute));
-      CK(e, cudaEventRecord(e->stage_done[qslot], e->compute));
-      qn[qslot] = n; queued += n; qslot ^= 1; ++inflight;
-    }
-    CK(e, cudaEventSynchronize(e->stage_done[pslot]));
-    memcpy(dst + done, e->h_stage + pslot * half, qn[pslot]);
-    done += qn[pslot]; pslot ^= 1; --inflight;
-  }
-  return SAME_OK;
+  return stage_out(e, src, bytes, [&dst](const uint8_t* h, size_t n) { memcpy(dst, h, n); dst += n; });
 }
 
 // host -> device, the same way round
@@ -1232,17 +1065,18 @@ int check_ids(same_engine* e, const uint32_t* ids, uint32_t n, uint32_t limit, b
 
 }  // namespace
 
-// ---- helpers shared with same_multi.cu (C++ linkage; the engine must be synced and the arguments checked) ----
-size_t same_state_header_bytes() { return kStHeaderBytes; }
+// ---- helpers shared with same_multi.cu (the engine must be synced and the arguments checked) ----
 size_t same_state_engine_record_bytes(const same_engine* e) { return same_state_record_bytes(e->p.layout.n_words); }
-void same_state_write_header(const same_engine* e, uint32_t n, void* dst) { write_header(e, n, static_cast<uint8_t*>(dst)); }
 
-// header format + comparison with `e`; on failure the reason is the engine's last error
+void same_state_write_header(const same_engine* e, uint32_t n, void* dst) {
+  same_state::write_header(state_header(e, n), static_cast<uint8_t*>(dst));
+}
+
 int same_state_check_header(same_engine* e, const void* buf, size_t len, uint32_t* n_records) {
-  StateHeader s;
+  same_state::Header s;
   std::string why;
-  int rc = parse_header(buf, len, &s, &why);
-  if (rc == SAME_OK) rc = compare_header(e, s, &why);
+  int rc = same_state::parse_header(buf, len, &s, &why);
+  if (rc == SAME_OK) rc = same_state::compare_header(state_header(e, 0), s, &why);
   if (rc != SAME_OK) return fail(e, rc, why);
   *n_records = s.n_records;
   return SAME_OK;
@@ -1254,8 +1088,8 @@ int same_state_export_records(same_engine* e, const uint32_t* ids, uint32_t n, u
   if (rc) return rc;
   CK(e, cudaSetDevice(e->device));
   const size_t bytes = (size_t)n * same_state_engine_record_bytes(e);
-  rc = ensure_xfer(e, bytes, n);
-  if (rc) return rc;
+  CK(e, e->d_xfer.grow(bytes));
+  CK(e, e->d_xids.grow(n));
   const uint32_t* d_ids; uint32_t first;
   rc = upload_ids(e, ids, n, &d_ids, &first);
   if (rc) return rc;
@@ -1278,8 +1112,9 @@ int same_state_import_stage(same_engine* e, uint32_t n, const void* recs, uint32
   if (rc) return rc;
   CK(e, cudaSetDevice(e->device));
   const size_t bytes = (size_t)n * same_state_engine_record_bytes(e);
-  rc = ensure_xfer(e, bytes, n);
-  if (rc) return rc;
+  CK(e, e->d_xfer.grow(bytes));
+  CK(e, e->d_xids.grow(n));   // for the commit, which then allocates nothing
+  CK(e, e->d_xres.grow(2));
   const unsigned long long init[2] = {~0ull, 0ull};
   CK(e, cudaMemcpyAsync(e->d_xres, init, sizeof init, cudaMemcpyHostToDevice, e->compute));
   CK(e, cudaEventRecord(e->t_st[0], e->compute));
@@ -1296,8 +1131,7 @@ int same_state_import_stage(same_engine* e, uint32_t n, const void* recs, uint32
   CK(e, cudaEventElapsedTime(&e->st_kernel_ms, e->t_st[1], e->t_st[2]));
   if (res[0] != ~0ull) {
     const uint32_t code = (uint32_t)res[0], rec = (uint32_t)(res[0] >> 32);
-    const size_t nc = sizeof kCheckNames / sizeof kCheckNames[0];
-    return fail(e, SAME_ERR_INVALID_ARG, "state record " + std::to_string(rec) + ": " + (code < nc ? kCheckNames[code] : "invalid"));
+    return fail(e, SAME_ERR_INVALID_ARG, "state record " + std::to_string(rec) + ": " + same_state::check_name(code));
   }
   *rec_flags = (uint32_t)res[1];
   return SAME_OK;
@@ -1317,12 +1151,7 @@ int same_state_import_commit(same_engine* e, const uint32_t* ids, uint32_t n, ui
   float ms = 0.0f;
   CK(e, cudaEventElapsedTime(&ms, e->t_st[0], e->t_st[1]));
   e->st_kernel_ms += ms;
-  // undrained events of the target streams belong to the state that was replaced
-  std::vector<char> hit(e->n_streams, 0);
-  for (uint32_t i = 0; i < n; ++i) hit[ids ? ids[i] : i] = 1;
-  e->pend_events.erase(std::remove_if(e->pend_events.begin(), e->pend_events.end(),
-                                      [&](const same_event& ev) { return hit[ev.stream] != 0; }),
-                       e->pend_events.end());
+  forget_events(e, ids, n);   // they belong to the state that was replaced
   if (rec_flags & 1u) e->saw_f32 = true;
   return SAME_OK;
 }
@@ -1330,7 +1159,7 @@ int same_state_import_commit(same_engine* e, const uint32_t* ids, uint32_t n, ui
 extern "C" {
 
 size_t same_engine_state_bytes(const same_engine* e, uint32_t n) {
-  return e ? kStHeaderBytes + (size_t)n * same_state_engine_record_bytes(e) : 0;
+  return e ? same_state::kHeaderBytes + (size_t)n * same_state_engine_record_bytes(e) : 0;
 }
 
 int same_engine_export_streams(same_engine* e, const uint32_t* ids, uint32_t n, void* buf, size_t cap, size_t* written) {
@@ -1341,8 +1170,8 @@ int same_engine_export_streams(same_engine* e, const uint32_t* ids, uint32_t n, 
   const size_t need = same_engine_state_bytes(e, n);
   if (written) *written = need;
   if (!buf || cap < need) return fail(e, SAME_ERR_INVALID_ARG, "export buffer too small: " + std::to_string(need) + " bytes needed");
-  write_header(e, n, static_cast<uint8_t*>(buf));
-  return same_state_export_records(e, ids, n, 0, static_cast<uint8_t*>(buf) + kStHeaderBytes);
+  same_state_write_header(e, n, buf);
+  return same_state_export_records(e, ids, n, 0, static_cast<uint8_t*>(buf) + same_state::kHeaderBytes);
 }
 
 int same_engine_import_streams(same_engine* e, const uint32_t* ids, uint32_t n, const void* buf, size_t len) {
@@ -1355,15 +1184,15 @@ int same_engine_import_streams(same_engine* e, const uint32_t* ids, uint32_t n, 
   rc = check_ids(e, ids, n, e->n_streams, true);
   if (rc) return rc;
   uint32_t flags = 0;
-  rc = same_state_import_stage(e, n, static_cast<const uint8_t*>(buf) + kStHeaderBytes, &flags);
+  rc = same_state_import_stage(e, n, static_cast<const uint8_t*>(buf) + same_state::kHeaderBytes, &flags);
   if (rc) return rc;
   return same_state_import_commit(e, ids, n, flags);
 }
 
 int same_state_info(const void* buf, size_t len, same_config* cfg, uint32_t* n_records) {
-  StateHeader s;
+  same_state::Header s;
   std::string why;
-  const int rc = parse_header(buf, len, &s, &why);
+  const int rc = same_state::parse_header(buf, len, &s, &why);
   if (rc) return fail(nullptr, rc, why);
   if (cfg) *cfg = s.cfg;
   if (n_records) *n_records = s.n_records;
@@ -1384,12 +1213,14 @@ int same_h2d_probe(int device, const void* host, size_t row_stride_bytes, size_t
                    float* elapsed_ms) {
   if (!host || !elapsed_ms || !width_bytes || !rows || reps < 1 || width_bytes > row_stride_bytes)
     return fail(nullptr, SAME_ERR_INVALID_ARG, "bad probe arguments");
-  cudaStream_t st = nullptr; cudaEvent_t a = nullptr, b = nullptr; void* d = nullptr;
+  Stream st;
+  Event a, b;
+  DevBuf<uint8_t> d;
   cudaError_t err = cudaSetDevice(device);
-  if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
-  if (err == cudaSuccess) err = cudaEventCreate(&a);
-  if (err == cudaSuccess) err = cudaEventCreate(&b);
-  if (err == cudaSuccess) err = cudaMalloc(&d, width_bytes * rows);
+  if (err == cudaSuccess) err = st.create();
+  if (err == cudaSuccess) err = a.create();
+  if (err == cudaSuccess) err = b.create();
+  if (err == cudaSuccess) err = d.grow(width_bytes * rows);
   if (err == cudaSuccess) err = cudaMemcpy2DAsync(d, width_bytes, host, row_stride_bytes, width_bytes, rows, cudaMemcpyHostToDevice, st);  // warm-up
   if (err == cudaSuccess) err = cudaEventRecord(a, st);
   for (int i = 0; i < reps && err == cudaSuccess; ++i)
@@ -1397,10 +1228,6 @@ int same_h2d_probe(int device, const void* host, size_t row_stride_bytes, size_t
   if (err == cudaSuccess) err = cudaEventRecord(b, st);
   if (err == cudaSuccess) err = cudaEventSynchronize(b);
   if (err == cudaSuccess) err = cudaEventElapsedTime(elapsed_ms, a, b);
-  if (d) cudaFree(d);
-  if (a) cudaEventDestroy(a);
-  if (b) cudaEventDestroy(b);
-  if (st) cudaStreamDestroy(st);
   if (err != cudaSuccess) return fail(nullptr, SAME_ERR_CUDA, std::string("h2d probe: ") + cudaGetErrorString(err));
   return SAME_OK;
 }

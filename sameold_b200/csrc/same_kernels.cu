@@ -34,6 +34,7 @@
 #include <cuda_runtime.h>
 
 #include "same_fast.cuh"
+#include "same_internal.h"
 #include "same_lane.cuh"
 
 namespace same_dev {
@@ -1314,52 +1315,58 @@ __global__ void same_evsort_scatter(const same_event* __restrict__ ev, uint32_t 
 // ----------------------------------------------------------------------------------------------------------------
 // Launchers (called from same_engine.cu)
 // ----------------------------------------------------------------------------------------------------------------
-// kernel ids: 1 generic, 2 single-warp fast, 3 pipelined four-warp, 4 three-warp, 5 single-warp fast fed by the front-end
-// kernel's tiles (split pipeline), 6 look-ahead single-warp (16 resident warps per SM).
-extern "C" cudaError_t same_launch_rx(const SameParams* p, const SameTaps* taps, const SameTaps2* taps2, int force_generic,
+extern "C" cudaError_t same_launch_rx(const SameParams* p, const SameTaps* taps, const SameTaps2* taps2, Kernel kernel,
                                       uint32_t lanes_per_warp, const void* d_samples_v, int sample_fmt,
                                       const unsigned long long* d_offsets, const uint32_t* d_lengths,
                                       const SameTiles* tiles, cudaStream_t stream) {
   const uint32_t blocks = (p->n_streams + 31u) / 32u;
   const int16_t* d_samples = static_cast<const int16_t*>(d_samples_v);
-  // The fast kernels need the 22050 Hz geometry (42 taps, DC length 16) and s16 samples (their DC blocker is an
-  // integer recursion).
-  if (sample_fmt == 0 && force_generic != 1 && p->ntaps == FAST_NTAPS && p->dc_len == FAST_DCL) {
-    const uint32_t lanes = (force_generic == 5) ? 32u : (lanes_per_warp ? lanes_per_warp : 32u);
-    const uint32_t fblocks = (p->n_streams + lanes - 1u) / lanes;
-    SameTiles t{nullptr, nullptr, 0u, 32u, 1u};
-    if (force_generic == 5) {
+  const uint32_t lanes = (kernel == SPLIT) ? 32u : (lanes_per_warp ? lanes_per_warp : 32u);
+  const uint32_t fblocks = (p->n_streams + lanes - 1u) / lanes;
+  const SameTiles no_tiles{nullptr, nullptr, 0u, 32u, 1u};
+  switch (kernel) {
+    case SPLIT: {
       if (!tiles || !tiles->d || !d_samples) return cudaErrorInvalidValue;
-      t = *tiles;
+      const SameTiles t = *tiles;
       const unsigned long long grid = (unsigned long long)((t.n_max + FE_RUN * FE_WARPS - 1u) / (FE_RUN * FE_WARPS)) * blocks;
       if (grid == 0ull || grid > 0x7fffffffull) return cudaErrorInvalidValue;
       same_dev::same_frontend_kernel<<<(unsigned)grid, FE_WARPS * 32, 0, stream>>>(*p, d_samples, d_offsets, d_lengths, t);
       same_dev::same_rx_fast_kernel<true><<<fblocks, 32, 0, stream>>>(*p, *taps2, d_samples, d_offsets, d_lengths, lanes, t);
-    } else if (force_generic == 6) {
+      break;
+    }
+    case LOOKAHEAD:
       same_dev::same_rx_la_kernel<<<fblocks, 32, 0, stream>>>(*p, *taps2, d_samples, d_offsets, d_lengths, lanes);
-    } else if (force_generic == 2) {
-      same_dev::same_rx_fast_kernel<false><<<fblocks, 32, 0, stream>>>(*p, *taps2, d_samples, d_offsets, d_lengths, lanes, t);
-    } else if (force_generic == 3) {
+      break;
+    case SINGLE:
+      same_dev::same_rx_fast_kernel<false><<<fblocks, 32, 0, stream>>>(*p, *taps2, d_samples, d_offsets, d_lengths, lanes, no_tiles);
+      break;
+    case PIPE: {
       // per device, cheap: set on every launch rather than tracking which devices have seen it
       cudaError_t e = cudaFuncSetAttribute(same_dev::same_rx_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                            PK_DYN_SMEM);
       if (e != cudaSuccess) return e;
       same_dev::same_rx_pipe_kernel<<<fblocks, PK_THREADS, PK_DYN_SMEM, stream>>>(*p, *taps2, d_samples, d_offsets,
                                                                                    d_lengths, lanes);
-    } else {
+      break;
+    }
+    case THREE:
       same_dev::same_rx_ws_kernel<<<fblocks, WS_THREADS, 0, stream>>>(*p, *taps2, d_samples, d_offsets, d_lengths, lanes);
+      break;
+    case GENERIC: {
+      const bool small = p->ntaps <= 64 && p->dc_len <= 16;
+      const size_t smem = small ? (size_t)(64 + 2 * 16) * 32 * sizeof(float) : (size_t)(128 + 2 * 64) * 32 * sizeof(float);
+      if (sample_fmt == 1) {
+        const float* f = static_cast<const float*>(d_samples_v);
+        if (small) same_dev::same_rx_generic_kernel<64, 16, float><<<blocks, 32, smem, stream>>>(*p, *taps, f, d_offsets, d_lengths);
+        else same_dev::same_rx_generic_kernel<128, 64, float><<<blocks, 32, smem, stream>>>(*p, *taps, f, d_offsets, d_lengths);
+      } else {
+        if (small) same_dev::same_rx_generic_kernel<64, 16, int16_t><<<blocks, 32, smem, stream>>>(*p, *taps, d_samples, d_offsets, d_lengths);
+        else same_dev::same_rx_generic_kernel<128, 64, int16_t><<<blocks, 32, smem, stream>>>(*p, *taps, d_samples, d_offsets, d_lengths);
+      }
+      break;
     }
-  } else {
-    const bool small = p->ntaps <= 64 && p->dc_len <= 16;
-    const size_t smem = small ? (size_t)(64 + 2 * 16) * 32 * sizeof(float) : (size_t)(128 + 2 * 64) * 32 * sizeof(float);
-    if (sample_fmt == 1) {
-      const float* f = static_cast<const float*>(d_samples_v);
-      if (small) same_dev::same_rx_generic_kernel<64, 16, float><<<blocks, 32, smem, stream>>>(*p, *taps, f, d_offsets, d_lengths);
-      else same_dev::same_rx_generic_kernel<128, 64, float><<<blocks, 32, smem, stream>>>(*p, *taps, f, d_offsets, d_lengths);
-    } else {
-      if (small) same_dev::same_rx_generic_kernel<64, 16, int16_t><<<blocks, 32, smem, stream>>>(*p, *taps, d_samples, d_offsets, d_lengths);
-      else same_dev::same_rx_generic_kernel<128, 64, int16_t><<<blocks, 32, smem, stream>>>(*p, *taps, d_samples, d_offsets, d_lengths);
-    }
+    default:
+      return cudaErrorInvalidValue;
   }
   return cudaGetLastError();
 }

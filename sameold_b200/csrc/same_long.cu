@@ -26,6 +26,7 @@
 #include <cuda_runtime.h>
 
 #include "same_fast.cuh"
+#include "same_internal.h"
 #include "same_lane.cuh"
 
 namespace same_dev {

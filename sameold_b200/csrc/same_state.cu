@@ -7,9 +7,13 @@
 //   scatter   records -> state32 + blobs (launched only after every record of the batch passed validation)
 // Word rows are moved through shared memory 32 streams x 32 words at a time: for a contiguous id run each row of a
 // tile is one 128-byte line of state32; for an arbitrary id list the same code gathers stream by stream.
+// The host half of the format, the header that names the configuration a state was produced under, is here too.
 #include <cuda_runtime.h>
 
-#include "same_params.h"
+#include <cstring>
+#include <string>
+
+#include "same_internal.h"
 
 namespace same_state {
 
@@ -178,11 +182,17 @@ __global__ void __launch_bounds__(kThreads) gather_kernel(const __grid_constant_
   }
 }
 
-// Failure codes of validate (0 = valid); the host names them (same_engine.cu: state_check_name)
+// Failure codes of validate (0 = valid), and their text in the same order
 enum Check : uint32_t {
   CK_OK = 0, CK_CRC, CK_REC_FLAGS, CK_FLAGS, CK_FRAMER, CK_TRANSPORT, CK_CLOCK, CK_TEDCNT, CK_BYTECLK, CK_SQ_HEAD,
-  CK_HIST_N, CK_HIST_LEN, CK_PENDING_LEN, CK_PENDING_KIND, CK_PENDING_ERR, CK_PENDING_OFFSET, CK_PREV_LEN
+  CK_HIST_N, CK_HIST_LEN, CK_PENDING_LEN, CK_PENDING_KIND, CK_PENDING_ERR, CK_PENDING_OFFSET, CK_PREV_LEN, CK_COUNT
 };
+const char* const kCheckNames[] = {
+    "valid", "CRC mismatch", "record flags (only bit 0 is defined)", "F_FLAGS (undefined bits)", "framer state > 2",
+    "transport state > 2", "F_CLOCK > 2^22", "F_TEDCNT not in {0, 1}", "F_SQ_BYTECLK not in -1..7", "F_SQ_HEAD >= 64",
+    "F_HIST_N > 3", "burst history length > 268", "pending length > 268", "pending kind > 2", "pending error > 3",
+    "pending_offset beyond the pending text", "previous-message length > 268"};
+static_assert(sizeof kCheckNames / sizeof kCheckNames[0] == CK_COUNT, "one text per Check code");
 
 // Every field a receiver kernel uses as an index, a length or a loop bound (same_lane.cuh, same_transport.cuh,
 // same_kernels.cu), checked against the range the kernels can produce themselves
@@ -254,30 +264,128 @@ __global__ void __launch_bounds__(kThreads) scatter_kernel(const __grid_constant
     warp_copy_blob(reinterpret_cast<uint8_t*>(p.blobs + stream_of(ids, first, r0 + r)), in + (size_t)(r0 + r) * g.bytes + g.blob_off);
 }
 
-// host CRC-32 (zlib) for the export header
-uint32_t crc32_host(const uint8_t* d, size_t n) {
-  static uint32_t t[256];
-  static bool init = false;
-  if (!init) {
-    for (uint32_t i = 0; i < 256; ++i) {
-      uint32_t c = i;
-      for (int k = 0; k < 8; ++k) c = (c & 1u) ? (c >> 1) ^ kCrcPoly : c >> 1;
-      t[i] = c;
-    }
-    init = true;
+// ---- header (host) ----
+
+struct CrcTable { uint32_t t[256]; };
+
+CrcTable make_crc_table() {
+  CrcTable tbl;
+  for (uint32_t i = 0; i < 256; ++i) {
+    uint32_t c = i;
+    for (int k = 0; k < 8; ++k) c = (c & 1u) ? (c >> 1) ^ kCrcPoly : c >> 1;
+    tbl.t[i] = c;
   }
+  return tbl;
+}
+
+// host CRC-32 (zlib) for the header
+uint32_t crc32_host(const uint8_t* d, size_t n) {
+  static const CrcTable tbl = make_crc_table();   // initialised once, thread-safe
   uint32_t c = 0xFFFFFFFFu;
-  for (size_t i = 0; i < n; ++i) c = t[(c ^ d[i]) & 0xffu] ^ (c >> 8);
+  for (size_t i = 0; i < n; ++i) c = tbl.t[(c ^ d[i]) & 0xffu] ^ (c >> 8);
   return ~c;
 }
+
+constexpr uint32_t kStMagic = 0x54534D53u;   // "SMST"
+constexpr uint32_t kStVersion = 1u;
+constexpr uint32_t kStBom = 0x01020304u;
+constexpr size_t kStOffConfig = 40, kStOffDerived = 116, kStOffMark = 164, kStOffSpace = 1188, kStOffCrc = 2220;
+static_assert(sizeof(same_config) == 19 * 4 && sizeof(same_derived) == 12 * 4, "4-byte fields only");
+static_assert(kStOffDerived == kStOffConfig + sizeof(same_config) && kStOffMark == kStOffDerived + sizeof(same_derived) &&
+              kStOffSpace == kStOffMark + 8 * SAME_MAX_TAPS && kStOffCrc + 4 == kHeaderBytes, "header layout");
+
+void put32(uint8_t* p, uint32_t v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); p[2] = (uint8_t)(v >> 16); p[3] = (uint8_t)(v >> 24); }
+uint32_t get32(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24); }
+// a struct of 4-byte fields <-> little-endian words
+void put_words(uint8_t* p, const void* src, size_t bytes) {
+  for (size_t i = 0; i < bytes; i += 4) { uint32_t v; memcpy(&v, static_cast<const uint8_t*>(src) + i, 4); put32(p + i, v); }
+}
+void get_words(void* dst, const uint8_t* p, size_t bytes) {
+  for (size_t i = 0; i < bytes; i += 4) { const uint32_t v = get32(p + i); memcpy(static_cast<uint8_t*>(dst) + i, &v, 4); }
+}
+
+const char* const kConfigFields[19] = {
+    "input_rate", "dc_blocker_len", "agc_bandwidth", "agc_gain_min", "agc_gain_max", "timing_bw_unlocked",
+    "timing_bw_locked", "timing_max_deviation", "squelch_power_open", "squelch_power_close", "squelch_bandwidth",
+    "preamble_max_errors", "eq_enabled", "eq_nff", "eq_nfb", "eq_relaxation", "eq_regularization",
+    "frame_prefix_max_errors", "frame_max_invalid_bytes"};
+const char* const kDerivedFields[12] = {"sps", "agc_bw", "agc_gain0", "samples_per_ted", "period_min", "period_max",
+                                        "alpha_unlocked", "beta_unlocked", "alpha_locked", "beta_locked", "dc_len", "ntaps"};
+
+Header make_header(const same_config& cfg, const same_derived& derived, const SameTaps& taps, uint32_t ntaps,
+                   uint32_t n_words, uint32_t n_records) {
+  Header s;
+  memset(&s, 0, sizeof s);
+  s.cfg = cfg; s.derived = derived;
+  s.n_records = n_records; s.n_words = n_words; s.record_bytes = same_state_record_bytes(n_words);
+  for (uint32_t i = 0; i < ntaps; ++i) {
+    const float v[4] = {taps.mark_re[i], taps.mark_im[i], taps.space_re[i], taps.space_im[i]};
+    put_words(s.taps + 8 * i, v, 8);
+    put_words(s.taps + 8 * SAME_MAX_TAPS + 8 * i, v + 2, 8);
+  }
+  return s;
+}
+
+void write_header(const Header& s, uint8_t* h) {
+  memset(h, 0, kHeaderBytes);
+  put32(h + 0, kStMagic); put32(h + 4, kStVersion); put32(h + 8, kStBom); put32(h + 12, (uint32_t)kHeaderBytes);
+  put32(h + 16, s.n_records); put32(h + 20, s.n_words); put32(h + 24, (uint32_t)sizeof(StreamBlob));
+  put32(h + 28, SAME_BURST_CAP); put32(h + 32, s.record_bytes);
+  put_words(h + kStOffConfig, &s.cfg, sizeof(same_config));
+  put_words(h + kStOffDerived, &s.derived, sizeof(same_derived));
+  memcpy(h + kStOffMark, s.taps, sizeof s.taps);
+  put32(h + kStOffCrc, crc32_host(h, kStOffCrc));
+}
+
+int parse_header(const void* buf, size_t len, Header* out, std::string* why) {
+  const uint8_t* h = static_cast<const uint8_t*>(buf);
+  auto bad = [&](const std::string& m) { *why = "state buffer: " + m; return (int)SAME_ERR_INVALID_ARG; };
+  if (!h) return bad("null pointer");
+  if (len < 16) return bad("truncated header");
+  if (get32(h) != kStMagic) return bad("bad magic");
+  if (get32(h + 8) != kStBom) return bad("wrong byte order");
+  if (get32(h + 4) != kStVersion) return bad("format version " + std::to_string(get32(h + 4)) + ", this library reads version " + std::to_string(kStVersion));
+  if (get32(h + 12) != kHeaderBytes) return bad("bad header size");
+  if (len < kHeaderBytes) return bad("truncated header");
+  if (get32(h + kStOffCrc) != crc32_host(h, kStOffCrc)) return bad("header CRC mismatch");
+  Header s;
+  s.n_records = get32(h + 16); s.n_words = get32(h + 20); s.record_bytes = get32(h + 32);
+  if (get32(h + 24) != sizeof(StreamBlob) || get32(h + 28) != SAME_BURST_CAP) return bad("stream blob layout differs from this library's");
+  if (s.n_words < F_NUM_SCALARS || s.n_words > (1u << 16) || s.record_bytes != same_state_record_bytes(s.n_words))
+    return bad("inconsistent record size");
+  const size_t need = kHeaderBytes + (size_t)s.n_records * s.record_bytes;
+  if (len < need) return bad("truncated: " + std::to_string(len) + " bytes, the header announces " + std::to_string(need));
+  if (len > need) return bad("trailing bytes after the last record");
+  get_words(&s.cfg, h + kStOffConfig, sizeof(same_config));
+  get_words(&s.derived, h + kStOffDerived, sizeof(same_derived));
+  memcpy(s.taps, h + kStOffMark, sizeof s.taps);
+  *out = s;
+  return SAME_OK;
+}
+
+// derived values and taps are compared bit for bit: they are libm results of the exporting host
+int compare_header(const Header& mine, const Header& s, std::string* why) {
+  uint32_t a[19], b[19];
+  memcpy(a, &mine.cfg, sizeof a); memcpy(b, &s.cfg, sizeof b);
+  for (int i = 0; i < 19; ++i)
+    if (a[i] != b[i]) { *why = std::string("state was produced under another configuration: ") + kConfigFields[i] + " differs"; return SAME_ERR_INVALID_CONFIG; }
+  uint32_t c[12], d[12];
+  memcpy(c, &mine.derived, sizeof c); memcpy(d, &s.derived, sizeof d);
+  for (int i = 0; i < 12; ++i)
+    if (c[i] != d[i]) { *why = std::string("derived constant ") + kDerivedFields[i] + " differs from this engine's (another host's libm?)"; return SAME_ERR_INVALID_CONFIG; }
+  if (memcmp(mine.taps, s.taps, 8 * SAME_MAX_TAPS) != 0) { *why = "mark filter taps differ from this engine's"; return SAME_ERR_INVALID_CONFIG; }
+  if (memcmp(mine.taps + 8 * SAME_MAX_TAPS, s.taps + 8 * SAME_MAX_TAPS, 8 * SAME_MAX_TAPS) != 0) {
+    *why = "space filter taps differ from this engine's"; return SAME_ERR_INVALID_CONFIG;
+  }
+  if (s.n_words != mine.n_words) { *why = "state words per stream differ from this engine's"; return SAME_ERR_INVALID_CONFIG; }
+  return SAME_OK;
+}
+
+const char* check_name(uint32_t code) { return code < CK_COUNT ? kCheckNames[code] : "invalid"; }
 
 }  // namespace same_state
 
 extern "C" uint32_t same_state_record_bytes(uint32_t n_words) { return same_state::rec_geom(n_words).bytes; }
-
-extern "C" uint32_t same_state_crc32(const void* data, size_t n) {
-  return same_state::crc32_host(static_cast<const uint8_t*>(data), n);
-}
 
 // ids == nullptr: the contiguous run first .. first+n-1
 extern "C" cudaError_t same_state_launch_gather(const SameParams* p, const uint32_t* d_ids, uint32_t first, uint32_t n,
