@@ -238,7 +238,7 @@ int same_engine_read_soft_trace(same_engine* e, uint32_t stream, same_soft_symbo
 /* Engine options (diagnostic; every setting must produce identical results, the tests cross-check them).  The library
  * reads no environment variables: this call is the only way to override the measured kernel policy.
  *   "kernel"          0 engine picks the kernel from the batch size (default); 1 rate-generic kernel even where the
- *                     22050 Hz fast kernels apply; 2 single-warp fast kernel; 3 four-warp pipelined kernel;
+ *                     22050 Hz fast kernels apply; 2 single-warp fast kernel; 3 five-warp pipelined kernel;
  *                     4 three-warp kernel; 5 split pipeline: the time-parallel front-end kernel (s16 -> exact DC-blocked
  *                     f32 tiles, HBM-bound) followed by the single-warp kernel fed from those tiles -- the measured
  *                     alternative to the fused kernels (DESIGN.md section 5); 6 look-ahead single-warp kernel (throughput
@@ -253,7 +253,8 @@ int same_engine_read_soft_trace(same_engine* e, uint32_t stream, same_soft_symbo
 int same_engine_set_option(same_engine* e, const char* key, int value);
 /* Reads an option back; additionally "kernel_selected": the kernel the next s16 submit will launch (1 generic,
  * 2 single-warp, 3 pipelined, 4 three-warp, 6 look-ahead single-warp) — the policy result for this batch size unless
- * "kernel" overrides it. */
+ * "kernel" overrides it; "rollbacks": how often the pipelined kernel's timing warp resumed a stream from a symbol whose
+ * symbol stages changed its state (sync found or end of a burst), counted up to the last sync (diagnostic). */
 int same_engine_get_option(same_engine* e, const char* key, int* value);
 
 /* Measurement aid: runs only the front-end kernel (feed-forward stages: s16 -> f32, DC blocker; 2 B read + 4 B written

@@ -146,6 +146,7 @@ struct same_engine {
   uint64_t ls_spec_launches = 0, ls_fallback_launches = 0;
   bool saw_f32 = false;           // an f32 submit happened since create / reset(all): DC state may be non-integer -> generic kernel
   uint64_t lost_events = 0, lost_payloads = 0;
+  uint64_t rollbacks = 0;          // option "rollbacks"
   same_derived derived;
   DevBuf<uint32_t> d_state;
   DevBuf<StreamBlob> d_blobs;
@@ -244,6 +245,7 @@ int collect(same_engine* e) {
   CK(e, cudaMemcpyAsync(e->h_counters, e->d_counters, 4 * sizeof(unsigned int), cudaMemcpyDeviceToHost, e->compute));
   CK(e, cudaStreamSynchronize(e->compute));
   const size_t nev = e->h_counters[0], npay = e->h_counters[1];
+  e->rollbacks += e->h_counters[3];
   const size_t events_cap = e->d_events.size(), payload_cap = e->d_payload.size();
   int rc = SAME_OK;
   if (nev > events_cap || e->h_counters[2] != 0) {
@@ -382,8 +384,8 @@ int run_long(same_engine* e, const int16_t* d_src, uint32_t len) {
 //  * the generic kernel for any geometry but the 22050 Hz class (42 taps, DC length 16), the fast kernels' only one;
 //  * option "kernel";
 //  * else the policy for the 22050 Hz class (measured on B200, tables in profiles/README.md), by 32-stream blocks per SM:
-//    * <= 1: four-warp pipelined kernel (producer / AGC / space filter / consumer), every warp on its own scheduler:
-//      the per-stream dependent chain is what bounds the run time, so it is cut into stages.
+//    * <= 1: five-warp pipelined kernel (producer / AGC / space filter / timing loop / symbol stages), the timing warp
+//      on a scheduler of its own: the per-stream dependent chain is what bounds the run time, so it is cut into stages.
 //    * <= 4: three-warp kernel (producer / look-ahead AGC / consumer): fewer instructions in total, still
 //      latency-hiding across the co-resident blocks.
 //    * <= 8: single-warp fast kernel (8 resident blocks per SM: the whole batch is one wave; fewest instructions).
@@ -922,6 +924,7 @@ int same_engine_get_option(same_engine* e, const char* key, int* value) {
   if (strcmp(key, "state_kernel_us") == 0) { *value = (int)std::min(e->st_kernel_ms * 1000.0f, 2.0e9f); return SAME_OK; }
   if (strcmp(key, "state_copy_us") == 0) { *value = (int)std::min(e->st_copy_ms * 1000.0f, 2.0e9f); return SAME_OK; }
   if (strcmp(key, "kernel_selected") == 0) { *value = rx_kernel(e); return SAME_OK; }
+  if (strcmp(key, "rollbacks") == 0) { *value = (int)std::min<uint64_t>(e->rollbacks, 0x7fffffff); return SAME_OK; }
   return fail(e, SAME_ERR_INVALID_ARG, std::string("unknown option ") + key);
 }
 

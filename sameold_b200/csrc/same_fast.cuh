@@ -221,4 +221,31 @@ __device__ __forceinline__ float agc_step(float& g, const float d, const float b
   return y;
 }
 
+// Ring counters between warps of one block (same_long_seq_kernel, same_rx_pipe_kernel).  LS_RELEASE_ACQUIRE=1:
+// st.release.cta / ld.acquire.cta, the hand-off the PTX memory model defines (the acquire load is a plain LDS in SASS,
+// the release store a MEMBAR.ALL.CTA + STS).  0: volatile accesses, relying on one
+// thread's shared-memory stores being performed in program order.  Both are bit-exact over 24 h
+// (tests/test_zz_config5_24h.py); profiles/README.md has the A/B.
+#ifndef LS_RELEASE_ACQUIRE
+#define LS_RELEASE_ACQUIRE 1
+#endif
+__device__ __forceinline__ void ls_publish(volatile uint32_t* w, uint32_t v) {
+#if LS_RELEASE_ACQUIRE
+  asm volatile("st.release.cta.shared.u32 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(const_cast<uint32_t*>(w))), "r"(v)
+               : "memory");
+#else
+  *w = v;
+#endif
+}
+__device__ __forceinline__ uint32_t ls_observe(const volatile uint32_t* w) {
+#if LS_RELEASE_ACQUIRE
+  uint32_t v;
+  asm volatile("ld.acquire.cta.shared.u32 %0, [%1];" : "=r"(v) : "r"((uint32_t)__cvta_generic_to_shared(const_cast<uint32_t*>(w)))
+               : "memory");
+  return v;
+#else
+  return *w;
+#endif
+}
+
 }  // namespace same_dev

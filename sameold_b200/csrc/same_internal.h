@@ -13,7 +13,7 @@
 
 // Receiver kernels.  The values are those of the engine option "kernel" (include/same_engine.h); POLICY lets the
 // engine choose from the batch size.  GENERIC takes any rate and s16 or f32 samples; the others are the fast kernels of
-// the 22050 Hz class: SINGLE single-warp, PIPE four-warp pipelined, THREE three-warp, SPLIT front-end kernel followed by
+// the 22050 Hz class: SINGLE single-warp, PIPE five-warp pipelined, THREE three-warp, SPLIT front-end kernel followed by
 // the single-warp kernel fed from its tiles, LOOKAHEAD look-ahead single-warp (16 resident warps per SM).
 enum Kernel { POLICY = 0, GENERIC = 1, SINGLE = 2, PIPE = 3, THREE = 4, SPLIT = 5, LOOKAHEAD = 6 };
 

@@ -28,7 +28,7 @@
 //   same_rx_fast_kernel     one warp per 32 streams (also in tile-fed form behind same_frontend_kernel)
 //   same_rx_la_kernel       one warp, DC + AGC in static chunks ahead of the timing loop: 16 resident warps per SM
 //   same_rx_ws_kernel       three warps: producer, look-ahead AGC, consumer
-//   same_rx_pipe_kernel     four warps: producer, free-running AGC, space filter, consumer
+//   same_rx_pipe_kernel     five warps: producer, free-running AGC, space filter, timing loop, symbol stages
 //   same_frontend_kernel    time-parallel feed-forward stages (A0 + A1) into lane-major f32 tiles, HBM-bound
 // The engine (same_engine.cu) picks one from the batch size; every kernel reads and writes the same resident state.
 #include <cuda_runtime.h>
@@ -750,8 +750,9 @@ __device__ __forceinline__ void ws_bar_sync(int id, int n = 64) { asm volatile("
 __device__ __forceinline__ void ws_bar_arrive(int id, int n = 64) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 
 // Producer warp of the warp-specialised kernels: raw s16 -> exact DC-blocked f32 into the d ring (A0, A1).  Each round:
-// wait for the consumer's position (bar_pos), refill every lane that has room for a whole 32-sample chunk, publish rp,
-// arrive on bar_data.  Stores the DC-blocker state of the lane when the consumer signals the end.
+// wait for the position the consumer may still need samples from (bar_pos), refill every lane that has room for a whole
+// 32-sample chunk, publish rp, arrive on bar_data.  Stores the DC-blocker state of the lane when the consumer signals the end.
+template <uint32_t DRING>   // d ring slots (power of two)
 __device__ __forceinline__ void ws_producer(const SameParams& p, uint32_t* st, const int16_t* src, const uint32_t len,
                                             const int lane, const bool valid, float* dring, volatile uint32_t* sh_rp,
                                             volatile uint32_t* sh_pos, volatile uint32_t* sh_done, const int bar_pos,
@@ -772,9 +773,9 @@ __device__ __forceinline__ void ws_producer(const SameParams& p, uint32_t* st, c
     first = false;
     const uint32_t cpos = sh_pos[lane];
     // every lane with room for a whole chunk takes one: afterwards it holds >= 32 samples, more than any segment
-    const bool take = (rp < len) && (rp - cpos) <= (uint32_t)(WS_DRING - FAST_CHUNK);
+    const bool take = (rp < len) && (rp - cpos) <= DRING - FAST_CHUNK;
     const uint32_t nnew = take ? min((uint32_t)FAST_CHUNK, len - rp) : 0u;
-    float* dst = dring + (rp & (WS_DRING - 1)) * 32 + lane;  // rp % 32 == 0: the chunk never wraps
+    float* dst = dring + (rp & (DRING - 1)) * 32 + lane;  // rp % 32 == 0: the chunk never wraps
     if (nnew == FAST_CHUNK) {
       uint32_t cur[FAST_CHUNK / 2];
       feed.take_full(cur, rp, len);
@@ -845,7 +846,7 @@ __global__ void __launch_bounds__(WS_THREADS, 4) same_rx_ws_kernel(const __grid_
   __syncthreads();
 
   if (role == 1) {
-    ws_producer(p, st, src, len, lane, valid, dring, sh_rp, sh_pos, &sh_done, WS_BAR_POS, WS_THREADS, WS_BAR_DATA, 64);
+    ws_producer<WS_DRING>(p, st, src, len, lane, valid, dring, sh_rp, sh_pos, &sh_done, WS_BAR_POS, WS_THREADS, WS_BAR_DATA, 64);
     return;
   }
 
@@ -971,42 +972,62 @@ __global__ void __launch_bounds__(WS_THREADS, 4) same_rx_ws_kernel(const __grid_
 }
 
 // ----------------------------------------------------------------------------------------------------------------
-// Pipelined kernel: the receiver of 32 streams spread over four warps (one per scheduler of the SM), so that the
-// per-round critical path is "segment bookkeeping -> one matched filter -> timing loop -> squelch / byte path".
+// Pipelined kernel: the receiver of 32 streams spread over five warps, so that the per-round critical path is
+// "segment bookkeeping -> one matched filter -> timing loop" and the symbol stages run beside it.
 //
-//   warp P   producer   raw s16 -> exact DC-blocked f32 (d ring)                                          A0, A1
-//   warp A   AGC        free-running gain recurrence, up to PK_LEAD samples ahead of the consumer:
+//   warp P   producer   raw s16 -> exact DC-blocked f32 (d ring), refilled up to PK_RING samples past the oldest
+//                       position the timing warp may still roll back to                                    A0, A1
+//   warp A   AGC        free-running gain recurrence, up to PK_LEAD samples ahead of the timing warp:
 //                       y ring + gain ring (gain after every sample)                                       A2, A3
-//   warp S   space      the space matched filter and its magnitude at the consumer's TED instant          A4
-//   warp F   consumer   picks the gain that belongs to its position, mark matched filter and magnitude,
-//                       timing loop, squelch, equalizer, framer, transport                                 A4-A9
+//   warp X   space      the space matched filter and its magnitude at the timing warp's TED instant        A4
+//   warp T   timing     picks the gain that belongs to its position, mark matched filter and magnitude,
+//                       timing loop; every symbol goes into a per-lane ring of records                     A4, A5
+//   warp Y   symbols    consumes each lane's records in order: squelch, equalizer, framer, transport       A6-A9
 //
-// The AGC depends on the consumer only through the lock flag (agc.rs:74), so it runs ahead speculatively and exactly:
-// whenever the consumer's flag flips, or the AGC warp has not got far enough, the consumer runs the recurrence itself
-// with the same arithmetic (fallback below) and tells the AGC warp to restart from its position and gain.
-// Lockstep rounds on four named barriers:
-//   F: sync DONE -> segment -> publish pos -> arrive POS -> publish (gain, flag, restart) -> arrive AGC -> mark
-//      -> sync SPACE -> TED, symbol
-//   S: sync POS -> space filter at pos -> arrive SPACE     P: sync POS -> refill -> arrive DONE
+// The AGC depends on the timing warp only through the lock flag (agc.rs:74), so it runs ahead speculatively and exactly:
+// whenever T's flag flips, or the AGC warp has not got far enough, T runs the recurrence itself with the same
+// arithmetic (fallback below) and tells the AGC warp to restart from its position and gain.
+// Lockstep rounds of P, A, X and T on four named barriers:
+//   T: sync DONE -> roll-back -> segment -> publish pos -> arrive POS -> publish (gain, flag, restart) -> arrive AGC
+//      -> mark -> sync SPACE -> TED, record
+//   X: sync POS -> space filter at pos -> arrive SPACE     P: sync POS -> refill -> arrive DONE
 //   A: sync AGC -> recurrence -> arrive DONE
+//
+// The symbol stages feed back into the timing loop only through SameReceiver::end() (TED state reset, locks cleared) and
+// an adjusted squelch acquire (AGC and bandwidth locked), receiver.rs:423-438, 479-490: a dozen symbols per stream-minute.
+// So T runs ahead of Y without waiting, each record carrying T's state right after that symbol's TED step.  Y never
+// speculates: its lane state is the sequential receiver's, and so is every global write it makes.  When Y's symbol k
+// changes what T uses, Y posts that state (a roll-back) and waits for that lane; T resumes the lane from symbol k with
+// it and drops the records it wrote after k.  Records carry no epoch: T publishes its head count together with the
+// number of roll-backs it applied, and Y reads a lane's records only once that number matches its own.
+// T waits for Y only when a lane's ring is full (PK_REC records) or the lane is PK_TLEAD samples past its oldest
+// unconfirmed symbol: the rings keep everything a roll-back needs (d from that symbol on, y from 42 samples before it).
 // ----------------------------------------------------------------------------------------------------------------
-#define PK_THREADS 128
-#define PK_YRING 128       // y ring slots, each mirrored at slot + 128 so that a 42-tap window never wraps (dynamic smem)
-#define PK_GRING 128       // gain ring slots (same indexing as the d and y rings: one running offset serves all three)
-#define PK_DYN_SMEM ((PK_GRING + 2 * PK_YRING) * 32 * 4)   // gain ring, y ring, y mirror: contiguous
-#define PK_LEAD 48         // the AGC warp stays at most this far ahead of the consumer
+#define PK_THREADS 160
+#define PK_RING 512        // d, gain and y ring slots (one running offset serves all three)
+#define PK_OMASK ((PK_RING - 1) * 128u)   // ring byte offset ((slot * 32 + lane) * 4) mask for the slot part
+#define PK_YMIRROR (FAST_NTAPS - 1)       // y slots 0..40 are mirrored at PK_RING + slot: a 42-tap window never wraps
+#ifndef PK_REC
+#define PK_REC 8           // records per lane: T's maximum lead over Y in symbols (power of two)
+#endif
+#define PK_TLEAD (PK_RING - 128)   // T's maximum lead in samples over its oldest unconfirmed symbol (see the AGC stores)
+#define PK_RECW 8          // words per record: pos, zero, sym, until, pavg, pinst, ted0, g
+#define PK_PARK 4          // Y rounds a squelched byte may wait for more lanes' bytes (the byte path runs once per warp)
+#define PK_DYN_SMEM ((3 * PK_RING + PK_YMIRROR) * 32 * 4 + PK_RECW * PK_REC * 32 * 4)   // gain | y + mirror | d | records
+#define PK_LEAD 48         // the AGC warp stays at most this far ahead of the timing warp
 #define PK_ADV 32          // ... and advances at most this much per round
-#define PK_BAR_POS 1       // F -> S, P        (96 threads)   position published
-#define PK_BAR_DONE 2      // A, P -> F        (96 threads)
-#define PK_BAR_SPACE 3     // S -> F           (64 threads)
-#define PK_BAR_AGC 4       // F -> A           (64 threads)   gain / flag / restart published
+#define PK_BAR_POS 1       // T -> X, P        (96 threads)   position published
+#define PK_BAR_DONE 2      // A, P -> T        (96 threads)
+#define PK_BAR_SPACE 3     // X -> T           (64 threads)
+#define PK_BAR_AGC 4       // T -> A           (64 threads)   gain / flag / restart published
+#define PK_LOCKS (FLAG_AGC_LOCKED | FLAG_BW_LOCKED)
 
 // |matched filter output| over the 42 samples that end at sample index `end` (exclusive); taps from the constant bank.
 // One rounded multiply and one rounded add per component and tap, newest sample first (demod.rs:156-163).
 __device__ __forceinline__ float pk_mag(const float* yring, const float2* __restrict__ h, const int lane,
                                         const uint32_t end, const float f_one, const float f_negzero) {
-  int nslot = (int)((end - 1u) & (PK_YRING - 1));
-  if (nslot < FAST_NTAPS - 1) nslot += PK_YRING;
+  int nslot = (int)((end - 1u) & (PK_RING - 1));
+  if (nslot < PK_YMIRROR) nslot += PK_RING;
   const float* yp = yring + nslot * 32 + lane;
   // packed exact f32 ops (see mf_soft): 3 instructions per tap instead of 5; measured 60.9 against 62.3 ms on config 3
   // although the dependent FFMA2 chain is slower per step than FADD (6 against 4 cycles) -- the warp was issue-bound
@@ -1020,29 +1041,44 @@ __device__ __forceinline__ float pk_mag(const float* yring, const float2* __rest
   return hypot_fixed(acc.x, acc.y);
 }
 
-// one block per SM at most (engine policy): every register the role code wants
+// y of ring byte offset o (slot * 128 + lane * 4) into the y ring, and into its mirror for slots 0..40
+__device__ __forceinline__ void pk_store_y(const uint32_t y_lane, const uint32_t o, const float y) {
+  asm volatile("{\n\t.reg .pred m;\n\tsetp.lt.u32 m, %1, %3;\n\tst.shared.f32 [%0], %2;\n\t@m st.shared.f32 [%0+%4], %2;\n\t}"
+               ::"r"(y_lane + o), "r"(o), "f"(y), "n"(PK_YMIRROR * 128), "n"(PK_RING * 128) : "memory");
+}
+
+// one block per SM at most (engine policy): every register the role code wants.  Warp i runs on scheduler i mod 4:
+// T has one to itself, Y shares one with the producer, which waits most of the time.
 __global__ void __launch_bounds__(PK_THREADS, 1) same_rx_pipe_kernel(const __grid_constant__ SameParams p,
                                                                   const __grid_constant__ SameTaps2 taps,
                                                                   const int16_t* __restrict__ samples,
                                                                   const unsigned long long* __restrict__ offsets,
                                                                   const uint32_t* __restrict__ lengths,
                                                                   const uint32_t lanes) {
-  extern __shared__ float pk_dyn[];           // gring[128][32], yring[2 * 128][32]: one address register serves all
+  // gring[PK_RING][32] | yring[PK_RING + PK_YMIRROR][32] | dring[PK_RING][32] | rec[PK_RECW][PK_REC][32]
+  extern __shared__ float pk_dyn[];
   float* const gring = pk_dyn;
-  float* const yring = pk_dyn + PK_GRING * 32;
-  __shared__ float dring[WS_DRING * 32];
-  __shared__ volatile float sh_space[32];    // |space filter| at pos                  (S)
-  __shared__ volatile uint32_t sh_rp[32];    // samples produced per lane              (P)
-  __shared__ volatile uint32_t sh_apos[32];  // samples AGC'd per lane                 (A)
-  __shared__ volatile uint32_t sh_pos[32];   // samples consumed per lane              (F)
-  __shared__ volatile float sh_g[32];        // AGC gain at pos                        (F)
-  __shared__ volatile uint32_t sh_rq[32];    // bit 0 restart the AGC at pos, bit 1 AGC locked   (F)
-  __shared__ volatile uint32_t sh_frp[32];   // rp as the consumer saw it at the top of the round  (F)
+  float* const yring = gring + PK_RING * 32;
+  float* const dring = yring + (PK_RING + PK_YMIRROR) * 32;
+  float* const rec = dring + PK_RING * 32;
+  __shared__ volatile float sh_space[32];    // |space filter| at pos                                (X)
+  __shared__ volatile uint32_t sh_rp[32];    // samples produced per lane                            (P)
+  __shared__ volatile uint32_t sh_apos[32];  // samples AGC'd per lane                               (A)
+  __shared__ volatile uint32_t sh_pos[32];   // samples consumed per lane                            (T)
+  __shared__ volatile uint32_t sh_low[32];   // oldest position T may roll back to: P refills from it (T)
+  __shared__ volatile float sh_g[32];        // AGC gain at pos                                      (T)
+  __shared__ volatile uint32_t sh_rq[32];    // bit 0 restart the AGC at pos, bit 1 AGC locked       (T)
+  __shared__ volatile uint32_t sh_frp[32];   // rp as T saw it at the top of the round               (T)
+  __shared__ volatile uint32_t sh_head[32];  // records written (low 16 bits) | roll-backs applied << 16   (T)
+  __shared__ volatile uint32_t sh_tail[32];  // records confirmed (low 16 bits)                      (Y)
+  __shared__ volatile uint32_t sh_rbreq[32]; // roll-backs requested (low 16 bits)                   (Y)
+  __shared__ volatile uint32_t sh_rb[10][32];   // roll-back: pos, g, until, pavg, pinst, ted0..2, tedcnt | locks, head (Y)
+  __shared__ volatile uint32_t sh_fin[10][32];  // T's state at the end: pos, g, clock, until, pavg, pinst, ted0..2, tedcnt
   __shared__ volatile uint32_t sh_done;
 
   const SameLayout& L = p.layout;
   const int lane = threadIdx.x & 31;
-  enum { R_F = 0, R_S = 1, R_A = 2, R_P = 3 };
+  enum { R_Y = 0, R_T = 1, R_X = 2, R_A = 3, R_P = 4 };
   const int role = threadIdx.x >> 5;
   const uint32_t s = blockIdx.x * lanes + lane;
   const bool valid = (uint32_t)lane < lanes && s < p.n_streams;
@@ -1055,33 +1091,39 @@ __global__ void __launch_bounds__(PK_THREADS, 1) same_rx_pipe_kernel(const __gri
   const int16_t* src = (samples != nullptr && valid) ? samples + offsets[s] : nullptr;
 
   // ---- shared set-up ----
-  for (int i = role; i < WS_DRING; i += 4) dring[i * 32 + lane] = 0.0f;   // stale slots are read, never used: keep them finite
-  if (role == R_F) {
-    for (int i = 0; i < FAST_NTAPS; ++i) {   // demod window -> y ring slots of samples -42..-1 (86..127: no mirror)
+  for (int i = role; i < PK_RING; i += 5) dring[i * 32 + lane] = 0.0f;   // stale slots are read, never used: keep them finite
+  if (role == R_T) {
+    for (int i = 0; i < FAST_NTAPS; ++i) {   // demod window -> y ring slots of samples -42..-1 (470..511: no mirror)
       const float v = __uint_as_float(LANE_ST(st, L, L.win + i));
-      yring[((i - FAST_NTAPS) & (PK_YRING - 1)) * 32 + lane] = v;
+      yring[((i - FAST_NTAPS) & (PK_RING - 1)) * 32 + lane] = v;
     }
     sh_pos[lane] = 0u;
+    sh_low[lane] = 0u;
+    sh_head[lane] = 0u;
     if (lane == 0) sh_done = 0u;
   } else if (role == R_A) {
     sh_apos[lane] = 0u;
-    for (int i = 0; i < PK_YRING - FAST_NTAPS; ++i) yring[i * 32 + lane] = 0.0f;   // keep never-written slots finite
-  } else if (role == R_S) {
-    for (int i = 0; i < PK_YRING; ++i) yring[(PK_YRING + i) * 32 + lane] = 0.0f;
+    for (int i = 0; i < PK_RING - FAST_NTAPS; ++i) yring[i * 32 + lane] = 0.0f;   // keep never-written slots finite
+  } else if (role == R_X) {
+    for (int i = 0; i < PK_YMIRROR; ++i) yring[(PK_RING + i) * 32 + lane] = 0.0f;
     sh_space[lane] = 0.0f;
+  } else if (role == R_Y) {
+    sh_tail[lane] = 0u;
+    sh_rbreq[lane] = 0u;
   } else {
     sh_rp[lane] = 0u;
   }
   __syncthreads();
 
   if (role == R_P) {
-    ws_producer(p, st, src, len, lane, valid, dring, sh_rp, sh_pos, &sh_done, PK_BAR_POS, 96, PK_BAR_DONE, 96);
+    ws_producer<PK_RING>(p, st, src, len, lane, valid, dring, sh_rp, sh_low, &sh_done, PK_BAR_POS, 96, PK_BAR_DONE, 96);
     return;
   }
 
   const float bw = p.agc_bw, gmin = p.agc_min, gmax = p.agc_max;
   const uint32_t d_lane = smem_u32(dring) + ((uint32_t)lane << 2);
   const uint32_t g_lane = smem_u32(gring) + ((uint32_t)lane << 2);
+  const uint32_t y_lane = smem_u32(yring) + ((uint32_t)lane << 2);
 
   if (role == R_A) {
     // ================================================= AGC =================================================
@@ -1103,26 +1145,27 @@ __global__ void __launch_bounds__(PK_THREADS, 1) same_rx_pipe_kernel(const __gri
       // 8 samples per step, the d values of the next step prefetched.  One running byte offset (ring slot * 128 +
       // lane * 4) addresses all three rings.  Every lane stores all nmax (rounded up to 8) samples: what lies beyond
       // its own n is overwritten with the right values before anything reads it, and lands at most 79 samples ahead
-      // of the consumer, which aliases nothing live in 128-slot rings (the demod window reaches back 42 samples).
+      // of T.  T stays within PK_TLEAD = PK_RING - 128 samples of its oldest unconfirmed symbol, so these stores never
+      // reach the 42 samples before that symbol, which a roll-back needs.
       // Software pipeline, distance 2: the d value of sample j+2 is loaded right after the stores of sample j-1.
       // The explicit shared-memory accesses keep their program order, so the stores have to issue in the shadow of
       // the gain chain (one dependent op every 4-5 cycles) instead of in a bunch after it.
-      uint32_t o0 = (apos & (WS_DRING - 1)) << 7, o1 = (o0 + 128u) & 0x3f80u;
+      uint32_t o0 = (apos & (PK_RING - 1)) << 7, o1 = (o0 + 128u) & PK_OMASK;
       float d0 = lds_f32(d_lane + o0), d1 = lds_f32(d_lane + o1);
       for (int k = 0; k < nmax; k += 8) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
-          const uint32_t o2 = (o1 + 128u) & 0x3f80u;
+          const uint32_t o2 = (o1 + 128u) & PK_OMASK;
           const float d2 = lds_f32(d_lane + o2);
           const float y = agc_step(g, d0, bw_eff, gmin, gmax);                            // agc.rs:72-77
-          asm volatile("st.shared.f32 [%0], %1;\n\tst.shared.f32 [%0+16384], %2;\n\tst.shared.f32 [%0+32768], %2;"
-                       ::"r"(g_lane + o0), "f"(g), "f"(y) : "memory");                     // gain | y | y mirror
+          asm volatile("st.shared.f32 [%0], %1;" ::"r"(g_lane + o0), "f"(g) : "memory");
+          pk_store_y(y_lane, o0, y);
           o0 = o1; o1 = o2; d0 = d1; d1 = d2;
         }
       }
       if (n > 0) {
         apos += (uint32_t)n;
-        ag = gring[((apos - 1u) & (PK_GRING - 1)) * 32 + lane];         // the gain after this lane's last sample
+        ag = gring[((apos - 1u) & (PK_RING - 1)) * 32 + lane];          // the gain after this lane's last sample
       }
       sh_apos[lane] = apos;
       __threadfence_block();
@@ -1131,7 +1174,7 @@ __global__ void __launch_bounds__(PK_THREADS, 1) same_rx_pipe_kernel(const __gri
     return;
   }
 
-  if (role == R_S) {
+  if (role == R_X) {
     // ============================================== space filter ==============================================
     while (true) {
       ws_bar_sync(PK_BAR_POS, 96);
@@ -1143,59 +1186,156 @@ __global__ void __launch_bounds__(PK_THREADS, 1) same_rx_pipe_kernel(const __gri
     return;
   }
 
-  // ================================================= consumer =================================================
+  if (role == R_Y) {
+    // ============================================== symbol stages ==============================================
+    Lane a;
+    lane_load(a, p, st, s);
+    uint32_t tail = 0, ep = 0;   // records confirmed; roll-backs requested
+    bool wait_ack = false;       // a roll-back is posted and T has not applied it yet: consume nothing of this lane
+    uint32_t park = 0;           // SYM_BYTE_READY | SYM_ADJUSTED of a symbol whose byte path waits (see PK_PARK)
+    uint32_t r_pos = 0, r_lock = 0;
+    float r_g = 0.0f;
+    int age = 0;
+    while (true) {
+      const uint32_t hw = sh_head[lane];
+      if (wait_ack && (hw >> 16) == (ep & 0xffffu)) {      // T resumed from the roll-back's symbol: it is confirmed
+        wait_ack = false;
+        tail += 1u;
+        ls_publish(&sh_tail[lane], tail & 0xffffu);
+      }
+      const bool have = !wait_ack && park == 0u && (hw >> 16) == (ep & 0xffffu) && ((hw - tail) & 0xffffu) != 0u;
+      const bool any_have = __any_sync(0xffffffffu, have);
+      const bool any_park = __any_sync(0xffffffffu, park != 0u);
+      if (!any_have && !any_park) {
+        if (sh_done) break;   // T finishes only when every record is confirmed
+        continue;
+      }
+      bool sym_done = false;
+      if (any_have) {
+        __threadfence_block();   // with T's fence before the head word: the records are complete
+        if (have) {
+          const float* q = rec + (tail & (PK_REC - 1)) * 32 + lane;
+          r_pos = __float_as_uint(q[0]);
+          const float zero = q[1 * PK_REC * 32], sym = q[2 * PK_REC * 32];
+          a.until = q[3 * PK_REC * 32]; a.pavg = q[4 * PK_REC * 32]; a.pinst = q[5 * PK_REC * 32];
+          a.ted0 = q[6 * PK_REC * 32]; a.ted1 = zero; a.ted2 = sym; a.tedcnt = 1u;
+          r_g = q[7 * PK_REC * 32];
+          r_lock = a.flags & PK_LOCKS;
+          park = symbol_squelch(a, p, s, st, blob, zero, sym, a.n0 + r_pos);
+          sym_done = park == 0u;
+        }
+      }
+      // the byte path of parked lanes: when no lane has a new record, or after PK_PARK rounds
+      if (__any_sync(0xffffffffu, park != 0u) && (!any_have || ++age >= PK_PARK)) {
+        age = 0;
+        if (park != 0u) {
+          symbol_byte(a, p, s, st, blob, (park & SYM_ADJUSTED) != 0u, a.n0 + r_pos);
+          park = 0u;
+          sym_done = true;
+        }
+      }
+      if (sym_done) {
+        if ((a.flags & PK_LOCKS) != r_lock || a.tedcnt != 1u) {
+          // end() or an adjusted acquire changed the timing loop's state: T resumes from this symbol with it
+          sh_rb[0][lane] = r_pos; sh_rb[1][lane] = __float_as_uint(r_g); sh_rb[2][lane] = __float_as_uint(a.until);
+          sh_rb[3][lane] = __float_as_uint(a.pavg); sh_rb[4][lane] = __float_as_uint(a.pinst);
+          sh_rb[5][lane] = __float_as_uint(a.ted0); sh_rb[6][lane] = __float_as_uint(a.ted1);
+          sh_rb[7][lane] = __float_as_uint(a.ted2); sh_rb[8][lane] = a.tedcnt | (a.flags & PK_LOCKS) << 16;
+          sh_rb[9][lane] = (tail + 1u) & 0xffffu;
+          ep += 1u;
+          ls_publish(&sh_rbreq[lane], ep & 0xffffu);
+          wait_ack = true;
+          atomicAdd(&p.counters[3], 1u);
+        } else {
+          tail += 1u;
+          ls_publish(&sh_tail[lane], tail & 0xffffu);
+        }
+      }
+    }
+    if (!valid || len == 0u) return;
+    __threadfence_block();
+    const uint32_t pos = sh_fin[0][lane];
+    a.g = __uint_as_float(sh_fin[1][lane]); a.clock = (int)sh_fin[2][lane];
+    a.until = __uint_as_float(sh_fin[3][lane]); a.pavg = __uint_as_float(sh_fin[4][lane]);
+    a.pinst = __uint_as_float(sh_fin[5][lane]); a.ted0 = __uint_as_float(sh_fin[6][lane]);
+    a.ted1 = __uint_as_float(sh_fin[7][lane]); a.ted2 = __uint_as_float(sh_fin[8][lane]); a.tedcnt = sh_fin[9][lane];
+    lane_store(a, p, st, a.n0 + pos);
+    for (int i = 0; i < FAST_NTAPS; ++i)
+      LANE_ST(st, L, L.win + i) = __float_as_uint(yring[((int)(pos + i - FAST_NTAPS) & (PK_RING - 1)) * 32 + lane]);
+    return;
+  }
+
+  // ================================================= timing =================================================
   Lane a;
   lane_load(a, p, st, s);
   uint32_t pos = 0;
   int cfire = fire_clock(a.until, a.clock);
-  uint32_t pend = 0;       // SYM_BYTE_READY | SYM_ADJUSTED while parked (byte-phase alignment, see same_rx_fast_kernel)
   uint32_t round_ctr = 0;
-  bool la_valid = false;   // the AGC warp's chain continues this lane's exact state under the current lock flag
+  uint32_t head = 0, ep = 0;   // records written; roll-backs applied
+  bool la_valid = false;       // the AGC warp's chain continues this lane's exact state under the current lock flag
 
   while (true) {
     ws_bar_sync(PK_BAR_DONE, 96);           // refill and AGC of the previous round are complete and visible
-    if (!__any_sync(0xffffffffu, pos < len || pend != 0u)) {
-      if (lane == 0) sh_done = 1u;
+    // ---------------- roll-back: resume from the symbol Y names, with the state its symbol stages left ----------------
+    const uint32_t rq_ep = sh_rbreq[lane];
+    const bool rb = rq_ep != ep;
+    if (__any_sync(0xffffffffu, rb)) {
       __threadfence_block();
-      ws_bar_arrive(PK_BAR_POS, 96);
-      ws_bar_arrive(PK_BAR_AGC, 64);
-      break;
+      if (rb) {
+        pos = sh_rb[0][lane]; a.g = __uint_as_float(sh_rb[1][lane]); a.until = __uint_as_float(sh_rb[2][lane]);
+        a.pavg = __uint_as_float(sh_rb[3][lane]); a.pinst = __uint_as_float(sh_rb[4][lane]);
+        a.ted0 = __uint_as_float(sh_rb[5][lane]); a.ted1 = __uint_as_float(sh_rb[6][lane]);
+        a.ted2 = __uint_as_float(sh_rb[7][lane]);
+        const uint32_t w = sh_rb[8][lane];
+        a.tedcnt = w & 0xffffu;
+        a.flags = (a.flags & ~PK_LOCKS) | (w >> 16);
+        head = sh_rb[9][lane];
+        a.clock = 0;                         // the symbol's TED instant, where cfire was computed (before end())
+        cfire = fire_clock(a.until, 0);
+        la_valid = false;
+        ep = rq_ep;
+      }
     }
+    const uint32_t tail = sh_tail[lane];
+    const uint32_t inflight = (head - tail) & 0xffffu;
+    if (!__any_sync(0xffffffffu, pos < len || inflight != 0u)) break;
+    const uint32_t low = inflight ? __float_as_uint(rec[(tail & (PK_REC - 1)) * 32 + lane]) : pos;
     // ---------------- segment: this lane's samples up to its next TED instant (A2, A3) ----------------
     const uint32_t rp = sh_rp[lane];
     const uint32_t apos = sh_apos[lane];
     int nseg = 0;
     round_ctr += 1;
-    const bool byte_round = (round_ctr & 15u) == 0u;
-    if (pos < len && pend == 0u) nseg = min(cfire - a.clock, (int)(rp - pos));
-    if (((a.tedcnt ^ round_ctr) & 1u) != 0u) nseg = 0;   // TED-phase alignment (see same_rx_fast_kernel)
+    if (pos < len && inflight < (uint32_t)PK_REC)
+      nseg = min(min(cfire - a.clock, (int)(rp - pos)), (int)(low + PK_TLEAD - pos));
+    if (((a.tedcnt ^ round_ctr) & 1u) != 0u) nseg = 0;   // TED-phase alignment: Y gets the lanes' records together
     const uint32_t lock_now = a.flags & FLAG_AGC_LOCKED;
     const bool use_la = la_valid && (int)(apos - pos) >= nseg;
     const bool need_fb = nseg > 0 && !use_la;
     if (__any_sync(0xffffffffu, need_fb)) {
-      // fallback: run the recurrence here (start of a chunk, after a lock flip, AGC warp not far enough)
+      // fallback: run the recurrence here (start of a chunk, after a roll-back, AGC warp not far enough)
       const int nfb = __reduce_max_sync(0xffffffffu, need_fb ? nseg : 0);
       const float bw_eff = lock_now ? 0.0f : bw;
       float g = a.g;
       for (int k = 0; k < nfb; ++k) {
         const bool act = need_fb && k < nseg;
-        const float dv = lds_f32(d_lane + (((pos + (uint32_t)k) & (WS_DRING - 1)) << 7));
+        const uint32_t o = ((pos + (uint32_t)k) & (PK_RING - 1)) << 7;
+        const float dv = lds_f32(d_lane + o);
         float gn = g;
         const float y = agc_step(gn, dv, bw_eff, gmin, gmax);
         if (act) {
           g = gn;
-          const uint32_t slot = (pos + (uint32_t)k) & (PK_YRING - 1);
-          yring[slot * 32 + lane] = y;
-          yring[(slot + PK_YRING) * 32 + lane] = y;
+          pk_store_y(y_lane, o, y);
         }
       }
       if (need_fb) a.g = g;
     }
     // the position first: it is all the space-filter and producer warps wait for
     sh_pos[lane] = pos + (uint32_t)nseg;
+    sh_low[lane] = low;
     __threadfence_block();
+    sh_head[lane] = (head & 0xffffu) | (ep << 16);   // the records of earlier rounds, behind the fence above
     ws_bar_arrive(PK_BAR_POS, 96);
-    if (use_la && nseg > 0) a.g = lds_f32(g_lane + (((pos + (uint32_t)nseg - 1u) & (PK_GRING - 1)) << 7));
+    if (use_la && nseg > 0) a.g = lds_f32(g_lane + (((pos + (uint32_t)nseg - 1u) & (PK_RING - 1)) << 7));
     pos += (uint32_t)nseg;
     a.clock += nseg;
     const bool fire = (nseg > 0) && (a.clock == cfire);
@@ -1207,7 +1347,7 @@ __global__ void __launch_bounds__(PK_THREADS, 1) same_rx_pipe_kernel(const __gri
     __threadfence_block();
     ws_bar_arrive(PK_BAR_AGC, 64);
 
-    // ---------------- TED instant (A4, A5): mark here, space from warp S ----------------
+    // ---------------- TED instant (A4, A5): mark here, space from warp X ----------------
     // what the timing loop needs besides the soft symbol is computed first, off the critical path
     const float rem = FSUB(a.until, (float)a.clock);                         // receiver.rs:352
     const float off = rclamp(rem, -0.5f, 0.5f);                              // symsync.rs:220
@@ -1216,29 +1356,30 @@ __global__ void __launch_bounds__(PK_THREADS, 1) same_rx_pipe_kernel(const __gri
     const float mag_m = pk_mag(yring, taps.mark, lane, pos, p.f_one, p.f_negzero);
     asm volatile("" ::"f"(mag_m));          // keep the mark magnitude ahead of the wait for the space magnitude
     ws_bar_sync(PK_BAR_SPACE, 64);
-    bool have_sym = false;
     if (fire) {
       const float soft = rclamp(FSUB(mag_m, sh_space[lane]), -1.0f, 1.0f);   // demod.rs:163
       a.clock = 0;
-      have_sym = ted_step(a, p, soft, off, offq);
+      if (ted_step(a, p, soft, off, offq)) {
+        float* q = rec + (head & (PK_REC - 1)) * 32 + lane;                   // published with the next round's head
+        q[0] = __uint_as_float(pos); q[1 * PK_REC * 32] = a.ted1; q[2 * PK_REC * 32] = a.ted2;
+        q[3 * PK_REC * 32] = a.until; q[4 * PK_REC * 32] = a.pavg; q[5 * PK_REC * 32] = a.pinst;
+        q[6 * PK_REC * 32] = a.ted0; q[7 * PK_REC * 32] = a.g;
+        head += 1u;
+      }
       cfire = fire_clock(a.until, 0);
     }
-    // ---------------- symbol: squelch now (A6), byte path (A7-A9) on the aligned rounds ----------------
-    if (have_sym) pend = symbol_squelch(a, p, s, st, blob, a.ted1, a.ted2, a.n0 + pos);
-    if (byte_round && __any_sync(0xffffffffu, pend != 0u)) {
-      if (pend != 0u) {
-        symbol_byte(a, p, s, st, blob, (pend & SYM_ADJUSTED) != 0u, a.n0 + pos);
-        pend = 0u;
-      }
-    }
-    // a flipped lock flag invalidates what the AGC warp computed from pos on
-    if ((a.flags & FLAG_AGC_LOCKED) != lock_now) la_valid = false;
   }
 
-  if (!valid || len == 0u) return;
-  lane_store(a, p, st, a.n0 + pos);
-  for (int i = 0; i < FAST_NTAPS; ++i)
-    LANE_ST(st, L, L.win + i) = __float_as_uint(yring[((int)(pos + i - FAST_NTAPS) & (PK_YRING - 1)) * 32 + lane]);
+  // every record is confirmed and no roll-back is pending: hand the timing state to Y, which stores the lane
+  sh_fin[0][lane] = pos; sh_fin[1][lane] = __float_as_uint(a.g); sh_fin[2][lane] = (uint32_t)a.clock;
+  sh_fin[3][lane] = __float_as_uint(a.until); sh_fin[4][lane] = __float_as_uint(a.pavg);
+  sh_fin[5][lane] = __float_as_uint(a.pinst); sh_fin[6][lane] = __float_as_uint(a.ted0);
+  sh_fin[7][lane] = __float_as_uint(a.ted1); sh_fin[8][lane] = __float_as_uint(a.ted2); sh_fin[9][lane] = a.tedcnt;
+  __threadfence_block();
+  if (lane == 0) sh_done = 1u;
+  __threadfence_block();
+  ws_bar_arrive(PK_BAR_POS, 96);
+  ws_bar_arrive(PK_BAR_AGC, 64);
 }
 
 // Constructor state (receiver.rs:502-560) or SameReceiver::reset (receiver.rs:182-198) for the selected streams.

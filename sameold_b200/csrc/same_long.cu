@@ -164,37 +164,12 @@ __global__ void __launch_bounds__(256) same_long_mf_kernel(const __grid_constant
 #define LS_RING 64
 struct LsRec { uint32_t pos; float zero, sym, until, pavg, pinst, ted0; uint32_t pad; };
 
-// Ring counters.  LS_RELEASE_ACQUIRE=1: st.release.cta / ld.acquire.cta, the hand-off the PTX memory model defines (the
-// acquire load is a plain LDS in SASS, the release store a MEMBAR.ALL.CTA + STS).  0: volatile accesses, relying on one
-// thread's shared-memory stores being performed in program order.  Both are bit-exact over 24 h
-// (tests/test_zz_config5_24h.py); profiles/README.md has the A/B.
-#ifndef LS_RELEASE_ACQUIRE
-#define LS_RELEASE_ACQUIRE 1
-#endif
 // The counters are published in batches (the release store's MEMBAR is what costs): T every LS_HEAD_BATCH records and
 // when it finishes, S every LS_TAIL_BATCH records and whenever it has drained the ring.
 #ifndef LS_HEAD_BATCH
 #define LS_HEAD_BATCH 4u
 #endif
 #define LS_TAIL_BATCH 8u
-__device__ __forceinline__ void ls_publish(volatile uint32_t* w, uint32_t v) {
-#if LS_RELEASE_ACQUIRE
-  asm volatile("st.release.cta.shared.u32 [%0], %1;" ::"r"((uint32_t)__cvta_generic_to_shared(const_cast<uint32_t*>(w))), "r"(v)
-               : "memory");
-#else
-  *w = v;
-#endif
-}
-__device__ __forceinline__ uint32_t ls_observe(const volatile uint32_t* w) {
-#if LS_RELEASE_ACQUIRE
-  uint32_t v;
-  asm volatile("ld.acquire.cta.shared.u32 %0, [%1];" : "=r"(v) : "r"((uint32_t)__cvta_generic_to_shared(const_cast<uint32_t*>(w)))
-               : "memory");
-  return v;
-#else
-  return *w;
-#endif
-}
 
 __global__ void __launch_bounds__(64) same_long_seq_kernel(const __grid_constant__ SameParams p, const float* __restrict__ soft,
                                                            const float* __restrict__ yfull, const float* __restrict__ gspec,

@@ -122,7 +122,8 @@ struct SameParams {
   // output arenas
   same_event* events;
   uint8_t* payload;
-  unsigned int* counters;         // [0] events appended, [1] payload bytes appended, [2] payloads dropped (arena full)
+  unsigned int* counters;         // [0] events appended, [1] payload bytes appended, [2] payloads dropped (arena full),
+                                  // [3] roll-backs of the pipelined kernel (same_rx_pipe_kernel)
   uint32_t events_cap, payload_cap;
   same_soft_symbol* trace;        // [n_streams][trace_cap] or null
   uint32_t trace_cap;
