@@ -141,7 +141,9 @@ struct same_engine {
   // long-stream path (same_long.cu): one stream, long chunks
   int long_stream = 1;            // option "long_stream"
   DevBuf<float> ls_d, ls_y, ls_g, ls_soft, ls_gin;
-  DevBuf<uint32_t> ls_ctrl;       // {verified end, position reached, reason, -}
+  DevBuf<uint32_t> ls_ctrl;       // {verified end, position reached, reason, span length}
+  DevBuf<unsigned long long> ls_off;   // offset of an unverified span in the chunk (ordinary-kernel launch)
+  DevBuf<uint32_t> ls_dc_at;      // DC-blocker state at the start of an unverified span (34 words, word-major)
   PinnedBuf<uint32_t> ls_hctrl;   // mirror + scratch
   uint64_t ls_spec_launches = 0, ls_fallback_launches = 0;
   bool saw_f32 = false;           // an f32 submit happened since create / reset(all): DC state may be non-integer -> generic kernel
@@ -324,6 +326,8 @@ int ensure_tiles(same_engine* e, uint32_t max_len) {
 constexpr uint32_t kLongMinSamples = 65536;     // shorter chunks take the ordinary kernels
 constexpr uint32_t kLongChunk = 1u << 24;       // samples per internal pass (bounds the scratch buffers: 16 B per sample)
 constexpr uint32_t kLongSpan = 8192;            // samples per fallback launch while the AGC is locked (inside a burst)
+constexpr uint32_t kLongSpanMax = 1u << 20;     // longest fallback span after verification stops in a row
+constexpr uint32_t kLongMinPass = 1u << 16;     // shortest range of a speculative pass
 
 int ensure_long(same_engine* e, size_t n) {
   CK(e, e->ls_d.grow(n + 64));
@@ -333,22 +337,52 @@ int ensure_long(same_engine* e, size_t n) {
   CK(e, e->ls_gin.grow(n / 2048 + 8));
   CK(e, e->ls_ctrl.grow(4));
   CK(e, e->ls_hctrl.grow(8));
+  CK(e, e->ls_off.grow(1));
+  CK(e, e->ls_dc_at.grow((size_t)34 * e->p.layout.n_pad));
   CK(e, e->tiles_dc_next.grow((size_t)34 * e->p.layout.n_pad));
   bind(e);
   return SAME_OK;
 }
 
 // One stream, `len` device-resident s16 samples, on the compute stream.  Blocks the host (it steers the passes).
+// A speculative pass covers [pos, pos + window).  Where the speculative AGC's hand-overs verify (loud noise, a gain
+// pinned at a limit) the window doubles after every pass that consumed all of it, so a burst-free chunk takes one pass.
+// Where they do not (quiet noise, DESIGN.md §4) a pass stops at its verified end: the window halves, and the samples
+// after that end go to the ordinary pipelined kernel on the raw samples, in a span that doubles with every stop in a
+// row (the DC-blocker state is first brought to the span's start by kernel A).  So no pass costs more than a constant
+// times what it consumes plus what the pass before it consumed, and input that never verifies runs at the ordinary
+// kernel's speed.  Bursts (AGC locked) go to the tile-fed single-warp kernel on A's output, kLongSpan at a time.
 int run_long(same_engine* e, const int16_t* d_src, uint32_t len) {
   const SameLayout& L = e->p.layout;
   for (uint32_t base = 0; base < len; base += kLongChunk) {
     const uint32_t n = std::min(kLongChunk, len - base);
     int rc = ensure_long(e, n);
     if (rc) return rc;
-    CK(e, same_long_launch_dc(&e->p, d_src + base, n, e->ls_d, e->tiles_dc_next, e->compute));
+    const int16_t* src = d_src + base;
+    CK(e, same_long_launch_dc(&e->p, src, n, e->ls_d, e->tiles_dc_next, e->compute));
     e->launches += 1;
-    uint32_t pos = 0;
+    // dc_at: the position the resident DC-blocker state belongs to (the state words are committed at the chunk's end)
+    uint32_t pos = 0, window = n, unverified = 0, stops = 0, dc_at = 0;
     while (pos < n) {
+      if (unverified) {   // the span after a verification stop: the ordinary kernel on the raw samples
+        const uint32_t span = std::min(unverified, n - pos);
+        if (dc_at < pos) {
+          CK(e, same_long_launch_dc(&e->p, src + dc_at, pos - dc_at, e->ls_y, e->ls_dc_at, e->compute));
+          CK(e, same_long_launch_commit_dc(&e->p, e->ls_dc_at, e->compute));
+          e->launches += 2;
+        }
+        e->ls_hctrl[5] = span;
+        *reinterpret_cast<unsigned long long*>(e->ls_hctrl + 6) = pos;
+        CK(e, cudaMemcpyAsync(e->ls_ctrl + 3, e->ls_hctrl + 5, sizeof(uint32_t), cudaMemcpyHostToDevice, e->compute));
+        CK(e, cudaMemcpyAsync(e->ls_off, e->ls_hctrl + 6, sizeof(unsigned long long), cudaMemcpyHostToDevice, e->compute));
+        CK(e, same_launch_rx(&e->p, &e->taps, &e->taps2, PIPE, e->lanes_per_warp, src, 0, e->ls_off, e->ls_ctrl + 3, nullptr,
+                             e->compute));
+        e->launches += 1; e->ls_fallback_launches += 1;
+        pos += span;
+        dc_at = pos;
+        unverified = 0;
+        continue;
+      }
       // is the AGC locked (inside a burst)?  then the samples are the ordinary kernel's, span by span
       CK(e, cudaMemcpyAsync(e->ls_hctrl + 4, e->d_state + (size_t)F_FLAGS * L.n_pad, sizeof(uint32_t), cudaMemcpyDeviceToHost, e->compute));
       CK(e, cudaStreamSynchronize(e->compute));
@@ -362,15 +396,25 @@ int run_long(same_engine* e, const int16_t* d_src, uint32_t len) {
         pos += span;
         continue;
       }
-      CK(e, same_long_launch_speculative(&e->p, &e->taps2, e->ls_d, pos, n, e->ls_y, e->ls_g, e->ls_gin, e->ls_soft, e->ls_ctrl,
+      const uint32_t end = pos + std::min(window, n - pos);
+      CK(e, same_long_launch_speculative(&e->p, &e->taps2, e->ls_d, pos, end, e->ls_y, e->ls_g, e->ls_gin, e->ls_soft, e->ls_ctrl,
                                          e->compute));
       e->launches += 4; e->ls_spec_launches += 1;
       CK(e, cudaMemcpyAsync(e->ls_hctrl, e->ls_ctrl, 3 * sizeof(uint32_t), cudaMemcpyDeviceToHost, e->compute));
       CK(e, cudaStreamSynchronize(e->compute));
-      const uint32_t reached = e->ls_hctrl[1];
-      if (reached < pos || reached > n) return fail(e, SAME_ERR_CUDA, "long-stream pass reported an impossible position");
-      if (reached == pos && e->ls_hctrl[2] == 0u) return fail(e, SAME_ERR_CUDA, "long-stream pass made no progress");
+      const uint32_t reached = e->ls_hctrl[1], why = e->ls_hctrl[2];
+      if (reached < pos || reached > end) return fail(e, SAME_ERR_CUDA, "long-stream pass reported an impossible position");
+      if (reached == pos && why == 0u) return fail(e, SAME_ERR_CUDA, "long-stream pass made no progress");
       pos = reached;
+      if (why != 0u) continue;    // the symbol stages locked the AGC or reset the timing loop: the next round decides
+      if (reached == end) {       // all of the range verified
+        window = (uint32_t)std::min<uint64_t>(2ull * window, n);
+        stops = 0;
+      } else {                    // verification stop: the hand-over at `reached` did not match
+        window = std::max(kLongMinPass, window / 2u);
+        unverified = std::min(kLongSpanMax, kLongSpan << std::min(stops, 7u));
+        stops += 1;
+      }
     }
     CK(e, same_long_launch_commit_dc(&e->p, e->tiles_dc_next, e->compute));
     e->launches += 1;

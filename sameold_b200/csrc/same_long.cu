@@ -6,9 +6,12 @@
 //   A  same_long_dc_kernel    s16 -> exact DC-blocked f32, time-parallel (the integer recursion has 31 samples of memory)
 //   B  same_long_agc_kernel   the AGC recurrence (agc.rs:72-77) in blocks of 2048 samples, one thread per block.  Block 0
 //                             starts from the stream's true gain; every other block warms up on the 1024 samples before
-//                             it from a guessed gain.  The unlocked AGC map contracts (|1 - |d| bw| per sample), so the
-//                             trajectories coalesce BITWISE within ~300 samples on noise (worst seen 481) — and whether a
-//                             block's start gain really equals its predecessor's end gain is CHECKED, bit for bit:
+//                             it from a guessed gain.  The unlocked AGC map contracts (|1 - |d| bw| per sample), so
+//                             the trajectories coalesce BITWISE on loud noise (corpus level: within ~400 samples) and
+//                             when a gain limit pins them (quiet input at gmax) -- but NOT in between: with samedec
+//                             limits, noise of sigma ~300-1000 LSB (-40 to -30 dBFS) fails nearly every hand-over
+//                             (DESIGN.md §4).  So whether a block's start gain equals its predecessor's end gain is
+//                             CHECKED, bit for bit:
 //      same_long_verify_kernel   first block whose hand-over fails -> end of the range that may be consumed.
 //   C  same_long_mf_kernel    the mark/space matched filters (demod.rs:156-164) at EVERY sample position of that AGC
 //                             output, time-parallel: 21x the arithmetic of the sequential receiver, in parallel.
@@ -17,8 +20,11 @@
 //                             (A6-A9) on a second warp, one ring of symbol records behind: ~250 cycles per TED round
 //                             instead of ~1500.  It stops when the symbol stages lock the AGC (sync found: a burst
 //                             begins) or reset the timing loop, at the end of the verified range, or at the end.
-//   burst / unverified spans  the ordinary tile-fed single-warp kernel (same_rx_fast_kernel<true>) on A's output, until
+//   bursts                    the ordinary tile-fed single-warp kernel (same_rx_fast_kernel<true>) on A's output, until
 //                             the AGC is unlocked again; then B-D restart from the true state.
+//   unverified spans          after a pass that stopped at its verified end: the ordinary pipelined kernel on the raw
+//                             samples (DC state brought to the span start by A), in spans that grow while the stops
+//                             repeat; the host also bounds each pass's range (run_long, same_engine.cu).
 // The speculation in B never decides anything: a block is used only after its hand-over gain was verified, and D's
 // arithmetic is the sequential receiver's (same_lane.cuh), so the events are those of the reference, bit for bit
 // (tests: the full 24 h stream, the 16-minute stream in chunks, every single-stream test above the length threshold).
