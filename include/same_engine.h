@@ -31,7 +31,9 @@ extern "C" {
 enum same_status {
   SAME_OK = 0,
   SAME_ERR_INVALID_ARG = 1,    /* NULL pointer, stream id out of range, length too large */
-  SAME_ERR_INVALID_CONFIG = 2, /* a configuration the reference would panic on (e.g. DC length 0) or beyond engine limits */
+  SAME_ERR_INVALID_CONFIG = 2, /* a configuration the reference would panic on (e.g. DC length 0) or beyond engine limits:
+                                  matched filters of 1..512 taps (input_rate 521..267 185 Hz), DC blocker up to 512
+                                  samples, equalizer up to 16 taps per arm; the message names the limit */
   SAME_ERR_NO_DEVICE = 3,      /* no usable CUDA device / device index out of range */
   SAME_ERR_CUDA = 4,           /* CUDA runtime error; see same_engine_last_error */
   SAME_ERR_EVENT_OVERFLOW = 5, /* event or payload arena too small for what was produced between two syncs: the events
@@ -143,18 +145,20 @@ void same_snapshot_free(same_snapshot* snap);
  * processes (checkpoint / resume, moving a stream to another slot, engine or GPU).
  *
  * An export buffer is one header followed by n records.  All fields little-endian; offsets in bytes.
- *   Header (2224 bytes):
+ *   Header (H = 164 + 16 T + 12 bytes, T = max(128, ntaps) tap entries per filter section, ntaps =
+ *   floor((f32)input_rate / 520.83f); H = 2224 up to 128 taps, 3120 at 96 kHz, 6064 at 192 kHz):
  *     0  u32 magic 0x54534D53 ("SMST")          4  u32 format version (1; readers accept only their own)
- *     8  u32 byte-order mark 0x01020304         12 u32 header size (2224)
+ *     8  u32 byte-order mark 0x01020304         12 u32 header size H (must match the config's input_rate)
  *     16 u32 n_records                          20 u32 n_words (state words per stream)
  *     24 u32 sizeof(StreamBlob) (3240)          28 u32 SAME_BURST_CAP
  *     32 u32 record size R                      36 u32 reserved (0)
  *     40    same_config the state was produced under (sanitized; 19 x 4 bytes)
  *     116   same_derived of that engine (12 x 4 bytes)
- *     164   mark filter taps, raw f32 bits, (re, im) x 128, unused taps 0
- *     1188  space filter taps, same layout
- *     2212  8 bytes reserved (0)
- *     2220  u32 CRC-32 (zlib polynomial, as zlib.crc32) of bytes 0..2219
+ *     164           mark filter taps, raw f32 bits, (re, im) x T, unused taps 0
+ *     164 + 8 T     space filter taps, same layout
+ *     164 + 16 T    8 bytes reserved (0)
+ *     H - 4         u32 CRC-32 (zlib polynomial, as zlib.crc32) of bytes 0 .. H-5
+ *   (T = 128: space taps at 1188, CRC at 2220.)
  *   Record (R = W + B bytes, W = round_up(8 + 4 * n_words, 16), B = round_up(sizeof(StreamBlob) + 4, 16)):
  *     0      u32 source stream id
  *     4      u32 flags: bit 0 = the DC-blocker state may be non-integer (the engine had an f32 submit since
@@ -254,7 +258,9 @@ int same_engine_set_option(same_engine* e, const char* key, int value);
 /* Reads an option back; additionally "kernel_selected": the kernel the next s16 submit will launch (1 generic,
  * 2 single-warp, 3 pipelined, 4 three-warp, 6 look-ahead single-warp) — the policy result for this batch size unless
  * "kernel" overrides it; "rollbacks": how often the pipelined kernel's timing warp resumed a stream from a symbol whose
- * symbol stages changed its state (sync found or end of a burst), counted up to the last sync (diagnostic). */
+ * symbol stages changed its state (sync found or end of a burst), counted up to the last sync (diagnostic);
+ * "resident_blocks_per_sm": how many blocks of that kernel (each serves 32 streams) fit on one SM at this engine's
+ * geometry, from the CUDA runtime's occupancy calculator (registers, shared memory, block limits). */
 int same_engine_get_option(same_engine* e, const char* key, int* value);
 
 /* Measurement aid: runs only the front-end kernel (feed-forward stages: s16 -> f32, DC blocker; 2 B read + 4 B written

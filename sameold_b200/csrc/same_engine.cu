@@ -49,10 +49,15 @@ void loop_alphabeta(float bw, float& alpha, float& beta) {
   beta = k0 * (1.0f - k1 * (sh + 1.0f));
 }
 
-size_t f32_as_usize(float x) {  // `as usize`: truncating, saturating, NaN -> 0
-  if (!(x > 0.0f)) return 0;
-  if (x >= 1.8e19f) return (size_t)-1;
-  return (size_t)x;
+// The input rates whose matched filter has 1..max_taps taps, in the engine's own f32 arithmetic (same_ntaps)
+void rate_range(size_t max_taps, uint32_t* lo, uint32_t* hi) {
+  uint32_t r = 1;
+  while (same_ntaps(r) < 1) ++r;
+  *lo = r;
+  r = (uint32_t)((double)(max_taps + 1) * kBaudHz) + 2u;
+  while (same_ntaps(r) > max_taps) --r;
+  while (same_ntaps(r + 1) <= max_taps) ++r;
+  *hi = r;
 }
 
 // ---- owned CUDA resources: released when their owner goes, on the device that is current then ----
@@ -129,7 +134,8 @@ struct same_engine {
   int device = 0;
   uint32_t n_streams = 0;
   SameParams p;           // its pointers into the buffers below are set by bind()
-  SameTaps taps;
+  SameTapsWide taps_wide;   // every tap: the wide kernel's, the state header's and same_engine_get_derived's
+  SameTaps taps;            // the first SAME_GENERIC_TAPS of them for the generic kernel
   SameTaps2 taps2;
   Kernel kernel_override = POLICY;   // option "kernel"
   uint32_t lanes_per_warp = 32;   // streams per warp in the fast kernel (lane-sparse warps for small batches)
@@ -375,7 +381,7 @@ int run_long(same_engine* e, const int16_t* d_src, uint32_t len) {
         *reinterpret_cast<unsigned long long*>(e->ls_hctrl + 6) = pos;
         CK(e, cudaMemcpyAsync(e->ls_ctrl + 3, e->ls_hctrl + 5, sizeof(uint32_t), cudaMemcpyHostToDevice, e->compute));
         CK(e, cudaMemcpyAsync(e->ls_off, e->ls_hctrl + 6, sizeof(unsigned long long), cudaMemcpyHostToDevice, e->compute));
-        CK(e, same_launch_rx(&e->p, &e->taps, &e->taps2, PIPE, e->lanes_per_warp, src, 0, e->ls_off, e->ls_ctrl + 3, nullptr,
+        CK(e, same_launch_rx(&e->p, &e->taps, &e->taps2, &e->taps_wide, PIPE, e->lanes_per_warp, src, 0, e->ls_off, e->ls_ctrl + 3, nullptr,
                              e->compute));
         e->launches += 1; e->ls_fallback_launches += 1;
         pos += span;
@@ -525,7 +531,7 @@ int submit_common(same_engine* e, const void* host_samples, const void* dev_samp
       if (rc) return rc;
       e->launches += 1;   // the front-end kernel
     }
-    CK(e, same_launch_rx(&e->p, &e->taps, &e->taps2, kernel, e->lanes_per_warp, d_src, sample_fmt, b.d_off, b.d_len,
+    CK(e, same_launch_rx(&e->p, &e->taps, &e->taps2, &e->taps_wide, kernel, e->lanes_per_warp, d_src, sample_fmt, b.d_off, b.d_len,
                          &e->tiles, e->compute));
     e->launches += 1;
   }
@@ -604,12 +610,19 @@ int same_engine_create(const same_config* cfg_in, int device, uint32_t n_streams
 
   // ---- SameReceiver::from(&builder)  receiver.rs:502-560 ----
   const float rate_f = (float)cfg.input_rate;
-  const float sps = rate_f / kBaudHz;                                         // waveform.rs:29-31
-  const size_t dc_len = f32_as_usize(cfg.dc_blocker_len * sps);               // receiver.rs:509
-  const size_t ntaps = f32_as_usize(floorf(sps));                             // waveform.rs:40
+  const float sps = same_samples_per_symbol(cfg.input_rate);                  // waveform.rs:29-31
+  const size_t dc_len = same_f32_as_usize(cfg.dc_blocker_len * sps);          // receiver.rs:509
+  const size_t ntaps = same_ntaps(cfg.input_rate);                            // waveform.rs:40
   if (dc_len == 0) return fail(nullptr, SAME_ERR_INVALID_CONFIG, "DC blocker length is 0 samples (MovingAverage::new asserts len > 0, dcblock.rs:74)");
-  if (dc_len > SAME_MAX_DC) return fail(nullptr, SAME_ERR_INVALID_CONFIG, "DC blocker longer than the engine limit of 64 samples");
-  if (ntaps == 0 || ntaps > SAME_MAX_TAPS) return fail(nullptr, SAME_ERR_INVALID_CONFIG, "matched filter length outside 1..128 taps (input_rate 521..67186 Hz)");
+  if (dc_len > SAME_MAX_DC)
+    return fail(nullptr, SAME_ERR_INVALID_CONFIG, "DC blocker of " + std::to_string(dc_len) + " samples is longer than the engine limit of " +
+                                                      std::to_string(SAME_MAX_DC) + " samples");
+  if (ntaps == 0 || ntaps > SAME_MAX_TAPS) {
+    uint32_t lo, hi;
+    rate_range(SAME_MAX_TAPS, &lo, &hi);
+    return fail(nullptr, SAME_ERR_INVALID_CONFIG, "matched filter length outside 1.." + std::to_string(SAME_MAX_TAPS) + " taps (input_rate " +
+                                                      std::to_string(lo) + ".." + std::to_string(hi) + " Hz)");
+  }
   uint32_t nff = cfg.eq_enabled ? cfg.eq_nff : 1u, nfb = cfg.eq_enabled ? cfg.eq_nfb : 1u;   // disabled_equalizer() receiver.rs:585-590
   float relax = cfg.eq_enabled ? cfg.eq_relaxation : 0.0f;
   float regul = cfg.eq_enabled ? cfg.eq_regularization : 1.0e-6f;
@@ -619,6 +632,7 @@ int same_engine_create(const same_config* cfg_in, int device, uint32_t n_streams
   e->cfg = cfg; e->device = device; e->n_streams = n_streams;
   SameParams& p = e->p;
   memset(&p, 0, sizeof p);
+  memset(&e->taps_wide, 0, sizeof e->taps_wide);
   memset(&e->taps, 0, sizeof e->taps);
   p.n_streams = n_streams; p.input_rate = cfg.input_rate;
   p.dc_len = (uint32_t)dc_len;
@@ -628,8 +642,16 @@ int same_engine_create(const same_config* cfg_in, int device, uint32_t n_streams
   p.agc_min = cfg.agc_gain_min; p.agc_max = cfg.agc_gain_max;
   p.agc_gain0 = fminf(1.0f, cfg.agc_gain_min);                                // agc.rs:55
   p.ntaps = (uint32_t)ntaps;
-  cisoid_taps(p.ntaps, kMarkHz / rate_f, e->taps.mark_re, e->taps.mark_im);   // waveform.rs:41-42
-  cisoid_taps(p.ntaps, kSpaceHz / rate_f, e->taps.space_re, e->taps.space_im);
+  {
+    std::vector<float> mre(p.ntaps), mim(p.ntaps), sre(p.ntaps), sim(p.ntaps);
+    cisoid_taps(p.ntaps, kMarkHz / rate_f, mre.data(), mim.data());           // waveform.rs:41-42
+    cisoid_taps(p.ntaps, kSpaceHz / rate_f, sre.data(), sim.data());
+    for (uint32_t i = 0; i < p.ntaps; ++i) e->taps_wide.t[i] = make_float4(mre[i], mim[i], sre[i], sim[i]);
+  }
+  for (uint32_t i = 0; i < p.ntaps && i < SAME_GENERIC_TAPS; ++i) {
+    const float4 t = e->taps_wide.t[i];
+    e->taps.mark_re[i] = t.x; e->taps.mark_im[i] = t.y; e->taps.space_re[i] = t.z; e->taps.space_im[i] = t.w;
+  }
   memset(&e->taps2, 0, sizeof e->taps2);
   for (uint32_t i = 0; i < p.ntaps && i < 64; ++i) {
     e->taps2.mark[i] = make_float2(e->taps.mark_re[i], e->taps.mark_im[i]);
@@ -968,6 +990,11 @@ int same_engine_get_option(same_engine* e, const char* key, int* value) {
   if (strcmp(key, "state_kernel_us") == 0) { *value = (int)std::min(e->st_kernel_ms * 1000.0f, 2.0e9f); return SAME_OK; }
   if (strcmp(key, "state_copy_us") == 0) { *value = (int)std::min(e->st_copy_ms * 1000.0f, 2.0e9f); return SAME_OK; }
   if (strcmp(key, "kernel_selected") == 0) { *value = rx_kernel(e); return SAME_OK; }
+  if (strcmp(key, "resident_blocks_per_sm") == 0) {
+    CK(e, cudaSetDevice(e->device));
+    CK(e, same_rx_resident_blocks(&e->p, rx_kernel(e), value));
+    return SAME_OK;
+  }
   if (strcmp(key, "rollbacks") == 0) { *value = (int)std::min<uint64_t>(e->rollbacks, 0x7fffffff); return SAME_OK; }
   return fail(e, SAME_ERR_INVALID_ARG, std::string("unknown option ") + key);
 }
@@ -1033,8 +1060,9 @@ int same_engine_get_derived(const same_engine* e, same_derived* d, float* mark_r
   if (!e || !d) return SAME_ERR_INVALID_ARG;
   *d = e->derived;
   for (size_t i = 0; i < e->p.ntaps && i < cap_taps; ++i) {
-    if (mark_re_im) { mark_re_im[2 * i] = e->taps.mark_re[i]; mark_re_im[2 * i + 1] = e->taps.mark_im[i]; }
-    if (space_re_im) { space_re_im[2 * i] = e->taps.space_re[i]; space_re_im[2 * i + 1] = e->taps.space_im[i]; }
+    const float4 t = e->taps_wide.t[i];
+    if (mark_re_im) { mark_re_im[2 * i] = t.x; mark_re_im[2 * i + 1] = t.y; }
+    if (space_re_im) { space_re_im[2 * i] = t.z; space_re_im[2 * i + 1] = t.w; }
   }
   return SAME_OK;
 }
@@ -1049,7 +1077,7 @@ namespace {
 
 // the header of a state this engine exports, and that a state it imports must match
 same_state::Header state_header(const same_engine* e, uint32_t n) {
-  return same_state::make_header(e->cfg, e->derived, e->taps, e->p.ntaps, e->p.layout.n_words, n);
+  return same_state::make_header(e->cfg, e->derived, e->taps_wide, e->p.ntaps, e->p.layout.n_words, n);
 }
 
 bool is_pinned(const void* p) {
@@ -1114,6 +1142,7 @@ int check_ids(same_engine* e, const uint32_t* ids, uint32_t n, uint32_t limit, b
 
 // ---- helpers shared with same_multi.cu (the engine must be synced and the arguments checked) ----
 size_t same_state_engine_record_bytes(const same_engine* e) { return same_state_record_bytes(e->p.layout.n_words); }
+size_t same_state_engine_header_bytes(const same_engine* e) { return same_state::header_bytes(e->p.ntaps); }
 
 void same_state_write_header(const same_engine* e, uint32_t n, void* dst) {
   same_state::write_header(state_header(e, n), static_cast<uint8_t*>(dst));
@@ -1206,7 +1235,7 @@ int same_state_import_commit(same_engine* e, const uint32_t* ids, uint32_t n, ui
 extern "C" {
 
 size_t same_engine_state_bytes(const same_engine* e, uint32_t n) {
-  return e ? same_state::kHeaderBytes + (size_t)n * same_state_engine_record_bytes(e) : 0;
+  return e ? same_state_engine_header_bytes(e) + (size_t)n * same_state_engine_record_bytes(e) : 0;
 }
 
 int same_engine_export_streams(same_engine* e, const uint32_t* ids, uint32_t n, void* buf, size_t cap, size_t* written) {
@@ -1218,7 +1247,7 @@ int same_engine_export_streams(same_engine* e, const uint32_t* ids, uint32_t n, 
   if (written) *written = need;
   if (!buf || cap < need) return fail(e, SAME_ERR_INVALID_ARG, "export buffer too small: " + std::to_string(need) + " bytes needed");
   same_state_write_header(e, n, buf);
-  return same_state_export_records(e, ids, n, 0, static_cast<uint8_t*>(buf) + same_state::kHeaderBytes);
+  return same_state_export_records(e, ids, n, 0, static_cast<uint8_t*>(buf) + same_state_engine_header_bytes(e));
 }
 
 int same_engine_import_streams(same_engine* e, const uint32_t* ids, uint32_t n, const void* buf, size_t len) {
@@ -1231,7 +1260,7 @@ int same_engine_import_streams(same_engine* e, const uint32_t* ids, uint32_t n, 
   rc = check_ids(e, ids, n, e->n_streams, true);
   if (rc) return rc;
   uint32_t flags = 0;
-  rc = same_state_import_stage(e, n, static_cast<const uint8_t*>(buf) + same_state::kHeaderBytes, &flags);
+  rc = same_state_import_stage(e, n, static_cast<const uint8_t*>(buf) + same_state_engine_header_bytes(e), &flags);
   if (rc) return rc;
   return same_state_import_commit(e, ids, n, flags);
 }

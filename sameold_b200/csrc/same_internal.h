@@ -5,11 +5,22 @@
 #pragma once
 
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stddef.h>
 
 #include <string>
 
 #include "same_params.h"
+
+// `as usize` of Rust: truncating, saturating, NaN -> 0
+inline size_t same_f32_as_usize(float x) {
+  if (!(x > 0.0f)) return 0;
+  if (x >= 1.8e19f) return (size_t)-1;
+  return (size_t)x;
+}
+// Samples per symbol and matched-filter taps at `input_rate`, in the reference's f32 arithmetic (waveform.rs:29-40)
+inline float same_samples_per_symbol(uint32_t input_rate) { return (float)input_rate / 520.83f; }
+inline size_t same_ntaps(uint32_t input_rate) { return same_f32_as_usize(floorf(same_samples_per_symbol(input_rate))); }
 
 // Receiver kernels.  The values are those of the engine option "kernel" (include/same_engine.h); POLICY lets the
 // engine choose from the batch size.  GENERIC takes any rate and s16 or f32 samples; the others are the fast kernels of
@@ -19,11 +30,13 @@ enum Kernel { POLICY = 0, GENERIC = 1, SINGLE = 2, PIPE = 3, THREE = 4, SPLIT = 
 
 // ---- launchers: same_kernels.cu ----
 // `kernel` is resolved by the engine (never POLICY) and only dispatched here; for GENERIC, sample_fmt (0 = int16,
-// 1 = float32) picks the instantiation.
-extern "C" cudaError_t same_launch_rx(const SameParams* p, const SameTaps* taps, const SameTaps2* taps2, Kernel kernel,
-                                      uint32_t lanes_per_warp, const void* d_samples, int sample_fmt,
+// 1 = float32) picks the instantiation, and a geometry beyond SAME_GENERIC_TAPS / SAME_GENERIC_DC the wide kernel.
+extern "C" cudaError_t same_launch_rx(const SameParams* p, const SameTaps* taps, const SameTaps2* taps2,
+                                      const SameTapsWide* taps_wide, Kernel kernel, uint32_t lanes_per_warp, const void* d_samples, int sample_fmt,
                                       const unsigned long long* d_offsets, const uint32_t* d_lengths,
                                       const SameTiles* tiles, cudaStream_t stream);
+// resident blocks per SM of `kernel` (never POLICY) at this geometry, from the runtime's occupancy calculator
+extern "C" cudaError_t same_rx_resident_blocks(const SameParams* p, Kernel kernel, int* blocks);
 extern "C" cudaError_t same_launch_frontend(const SameParams* p, const int16_t* d_samples, const unsigned long long* d_offsets,
                                             const uint32_t* d_lengths, const SameTiles* tiles, cudaStream_t stream);
 extern "C" cudaError_t same_launch_rx_tilefed(const SameParams* p, const SameTaps2* taps2, const uint32_t* d_lengths,
@@ -53,20 +66,29 @@ extern "C" cudaError_t same_state_launch_scatter(const SameParams* p, const uint
 
 namespace same_state {
 
-constexpr size_t kHeaderBytes = 2224;
+// Header geometry of format version 1 (include/same_engine.h), independent of the kernels' ring sizes: each filter
+// section holds T = max(kMinTapSlots, ntaps) taps, the header is kFixedHeaderBytes + 16 T bytes (164 before the taps,
+// 8 reserved + 4 CRC after them)
+constexpr uint32_t kMinTapSlots = 128;
+constexpr size_t kFixedHeaderBytes = 164 + 12;
+inline constexpr uint32_t tap_slots(size_t ntaps) { return ntaps > kMinTapSlots ? (uint32_t)ntaps : kMinTapSlots; }
+inline constexpr size_t header_bytes(size_t ntaps) { return kFixedHeaderBytes + 16 * (size_t)tap_slots(ntaps); }
+constexpr size_t kHeaderBytes = header_bytes(0);   // 2224: every engine with at most 128 taps
+static_assert(kHeaderBytes == 2224, "version-1 header of engines with at most 128 taps");
 
 // What a state header says: the producing engine's configuration, derived constants and filter taps, and the records
 // that follow
 struct Header {
   same_config cfg;
   same_derived derived;
-  uint8_t taps[2 * 8 * SAME_MAX_TAPS];   // raw little-endian bits: mark (re, im) x 128, then space
+  uint32_t slots;                        // tap entries per section: tap_slots(ntaps)
+  uint8_t taps[2 * 8 * SAME_MAX_TAPS];   // raw little-endian bits: mark (re, im) x slots, then space x slots
   uint32_t n_records, n_words, record_bytes;
 };
 
-Header make_header(const same_config& cfg, const same_derived& derived, const SameTaps& taps, uint32_t ntaps,
+Header make_header(const same_config& cfg, const same_derived& derived, const SameTapsWide& taps, uint32_t ntaps,
                    uint32_t n_words, uint32_t n_records);
-void write_header(const Header& s, uint8_t* h);   // kHeaderBytes
+void write_header(const Header& s, uint8_t* h);   // header_bytes(s.slots)
 // Format checks only: SAME_ERR_INVALID_ARG on any failure, with the reason in *why
 int parse_header(const void* buf, size_t len, Header* out, std::string* why);
 // `theirs` must have been produced under exactly `mine`'s configuration: SAME_ERR_INVALID_CONFIG names the first field
@@ -79,6 +101,7 @@ const char* check_name(uint32_t code);
 
 // ---- engine-side stream-state helpers, same_engine.cu (same_multi.cu calls them; the arguments must be checked) ----
 size_t same_state_engine_record_bytes(const same_engine* e);
+size_t same_state_engine_header_bytes(const same_engine* e);
 void same_state_write_header(const same_engine* e, uint32_t n, void* dst);
 // header format + comparison with `e`; on failure the reason is the engine's last error
 int same_state_check_header(same_engine* e, const void* buf, size_t len, uint32_t* n_records);

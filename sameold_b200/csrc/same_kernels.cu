@@ -22,7 +22,8 @@
 // completed a byte run the equalizer/framer.  Lane sample cursors drift apart; nothing is shared between lanes.
 //
 //   same_rx_generic_kernel  any rate / DC length, s16 or f32 samples: literal f32 recursion (needed where the DC blocker
-//                           is not exact in integers).
+//                           is not exact in integers).  Up to 128 taps and DC length 64; beyond, the same arithmetic in
+//   same_rx_wide_kernel     shared memory sized to the geometry, packed FFMA2 filters (up to 512 taps / DC length 512).
 //   22050 Hz class (42 taps, DC length 16, s16 samples) -- shared helpers DcInt / RawFeedT / agc_step / agc_segment /
 //   mf_soft, exact integer DC blocker, 16-byte loads, per-lane shared-memory rings [slot][lane], packed FFMA2 filters:
 //   same_rx_fast_kernel     one warp per 32 streams (also in tile-fed form behind same_frontend_kernel)
@@ -161,6 +162,158 @@ __global__ void __launch_bounds__(32) same_rx_generic_kernel(const __grid_consta
     LANE_ST(st, L, L.dc_fb + i) = __float_as_uint(dcb[((dch - dcl + i) & (RD - 1)) * 32 + lane]);
   }
   for (int i = 0; i < ntaps; ++i) LANE_ST(st, L, L.win + i) = __float_as_uint(win[((wh - ntaps + i) & (RW - 1)) * 32 + lane]);
+}
+
+// ----------------------------------------------------------------------------------------------------------------
+// Wide kernel: the generic kernel's arithmetic for the geometries beyond its rings (ntaps > 128 or dc_len > 64: input
+// rates from 67 188 Hz, DC blockers longer than 64 samples).  Shared memory per warp follows the geometry instead of a
+// power-of-two ceiling, so that more warps fit on an SM (2 at 192 kHz, 4 at 96 kHz):
+//   win [2 * ntaps][32]  AGC output, mirrored: slot j and slot j + ntaps hold the same sample, so the newest ntaps
+//                        samples are always readable at descending addresses without a wrap
+//   dcb [dc_len][32]     DC feedback window, exactly dc_len slots: the aged value is read and replaced in place
+// The DC feed-forward window has no ring.  Its aged samples x[n - L] and x[n - L + 1] are read back from the chunk in
+// global memory, and for the chunk's first L - 1 samples from the window in the state words.  The matched filters
+// use the packed exact FFMA2 pair of mf_soft, taps from the kernel parameters.
+// ----------------------------------------------------------------------------------------------------------------
+template <typename T>
+__global__ void __launch_bounds__(32) same_rx_wide_kernel(const __grid_constant__ SameParams p,
+                                                          const __grid_constant__ SameTapsWide taps,
+                                                          const T* __restrict__ samples,
+                                                          const unsigned long long* __restrict__ offsets,
+                                                          const uint32_t* __restrict__ lengths) {
+  extern __shared__ float smem[];
+  const int dcl = (int)p.dc_len, ntaps = (int)p.ntaps;
+  float* win = smem;                  // [2 * ntaps][32]
+  float* dcb = win + 2 * ntaps * 32;  // [dcl][32]
+
+  const SameLayout& L = p.layout;
+  const int lane = threadIdx.x;
+  const uint32_t s = blockIdx.x * 32u + lane;
+  const bool valid = s < p.n_streams;
+  const uint32_t sidx = valid ? s : 0u;  // padded lanes read stream 0's words but never write
+  uint32_t* st = p.state32 + sidx;
+  StreamBlob* blob = p.blobs + sidx;
+
+  const uint32_t len = valid ? lengths[s] : 0u;
+  if (__all_sync(0xffffffffu, len == 0u)) return;
+  const T* src = (samples != nullptr && valid) ? samples + offsets[s] : nullptr;
+  // x[m] of this chunk (m >= -L); m < 0: the feed-forward window in the state, oldest first
+  auto xin = [&](int m) -> float {
+    if (m < 0) return __uint_as_float(LANE_ST(st, L, L.dc_ff + (uint32_t)(m + dcl)));
+    return src ? (float)src[m] : 0.0f;
+  };
+
+  Lane a;
+  lane_load(a, p, st, s);
+  float ffsum = __uint_as_float(LANE_ST(st, L, F_DC_FFSUM)), fbsum = __uint_as_float(LANE_ST(st, L, F_DC_FBSUM));
+  for (int i = 0; i < dcl; ++i) dcb[i * 32 + lane] = __uint_as_float(LANE_ST(st, L, L.dc_fb + i));
+  for (int i = 0; i < ntaps; ++i) {
+    const float v = __uint_as_float(LANE_ST(st, L, L.win + i));
+    win[i * 32 + lane] = v;
+    win[(i + ntaps) * 32 + lane] = v;
+  }
+  int dch = 0;   // dcb slot of the oldest feedback value, replaced next
+  int wh = 0;    // win slot of the oldest sample, replaced next (and its mirror)
+  float aged = xin(-dcl);   // x[n - L] of the next sample n
+  __syncwarp();
+
+  const float inv_len = p.dc_inv_len, gate = p.dc_gate;
+  const float bw = p.agc_bw, gmin = p.agc_min, gmax = p.agc_max;
+  const float2 one2 = make_float2(p.f_one, p.f_one), negz2 = make_float2(p.f_negzero, p.f_negzero);
+
+  uint32_t pos = 0;
+  int cfire = fire_clock(a.until, a.clock);
+
+  while (__any_sync(0xffffffffu, pos < len)) {
+    // ---------------- segment: this lane's samples up to its next TED instant (A0-A3) ----------------
+    int nseg = 0;
+    if (pos < len) nseg = min(cfire - a.clock, (int)min(len - pos, 1u << 20));
+    const int maxseg = __reduce_max_sync(0xffffffffu, nseg);
+    for (int k = 0; k < maxseg; ++k) {
+      if (k < nseg) {
+        const int n = (int)pos + k;
+        const float x = src ? (float)src[n] : 0.0f;
+        const float sig = xin(n - dcl + 1);
+        // DC blocker  dcblock.rs:45-49,104-108
+        ffsum = FADD(ffsum, FSUB(x, aged));
+        aged = sig;
+        const float ma0 = FMUL(ffsum, inv_len);
+        const float aged2 = dcb[dch * 32 + lane];
+        dcb[dch * 32 + lane] = ma0;
+        dch = (dch + 1 == dcl) ? 0 : dch + 1;
+        fbsum = FADD(fbsum, FSUB(ma0, aged2));
+        const float ma1 = FMUL(fbsum, inv_len);
+        const float d = FSUB(sig, FMUL(gate, ma1));
+        // AGC  agc.rs:72-77
+        const float y = FMUL(d, a.g);
+        const float u = (a.flags & FLAG_AGC_LOCKED) ? 0.0f : 1.0f;
+        a.g = FADD(a.g, FMUL(FMUL(u, FSUB(1.0f, fabsf(y))), bw));
+        a.g = rclamp(a.g, gmin, gmax);
+        // demod window  demod.rs:177-179
+        win[wh * 32 + lane] = y;
+        win[(wh + ntaps) * 32 + lane] = y;
+        wh = (wh + 1 == ntaps) ? 0 : wh + 1;
+      }
+    }
+    pos += (uint32_t)nseg;
+    a.clock += nseg;
+    const bool fire = (nseg > 0) && (a.clock == cfire);
+    if (!__any_sync(0xffffffffu, fire)) continue;
+
+    // ---------------- TED instant (A4, A5) ----------------
+    float soft;
+    {
+      // newest sample pairs with tap 0, sequential accumulation  filter.rs:363-377; exact packed pair as in mf_soft
+      float2 am = make_float2(0.0f, 0.0f), as = make_float2(0.0f, 0.0f);
+      const float* yp = win + (wh - 1 + ntaps) * 32 + lane;
+#pragma unroll 4
+      for (int i = 0; i < ntaps; ++i) {
+        const float v = yp[-i * 32];
+        const float4 t = taps.t[i];
+        const float2 vv = make_float2(v, v);
+        am = __ffma2_rn(am, one2, __ffma2_rn(vv, make_float2(t.x, t.y), negz2));
+        as = __ffma2_rn(as, one2, __ffma2_rn(vv, make_float2(t.z, t.w), negz2));
+      }
+      soft = rclamp(FSUB(hypot_fixed(am.x, am.y), hypot_fixed(as.x, as.y)), -1.0f, 1.0f);  // demod.rs:163
+    }
+    bool have_sym = false;
+    if (fire) {
+      const float rem = FSUB(a.until, (float)a.clock);  // receiver.rs:352
+      a.clock = 0;
+      have_sym = ted_step(a, p, soft, rem);
+      cfire = fire_clock(a.until, 0);
+    }
+    if (!__any_sync(0xffffffffu, have_sym)) continue;
+
+    // ---------------- symbol (A6-A9) ----------------
+    if (have_sym) symbol_step(a, p, s, st, blob, a.ted1, a.ted2, a.n0 + pos);
+  }
+
+  if (!valid || len == 0u) return;
+
+  // ---- store state (canonical order: oldest first) ----
+  lane_store(a, p, st, a.n0 + len);
+  LANE_ST(st, L, F_DC_FFSUM) = __float_as_uint(ffsum);
+  LANE_ST(st, L, F_DC_FBSUM) = __float_as_uint(fbsum);
+  // in place, ascending: word i takes x[len - L + i], which is word len + i of the old window when len < L
+  for (int i = 0; i < dcl; ++i) LANE_ST(st, L, L.dc_ff + i) = __float_as_uint(xin((int)len - dcl + i));
+  for (int i = 0; i < dcl; ++i) {
+    const int j = dch + i;
+    LANE_ST(st, L, L.dc_fb + i) = __float_as_uint(dcb[(j >= dcl ? j - dcl : j) * 32 + lane]);
+  }
+  for (int i = 0; i < ntaps; ++i) LANE_ST(st, L, L.win + i) = __float_as_uint(win[(wh + i) * 32 + lane]);
+}
+
+// dynamic shared memory of same_rx_wide_kernel, and its largest value (512 taps, DC length 512: 196 608 B)
+static size_t wide_smem_bytes(const SameParams& p) { return (size_t)(2 * p.ntaps + p.dc_len) * 32 * sizeof(float); }
+constexpr int kWideMaxSmem = (2 * SAME_MAX_TAPS + SAME_MAX_DC) * 32 * (int)sizeof(float);
+
+// The opt-in shared-memory cap of the kernels that need more than 48 KB.  The attribute belongs to the function on the
+// whole device, so it is set to a constant, not to one engine's geometry: engines of other geometries may launch the
+// same function from other host threads between this call and the launch.  It only caps what a launch may request.
+template <class F>
+static cudaError_t allow_smem(F* f, int bytes) {
+  return cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
 }
 
 // ----------------------------------------------------------------------------------------------------------------
@@ -1456,8 +1609,8 @@ __global__ void same_evsort_scatter(const same_event* __restrict__ ev, uint32_t 
 // ----------------------------------------------------------------------------------------------------------------
 // Launchers (called from same_engine.cu)
 // ----------------------------------------------------------------------------------------------------------------
-extern "C" cudaError_t same_launch_rx(const SameParams* p, const SameTaps* taps, const SameTaps2* taps2, Kernel kernel,
-                                      uint32_t lanes_per_warp, const void* d_samples_v, int sample_fmt,
+extern "C" cudaError_t same_launch_rx(const SameParams* p, const SameTaps* taps, const SameTaps2* taps2,
+                                      const SameTapsWide* taps_wide, Kernel kernel, uint32_t lanes_per_warp, const void* d_samples_v, int sample_fmt,
                                       const unsigned long long* d_offsets, const uint32_t* d_lengths,
                                       const SameTiles* tiles, cudaStream_t stream) {
   const uint32_t blocks = (p->n_streams + 31u) / 32u;
@@ -1483,8 +1636,7 @@ extern "C" cudaError_t same_launch_rx(const SameParams* p, const SameTaps* taps,
       break;
     case PIPE: {
       // per device, cheap: set on every launch rather than tracking which devices have seen it
-      cudaError_t e = cudaFuncSetAttribute(same_dev::same_rx_pipe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           PK_DYN_SMEM);
+      cudaError_t e = same_dev::allow_smem(same_dev::same_rx_pipe_kernel, PK_DYN_SMEM);
       if (e != cudaSuccess) return e;
       same_dev::same_rx_pipe_kernel<<<fblocks, PK_THREADS, PK_DYN_SMEM, stream>>>(*p, *taps2, d_samples, d_offsets,
                                                                                    d_lengths, lanes);
@@ -1494,6 +1646,19 @@ extern "C" cudaError_t same_launch_rx(const SameParams* p, const SameTaps* taps,
       same_dev::same_rx_ws_kernel<<<fblocks, WS_THREADS, 0, stream>>>(*p, *taps2, d_samples, d_offsets, d_lengths, lanes);
       break;
     case GENERIC: {
+      if (p->ntaps > SAME_GENERIC_TAPS || p->dc_len > SAME_GENERIC_DC) {
+        const size_t smem = same_dev::wide_smem_bytes(*p);
+        // per device, cheap: set on every launch, as for the pipelined kernel
+        cudaError_t e = sample_fmt == 1 ? same_dev::allow_smem(same_dev::same_rx_wide_kernel<float>, same_dev::kWideMaxSmem)
+                                        : same_dev::allow_smem(same_dev::same_rx_wide_kernel<int16_t>, same_dev::kWideMaxSmem);
+        if (e != cudaSuccess) return e;
+        if (sample_fmt == 1)
+          same_dev::same_rx_wide_kernel<float><<<blocks, 32, smem, stream>>>(*p, *taps_wide, static_cast<const float*>(d_samples_v),
+                                                                             d_offsets, d_lengths);
+        else
+          same_dev::same_rx_wide_kernel<int16_t><<<blocks, 32, smem, stream>>>(*p, *taps_wide, d_samples, d_offsets, d_lengths);
+        break;
+      }
       const bool small = p->ntaps <= 64 && p->dc_len <= 16;
       const size_t smem = small ? (size_t)(64 + 2 * 16) * 32 * sizeof(float) : (size_t)(128 + 2 * 64) * 32 * sizeof(float);
       if (sample_fmt == 1) {
@@ -1510,6 +1675,39 @@ extern "C" cudaError_t same_launch_rx(const SameParams* p, const SameTaps* taps,
       return cudaErrorInvalidValue;
   }
   return cudaGetLastError();
+}
+
+// Resident blocks per SM of `kernel` at this geometry, from the runtime's occupancy calculator (registers, shared memory
+// and block limits), for s16 samples
+extern "C" cudaError_t same_rx_resident_blocks(const SameParams* p, Kernel kernel, int* blocks) {
+  cudaError_t e = cudaSuccess;
+  *blocks = 0;
+  switch (kernel) {
+    case GENERIC:
+      if (p->ntaps > SAME_GENERIC_TAPS || p->dc_len > SAME_GENERIC_DC) {
+        e = same_dev::allow_smem(same_dev::same_rx_wide_kernel<int16_t>, same_dev::kWideMaxSmem);
+        if (e == cudaSuccess)
+          e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks, same_dev::same_rx_wide_kernel<int16_t>, 32, same_dev::wide_smem_bytes(*p));
+      } else if (p->ntaps <= 64 && p->dc_len <= 16) {
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks, same_dev::same_rx_generic_kernel<64, 16, int16_t>, 32,
+                                                          (size_t)(64 + 2 * 16) * 32 * sizeof(float));
+      } else {
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks, same_dev::same_rx_generic_kernel<128, 64, int16_t>, 32,
+                                                          (size_t)(128 + 2 * 64) * 32 * sizeof(float));
+      }
+      break;
+    case SINGLE: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks, same_dev::same_rx_fast_kernel<false>, 32, 0); break;
+    case SPLIT: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks, same_dev::same_rx_fast_kernel<true>, 32, 0); break;
+    case LOOKAHEAD: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks, same_dev::same_rx_la_kernel, 32, 0); break;
+    case THREE: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks, same_dev::same_rx_ws_kernel, WS_THREADS, 0); break;
+    case PIPE:
+      e = same_dev::allow_smem(same_dev::same_rx_pipe_kernel, PK_DYN_SMEM);
+      if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks, same_dev::same_rx_pipe_kernel, PK_THREADS, PK_DYN_SMEM);
+      break;
+    default:
+      return cudaErrorInvalidValue;
+  }
+  return e;
 }
 
 // The tile-fed single-warp kernel on its own, on DC-blocked samples some front end already produced (the long-stream path

@@ -270,7 +270,7 @@ int same_multi_drain_events(same_multi* m, same_event* events, size_t events_cap
 
 // ---- portable stream state with global ids ----
 size_t same_multi_state_bytes(const same_multi* m, uint32_t n) {
-  return m ? same_state::kHeaderBytes + (size_t)n * same_state_engine_record_bytes(m->shards[0]->eng) : 0;
+  return m ? same_state_engine_header_bytes(m->shards[0]->eng) + (size_t)n * same_state_engine_record_bytes(m->shards[0]->eng) : 0;
 }
 
 // ids -> each shard's local ids and positions in `ids`; false on an id out of range (or a duplicate, if unique)
@@ -299,7 +299,7 @@ int same_multi_export_streams(same_multi* m, const uint32_t* ids, uint32_t n, vo
   const size_t need = same_multi_state_bytes(m, n);
   if (written) *written = need;
   if (!buf || cap < need) return mfail(m, SAME_ERR_INVALID_ARG, "export buffer too small: " + std::to_string(need) + " bytes needed");
-  const size_t hdr = same_state::kHeaderBytes, rec = same_state_engine_record_bytes(m->shards[0]->eng);
+  const size_t hdr = same_state_engine_header_bytes(m->shards[0]->eng), rec = same_state_engine_record_bytes(m->shards[0]->eng);
   same_state_write_header(m->shards[0]->eng, n, buf);
   uint8_t* out = static_cast<uint8_t*>(buf) + hdr;
   return run_all(m, [=](Shard& s) {
@@ -325,7 +325,7 @@ int same_multi_import_streams(same_multi* m, const uint32_t* ids, uint32_t n, co
   if (!ids && n != m->n_streams) return mfail(m, SAME_ERR_INVALID_ARG, "ids == NULL imports into every stream: n must equal the number of streams");
   if (n != n_records) return mfail(m, SAME_ERR_INVALID_ARG, "n = " + std::to_string(n) + " but the buffer holds " + std::to_string(n_records) + " records");
   if (!split_ids(m, ids, n, true)) return SAME_ERR_INVALID_ARG;
-  const size_t hdr = same_state::kHeaderBytes, rec = same_state_engine_record_bytes(e0);
+  const size_t hdr = same_state_engine_header_bytes(e0), rec = same_state_engine_record_bytes(e0);
   const uint8_t* in = static_cast<const uint8_t*>(buf) + hdr;
   // every shard stages and validates its records; only if all of them passed does any shard write its streams
   rc = run_all(m, [=](Shard& s) {

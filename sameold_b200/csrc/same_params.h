@@ -14,8 +14,10 @@
 
 #include "../../include/same_engine.h"
 
-#define SAME_MAX_TAPS 128      // matched filter taps (floor(rate/520.83)): 42 @22050, 84 @44100, 92 @48000
-#define SAME_MAX_DC 64         // DC blocker length ((0.38*sps) as usize): 16 @22050, 32 @44100, 35 @48000
+#define SAME_MAX_TAPS 512      // matched filter taps (floor(rate/520.83)): 42 @22050, 92 @48000, 184 @96000, 368 @192000
+#define SAME_MAX_DC 512        // DC blocker length ((0.38*sps) as usize): 16 @22050, 35 @48000, 70 @96000, 140 @192000
+#define SAME_GENERIC_TAPS 128  // widest geometry of the shared-memory rings of same_rx_generic_kernel (SameTaps)
+#define SAME_GENERIC_DC 64     // beyond either: same_rx_wide_kernel, rings sized to the geometry (SameTapsWide)
 #define SAME_MAX_EQ 16         // equalizer taps per arm
 #define SAME_SQ_HIST 64        // codesquelch.rs:145 sample history
 #define SAME_MAX_MESSAGE_LENGTH 268  // assembler.rs:70
@@ -154,5 +156,11 @@ struct SameTaps2 {                // the same taps as (re, im) pairs for the pac
 };
 
 struct SameTaps {                 // matched filter taps, tap i pairs with the sample i steps back from the newest
-  float mark_re[SAME_MAX_TAPS], mark_im[SAME_MAX_TAPS], space_re[SAME_MAX_TAPS], space_im[SAME_MAX_TAPS];
+  float mark_re[SAME_GENERIC_TAPS], mark_im[SAME_GENERIC_TAPS], space_re[SAME_GENERIC_TAPS], space_im[SAME_GENERIC_TAPS];
+};
+
+// All taps of any geometry as (mark re, mark im, space re, space im), the pairs the packed-FFMA2 filter takes.  8 KiB:
+// a kernel parameter of same_rx_wide_kernel alone, so the other kernels' parameters do not grow with it.
+struct SameTapsWide {
+  float4 t[SAME_MAX_TAPS];
 };

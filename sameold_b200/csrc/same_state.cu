@@ -289,10 +289,13 @@ uint32_t crc32_host(const uint8_t* d, size_t n) {
 constexpr uint32_t kStMagic = 0x54534D53u;   // "SMST"
 constexpr uint32_t kStVersion = 1u;
 constexpr uint32_t kStBom = 0x01020304u;
-constexpr size_t kStOffConfig = 40, kStOffDerived = 116, kStOffMark = 164, kStOffSpace = 1188, kStOffCrc = 2220;
+// Offsets of the sections after the derived constants follow the tap entries per section T = tap_slots(ntaps):
+// mark taps at 164, space taps at 164 + 8 T, 8 zero bytes, CRC at 164 + 16 T + 8 (2220 for T = 128)
+constexpr size_t kStOffConfig = 40, kStOffDerived = 116, kStOffMark = 164;
+constexpr size_t off_crc(uint32_t slots) { return kStOffMark + 16 * (size_t)slots + 8; }
 static_assert(sizeof(same_config) == 19 * 4 && sizeof(same_derived) == 12 * 4, "4-byte fields only");
 static_assert(kStOffDerived == kStOffConfig + sizeof(same_config) && kStOffMark == kStOffDerived + sizeof(same_derived) &&
-              kStOffSpace == kStOffMark + 8 * SAME_MAX_TAPS && kStOffCrc + 4 == kHeaderBytes, "header layout");
+              off_crc(kMinTapSlots) + 4 == kHeaderBytes, "header layout");
 
 void put32(uint8_t* p, uint32_t v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); p[2] = (uint8_t)(v >> 16); p[3] = (uint8_t)(v >> 24); }
 uint32_t get32(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24); }
@@ -312,29 +315,31 @@ const char* const kConfigFields[19] = {
 const char* const kDerivedFields[12] = {"sps", "agc_bw", "agc_gain0", "samples_per_ted", "period_min", "period_max",
                                         "alpha_unlocked", "beta_unlocked", "alpha_locked", "beta_locked", "dc_len", "ntaps"};
 
-Header make_header(const same_config& cfg, const same_derived& derived, const SameTaps& taps, uint32_t ntaps,
+Header make_header(const same_config& cfg, const same_derived& derived, const SameTapsWide& taps, uint32_t ntaps,
                    uint32_t n_words, uint32_t n_records) {
   Header s;
   memset(&s, 0, sizeof s);
   s.cfg = cfg; s.derived = derived;
+  s.slots = tap_slots(ntaps);
   s.n_records = n_records; s.n_words = n_words; s.record_bytes = same_state_record_bytes(n_words);
   for (uint32_t i = 0; i < ntaps; ++i) {
-    const float v[4] = {taps.mark_re[i], taps.mark_im[i], taps.space_re[i], taps.space_im[i]};
+    const float v[4] = {taps.t[i].x, taps.t[i].y, taps.t[i].z, taps.t[i].w};
     put_words(s.taps + 8 * i, v, 8);
-    put_words(s.taps + 8 * SAME_MAX_TAPS + 8 * i, v + 2, 8);
+    put_words(s.taps + 8 * s.slots + 8 * i, v + 2, 8);
   }
   return s;
 }
 
 void write_header(const Header& s, uint8_t* h) {
-  memset(h, 0, kHeaderBytes);
-  put32(h + 0, kStMagic); put32(h + 4, kStVersion); put32(h + 8, kStBom); put32(h + 12, (uint32_t)kHeaderBytes);
+  const size_t bytes = header_bytes(s.slots);
+  memset(h, 0, bytes);
+  put32(h + 0, kStMagic); put32(h + 4, kStVersion); put32(h + 8, kStBom); put32(h + 12, (uint32_t)bytes);
   put32(h + 16, s.n_records); put32(h + 20, s.n_words); put32(h + 24, (uint32_t)sizeof(StreamBlob));
   put32(h + 28, SAME_BURST_CAP); put32(h + 32, s.record_bytes);
   put_words(h + kStOffConfig, &s.cfg, sizeof(same_config));
   put_words(h + kStOffDerived, &s.derived, sizeof(same_derived));
-  memcpy(h + kStOffMark, s.taps, sizeof s.taps);
-  put32(h + kStOffCrc, crc32_host(h, kStOffCrc));
+  memcpy(h + kStOffMark, s.taps, 16 * (size_t)s.slots);
+  put32(h + off_crc(s.slots), crc32_host(h, off_crc(s.slots)));
 }
 
 int parse_header(const void* buf, size_t len, Header* out, std::string* why) {
@@ -345,20 +350,30 @@ int parse_header(const void* buf, size_t len, Header* out, std::string* why) {
   if (get32(h) != kStMagic) return bad("bad magic");
   if (get32(h + 8) != kStBom) return bad("wrong byte order");
   if (get32(h + 4) != kStVersion) return bad("format version " + std::to_string(get32(h + 4)) + ", this library reads version " + std::to_string(kStVersion));
-  if (get32(h + 12) != kHeaderBytes) return bad("bad header size");
-  if (len < kHeaderBytes) return bad("truncated header");
-  if (get32(h + kStOffCrc) != crc32_host(h, kStOffCrc)) return bad("header CRC mismatch");
+  // the header size says how many tap entries each section holds; checked against the configuration below
+  const uint32_t hbytes = get32(h + 12);
+  if (hbytes < kHeaderBytes || hbytes > header_bytes(SAME_MAX_TAPS) || (hbytes - kHeaderBytes) % 16u != 0)
+    return bad("bad header size");
+  const uint32_t slots = (uint32_t)((hbytes - kFixedHeaderBytes) / 16u);
+  if (len < hbytes) return bad("truncated header");
+  if (get32(h + off_crc(slots)) != crc32_host(h, off_crc(slots))) return bad("header CRC mismatch");
   Header s;
+  memset(&s, 0, sizeof s);
+  s.slots = slots;
+  get_words(&s.cfg, h + kStOffConfig, sizeof(same_config));
+  const size_t ntaps = same_ntaps(s.cfg.input_rate);
+  if (ntaps > SAME_MAX_TAPS || hbytes != header_bytes(ntaps))
+    return bad("header size " + std::to_string(hbytes) + " does not match the " + std::to_string(ntaps) + "-tap filters of input_rate " +
+               std::to_string(s.cfg.input_rate) + " Hz (" + std::to_string(header_bytes(ntaps)) + " bytes)");
   s.n_records = get32(h + 16); s.n_words = get32(h + 20); s.record_bytes = get32(h + 32);
   if (get32(h + 24) != sizeof(StreamBlob) || get32(h + 28) != SAME_BURST_CAP) return bad("stream blob layout differs from this library's");
   if (s.n_words < F_NUM_SCALARS || s.n_words > (1u << 16) || s.record_bytes != same_state_record_bytes(s.n_words))
     return bad("inconsistent record size");
-  const size_t need = kHeaderBytes + (size_t)s.n_records * s.record_bytes;
+  const size_t need = hbytes + (size_t)s.n_records * s.record_bytes;
   if (len < need) return bad("truncated: " + std::to_string(len) + " bytes, the header announces " + std::to_string(need));
   if (len > need) return bad("trailing bytes after the last record");
-  get_words(&s.cfg, h + kStOffConfig, sizeof(same_config));
   get_words(&s.derived, h + kStOffDerived, sizeof(same_derived));
-  memcpy(s.taps, h + kStOffMark, sizeof s.taps);
+  memcpy(s.taps, h + kStOffMark, 16 * (size_t)slots);
   *out = s;
   return SAME_OK;
 }
@@ -373,8 +388,10 @@ int compare_header(const Header& mine, const Header& s, std::string* why) {
   memcpy(c, &mine.derived, sizeof c); memcpy(d, &s.derived, sizeof d);
   for (int i = 0; i < 12; ++i)
     if (c[i] != d[i]) { *why = std::string("derived constant ") + kDerivedFields[i] + " differs from this engine's (another host's libm?)"; return SAME_ERR_INVALID_CONFIG; }
-  if (memcmp(mine.taps, s.taps, 8 * SAME_MAX_TAPS) != 0) { *why = "mark filter taps differ from this engine's"; return SAME_ERR_INVALID_CONFIG; }
-  if (memcmp(mine.taps + 8 * SAME_MAX_TAPS, s.taps + 8 * SAME_MAX_TAPS, 8 * SAME_MAX_TAPS) != 0) {
+  // equal input rates (checked above) mean equal tap entries per section
+  const size_t sec = 8 * (size_t)mine.slots;
+  if (memcmp(mine.taps, s.taps, sec) != 0) { *why = "mark filter taps differ from this engine's"; return SAME_ERR_INVALID_CONFIG; }
+  if (memcmp(mine.taps + sec, s.taps + sec, sec) != 0) {
     *why = "space filter taps differ from this engine's"; return SAME_ERR_INVALID_CONFIG;
   }
   if (s.n_words != mine.n_words) { *why = "state words per stream differ from this engine's"; return SAME_ERR_INVALID_CONFIG; }

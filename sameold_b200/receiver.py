@@ -313,12 +313,12 @@ class SameBatchReceiver:
 
     def derived(self):
         d = _lib.SameDerived()
-        mark = np.zeros(2 * 128, np.float32)
-        space = np.zeros(2 * 128, np.float32)
-        self._ck(self._lib.same_engine_get_derived(self._h, C.byref(d), mark.ctypes.data, space.ctypes.data, 128))
+        self._ck(self._lib.same_engine_get_derived(self._h, C.byref(d), None, None, 0))
+        mark = np.zeros((d.ntaps, 2), np.float32)
+        space = np.zeros((d.ntaps, 2), np.float32)
+        self._ck(self._lib.same_engine_get_derived(self._h, C.byref(d), mark.ctypes.data, space.ctypes.data, d.ntaps))
         out = {n: getattr(d, n) for n, _ in _lib.SameDerived._fields_}
-        out["mark"] = mark[: 2 * d.ntaps].reshape(-1, 2).copy()
-        out["space"] = space[: 2 * d.ntaps].reshape(-1, 2).copy()
+        out["mark"], out["space"] = mark, space
         return out
 
     # -- submit / drain --
