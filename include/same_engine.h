@@ -249,7 +249,9 @@ int same_engine_read_soft_trace(same_engine* e, uint32_t stream, same_soft_symbo
  *                     regime: 16 resident warps per SM).  ("force_generic": old name.)
  *   "long_stream"     1 (default): an engine with ONE stream sends chunks of >= 65536 s16 samples down the long-stream
  *                     path (same_long.cu: DC blocker, AGC and matched filters time-parallel, timing loop sequential;
- *                     such a submit returns when the chunk is done); 0: always the ordinary kernels
+ *                     such a submit returns when the chunk is done), at any geometry the engine accepts, s16 only: not
+ *                     after an f32 submit since create / reset(all), nor with option "kernel" set; 0: always the
+ *                     ordinary kernels
  *   "lanes_per_warp"  streams per warp of the fast kernels (1..32)
  *   "device_sort"     1 (default): big batches of events are put into per-stream order on the device before the
  *                     read-back; 0: always on the host

@@ -150,6 +150,8 @@ struct same_engine {
   DevBuf<uint32_t> ls_ctrl;       // {verified end, position reached, reason, span length}
   DevBuf<unsigned long long> ls_off;   // offset of an unverified span in the chunk (ordinary-kernel launch)
   DevBuf<uint32_t> ls_dc_at;      // DC-blocker state at the start of an unverified span (34 words, word-major)
+  DevBuf<float> ls_ma0, ls_fbs;   // general geometry: ma0 and fbsum of every sample of the chunk
+  DevBuf<uint32_t> ls_dc0;        // general geometry: the DC words the chunk started with (2 dc_len + 3)
   PinnedBuf<uint32_t> ls_hctrl;   // mirror + scratch
   uint64_t ls_spec_launches = 0, ls_fallback_launches = 0;
   bool saw_f32 = false;           // an f32 submit happened since create / reset(all): DC state may be non-integer -> generic kernel
@@ -334,10 +336,22 @@ constexpr uint32_t kLongChunk = 1u << 24;       // samples per internal pass (bo
 constexpr uint32_t kLongSpan = 8192;            // samples per fallback launch while the AGC is locked (inside a burst)
 constexpr uint32_t kLongSpanMax = 1u << 20;     // longest fallback span after verification stops in a row
 constexpr uint32_t kLongMinPass = 1u << 16;     // shortest range of a speculative pass
+// The three above are samples of the 22050 Hz class.  Any other geometry scales them by ntaps / 42, so that they cover
+// the same audio time (the ordinary spans then cost the same share of a stream, and a pass the same number of TED
+// rounds); the speculative AGC's block and warm-up (same_long.cu) stay in samples, its bandwidth per sample being the
+// same at every rate.
+
+// Any geometry but the 22050 Hz class's (42 taps, DC length 16): the general DC front and the ordinary generic kernel
+bool long_general(const same_engine* e) { return e->p.ntaps != 42 || e->p.dc_len != 16; }
 
 int ensure_long(same_engine* e, size_t n) {
   CK(e, e->ls_d.grow(n + 64));
-  CK(e, e->ls_y.grow(n + 128));
+  CK(e, e->ls_y.grow(n + 128 + e->p.ntaps));   // + the demod window before the range
+  if (long_general(e)) {
+    CK(e, e->ls_ma0.grow(n + 64));
+    CK(e, e->ls_fbs.grow(n + 2 * 4096 + 64));  // + two tiles: the scan stages ahead
+    CK(e, e->ls_dc0.grow(2 * (size_t)e->p.dc_len + 3));
+  }
   CK(e, e->ls_g.grow(n + 64));
   CK(e, e->ls_soft.grow(n + 2 * 4096 + 64));   // + two tiles: the sequential kernel stages ahead
   CK(e, e->ls_gin.grow(n / 2048 + 8));
@@ -358,34 +372,54 @@ int ensure_long(same_engine* e, size_t n) {
 // row (the DC-blocker state is first brought to the span's start by kernel A).  So no pass costs more than a constant
 // times what it consumes plus what the pass before it consumed, and input that never verifies runs at the ordinary
 // kernel's speed.  Bursts (AGC locked) go to the tile-fed single-warp kernel on A's output, kLongSpan at a time.
+// Any other geometry (long_general): A is the general DC front, which keeps ma0 and fbsum of every sample, and both
+// kinds of span go to the ordinary generic (or wide) kernel on the raw samples after a DC commit at the span's start.
 int run_long(same_engine* e, const int16_t* d_src, uint32_t len) {
   const SameLayout& L = e->p.layout;
+  const bool general = long_general(e);
+  const auto scaled = [&](uint32_t v) { return general ? (uint32_t)std::max<uint64_t>(1u, (uint64_t)v * e->p.ntaps / 42u) : v; };
+  const uint32_t span_locked = scaled(kLongSpan), span_max = scaled(kLongSpanMax), min_pass = scaled(kLongMinPass);
   for (uint32_t base = 0; base < len; base += kLongChunk) {
     const uint32_t n = std::min(kLongChunk, len - base);
     int rc = ensure_long(e, n);
     if (rc) return rc;
     const int16_t* src = d_src + base;
-    CK(e, same_long_launch_dc(&e->p, src, n, e->ls_d, e->tiles_dc_next, e->compute));
-    e->launches += 1;
+    if (general) {
+      CK(e, same_long_launch_dc_general(&e->p, src, n, e->ls_dc0, e->ls_ma0, e->ls_fbs, e->ls_d, e->compute));
+      e->launches += 5;
+    } else {
+      CK(e, same_long_launch_dc(&e->p, src, n, e->ls_d, e->tiles_dc_next, e->compute));
+      e->launches += 1;
+    }
     // dc_at: the position the resident DC-blocker state belongs to (the state words are committed at the chunk's end)
     uint32_t pos = 0, window = n, unverified = 0, stops = 0, dc_at = 0;
-    while (pos < n) {
-      if (unverified) {   // the span after a verification stop: the ordinary kernel on the raw samples
-        const uint32_t span = std::min(unverified, n - pos);
-        if (dc_at < pos) {
+    // `span` samples from pos on by the ordinary kernel `k` on the raw samples, the DC state first brought to pos
+    const auto ordinary_span = [&](uint32_t span, Kernel k) -> int {
+      if (dc_at < pos) {
+        if (general) {
+          CK(e, same_long_launch_commit_dc_general(&e->p, src, pos, e->ls_dc0, e->ls_ma0, e->ls_fbs, e->compute));
+          e->launches += 1;
+        } else {
           CK(e, same_long_launch_dc(&e->p, src + dc_at, pos - dc_at, e->ls_y, e->ls_dc_at, e->compute));
           CK(e, same_long_launch_commit_dc(&e->p, e->ls_dc_at, e->compute));
           e->launches += 2;
         }
-        e->ls_hctrl[5] = span;
-        *reinterpret_cast<unsigned long long*>(e->ls_hctrl + 6) = pos;
-        CK(e, cudaMemcpyAsync(e->ls_ctrl + 3, e->ls_hctrl + 5, sizeof(uint32_t), cudaMemcpyHostToDevice, e->compute));
-        CK(e, cudaMemcpyAsync(e->ls_off, e->ls_hctrl + 6, sizeof(unsigned long long), cudaMemcpyHostToDevice, e->compute));
-        CK(e, same_launch_rx(&e->p, &e->taps, &e->taps2, &e->taps_wide, PIPE, e->lanes_per_warp, src, 0, e->ls_off, e->ls_ctrl + 3, nullptr,
-                             e->compute));
-        e->launches += 1; e->ls_fallback_launches += 1;
-        pos += span;
-        dc_at = pos;
+      }
+      e->ls_hctrl[5] = span;
+      *reinterpret_cast<unsigned long long*>(e->ls_hctrl + 6) = pos;
+      CK(e, cudaMemcpyAsync(e->ls_ctrl + 3, e->ls_hctrl + 5, sizeof(uint32_t), cudaMemcpyHostToDevice, e->compute));
+      CK(e, cudaMemcpyAsync(e->ls_off, e->ls_hctrl + 6, sizeof(unsigned long long), cudaMemcpyHostToDevice, e->compute));
+      CK(e, same_launch_rx(&e->p, &e->taps, &e->taps2, &e->taps_wide, k, e->lanes_per_warp, src, 0, e->ls_off, e->ls_ctrl + 3, nullptr,
+                           e->compute));
+      e->launches += 1; e->ls_fallback_launches += 1;
+      pos += span;
+      dc_at = pos;
+      return SAME_OK;
+    };
+    while (pos < n) {
+      if (unverified) {   // the span after a verification stop: the ordinary kernel on the raw samples
+        rc = ordinary_span(std::min(unverified, n - pos), general ? GENERIC : PIPE);
+        if (rc) return rc;
         unverified = 0;
         continue;
       }
@@ -393,7 +427,12 @@ int run_long(same_engine* e, const int16_t* d_src, uint32_t len) {
       CK(e, cudaMemcpyAsync(e->ls_hctrl + 4, e->d_state + (size_t)F_FLAGS * L.n_pad, sizeof(uint32_t), cudaMemcpyDeviceToHost, e->compute));
       CK(e, cudaStreamSynchronize(e->compute));
       if (e->ls_hctrl[4] & FLAG_AGC_LOCKED) {
-        const uint32_t span = std::min(kLongSpan, n - pos);
+        const uint32_t span = std::min(span_locked, n - pos);
+        if (general) {
+          rc = ordinary_span(span, GENERIC);
+          if (rc) return rc;
+          continue;
+        }
         e->ls_hctrl[5] = span;
         CK(e, cudaMemcpyAsync(e->ls_ctrl + 3, e->ls_hctrl + 5, sizeof(uint32_t), cudaMemcpyHostToDevice, e->compute));
         SameTiles t{e->ls_d + pos, e->tiles_dc_next, span, 1u, 0u};
@@ -403,8 +442,8 @@ int run_long(same_engine* e, const int16_t* d_src, uint32_t len) {
         continue;
       }
       const uint32_t end = pos + std::min(window, n - pos);
-      CK(e, same_long_launch_speculative(&e->p, &e->taps2, e->ls_d, pos, end, e->ls_y, e->ls_g, e->ls_gin, e->ls_soft, e->ls_ctrl,
-                                         e->compute));
+      CK(e, same_long_launch_speculative(&e->p, &e->taps2, &e->taps_wide, e->ls_d, pos, end, e->ls_y, e->ls_g, e->ls_gin, e->ls_soft,
+                                         e->ls_ctrl, e->compute));
       e->launches += 4; e->ls_spec_launches += 1;
       CK(e, cudaMemcpyAsync(e->ls_hctrl, e->ls_ctrl, 3 * sizeof(uint32_t), cudaMemcpyDeviceToHost, e->compute));
       CK(e, cudaStreamSynchronize(e->compute));
@@ -417,13 +456,18 @@ int run_long(same_engine* e, const int16_t* d_src, uint32_t len) {
         window = (uint32_t)std::min<uint64_t>(2ull * window, n);
         stops = 0;
       } else {                    // verification stop: the hand-over at `reached` did not match
-        window = std::max(kLongMinPass, window / 2u);
-        unverified = std::min(kLongSpanMax, kLongSpan << std::min(stops, 7u));
+        window = std::max(min_pass, window / 2u);
+        unverified = std::min(span_max, span_locked << std::min(stops, 7u));
         stops += 1;
       }
     }
-    CK(e, same_long_launch_commit_dc(&e->p, e->tiles_dc_next, e->compute));
-    e->launches += 1;
+    if (!general) {
+      CK(e, same_long_launch_commit_dc(&e->p, e->tiles_dc_next, e->compute));
+      e->launches += 1;
+    } else if (dc_at < n) {   // (an ordinary span that ended the chunk has left the state at n)
+      CK(e, same_long_launch_commit_dc_general(&e->p, src, n, e->ls_dc0, e->ls_ma0, e->ls_fbs, e->compute));
+      e->launches += 1;
+    }
   }
   return SAME_OK;
 }
@@ -514,8 +558,9 @@ int submit_common(same_engine* e, const void* host_samples, const void* dev_samp
   CK(e, cudaStreamWaitEvent(e->compute, b.copied, 0));
   CK(e, cudaEventRecord(e->t_k0, e->compute));
   Kernel kernel = rx_kernel(e);
-  // one stream, a long chunk: the long-stream path (time-parallel DC / AGC / matched filters, sequential timing loop)
-  const bool long_path = e->long_stream && e->n_streams == 1 && d_src && e->kernel_override == POLICY && kernel != GENERIC &&
+  // one stream, a long chunk: the long-stream path (time-parallel DC / AGC / matched filters, sequential timing loop), at
+  // any geometry; s16 only: once f32 input reached the state its DC sums need not be integers
+  const bool long_path = e->long_stream && e->n_streams == 1 && d_src && e->kernel_override == POLICY && !e->saw_f32 &&
                          lengths[0] >= kLongMinSamples;
   // the split pipeline's front end needs real samples: a zeros submit has none and takes the fused single-warp kernel
   // (the resident state is the same)

@@ -51,9 +51,14 @@ extern "C" cudaError_t same_launch_init(const SameParams* p, const uint32_t* d_i
 extern "C" cudaError_t same_long_launch_dc(const SameParams* p, const int16_t* d_src, uint32_t len, float* d, uint32_t* dc_next,
                                            cudaStream_t stream);
 extern "C" cudaError_t same_long_launch_commit_dc(const SameParams* p, const uint32_t* dc_next, cudaStream_t stream);
-extern "C" cudaError_t same_long_launch_speculative(const SameParams* p, const SameTaps2* taps2, const float* d, uint32_t pos0,
-                                                    uint32_t end, float* yfull, float* gspec, float* g_in, float* soft,
-                                                    uint32_t* ctrl, cudaStream_t stream);
+// any other DC geometry (same_long.cu, "A, general"): dc0 holds 2 dc_len + 3 words, ma0 len, fbsum len + 2 * 4096 + 64
+extern "C" cudaError_t same_long_launch_dc_general(const SameParams* p, const int16_t* d_src, uint32_t len, uint32_t* dc0, float* ma0,
+                                                   float* fbsum, float* d, cudaStream_t stream);
+extern "C" cudaError_t same_long_launch_commit_dc_general(const SameParams* p, const int16_t* d_src, uint32_t pos, const uint32_t* dc0,
+                                                          const float* ma0, const float* fbsum, cudaStream_t stream);
+extern "C" cudaError_t same_long_launch_speculative(const SameParams* p, const SameTaps2* taps2, const SameTapsWide* taps_wide,
+                                                    const float* d, uint32_t pos0, uint32_t end, float* yfull, float* gspec,
+                                                    float* g_in, float* soft, uint32_t* ctrl, cudaStream_t stream);
 
 // ---- portable stream state, record format and launchers: same_state.cu ----
 extern "C" uint32_t same_state_record_bytes(uint32_t n_words);

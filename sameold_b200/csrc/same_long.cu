@@ -29,6 +29,16 @@
 // arithmetic is the sequential receiver's (same_lane.cuh), so the events are those of the reference, bit for bit
 // (tests: the full 24 h stream, the 16-minute stream in chunks, every single-stream test above the length threshold).
 // All state stays in the ordinary resident layout between kernels; the DC-blocker state is committed at the end.
+//
+// Every other geometry (1..512 taps, DC length 1..512: 11 025, 44 100, 48 000, 88 200-192 000 Hz, 22 050 Hz with another
+// DC length), s16 input only:
+//   A  the general DC front ("A, general" below): the literal f32 recursion of the generic / wide kernels split into an
+//      exact integer feed-forward sum, time-parallel, and the rounded feedback sum as one sequential scan; ma0 and
+//      fbsum are kept for the whole chunk, so that same_long_commit_dcg_kernel can write the state at any position
+//   B, D  the same kernels instantiated for p.ntaps (template argument 0)
+//   C  same_long_mf_wide_kernel: the taps of SameTapsWide, the packed exact FFMA2 pair
+//   bursts and unverified spans   the ordinary generic (or wide) kernel on the raw samples, after a DC commit at the
+//      span's start: the tile-fed and pipelined kernels exist for the 22050 Hz class only.
 #include <cuda_runtime.h>
 
 #include "same_fast.cuh"
@@ -87,13 +97,168 @@ __global__ void same_long_commit_dc_kernel(const __grid_constant__ SameParams p,
   if (threadIdx.x < DCW_WORDS) DcToState{p.state32, L}(threadIdx.x, dc_next[(size_t)threadIdx.x * L.n_pad]);
 }
 
+// -------------------------------------------------------------------------------------------------------- A, general
+// Any other geometry (DC length L = 1..512, s16 samples): the literal f32 recursion of dcblock.rs:45-49,104-108 (as in
+// same_rx_generic_kernel / same_rx_wide_kernel) split into what is exact and what is not.
+//   ffsum[n] = ffsum[n-1] + (x[n] - x[n-L])   every operand an integer, |ffsum| <= 512 * 32768 = 2^24: exact, so it is
+//                                             the integer D + (x[n-L+1] + ... + x[n]) (D = ffsum - window sum of the
+//                                             state, 0 unless the state came from elsewhere), time-parallel
+//   ma0[n]   = ffsum[n] * inv_len             time-parallel
+//   fbsum[n] = fbsum[n-1] + (ma0[n] - ma0[n-L])   rounded (inv_len is not dyadic, or |fbsum| > 2^19 at L = 32): a
+//                                             sequential scan of one thread, tiles staged by the rest of the warp
+//   d[n]     = x[n-L+1] - gate * (fbsum[n] * inv_len)   time-parallel
+// x[m] and ma0[m] for m < 0 are the windows the chunk started with: dc0, a copy of the state's DC words taken before
+// the first launch, because ordinary-kernel spans overwrite the resident words.  Every zero is +0 here as in the
+// recursion (integer input, x - x = +0).  ma0 and fbsum are kept for the whole chunk, so that the state can be
+// committed at any position (same_long_commit_dcg_kernel).
+// dc0 words: [0, L) ff window, [L, 2L) fb window (oldest first), 2L ffsum, 2L+1 fbsum, 2L+2 D (int).
+#define LG_RUN 1024       // samples per thread in the feed-forward kernel
+
+// x[m] of the chunk as an integer, m >= -L
+__device__ __forceinline__ int lg_x(const int16_t* src, const uint32_t* dc0, int L, int m) {
+  return m >= 0 ? (int)src[m] : __float2int_rn(__uint_as_float(dc0[m + L]));
+}
+
+__global__ void __launch_bounds__(512) same_long_dc_save_kernel(const __grid_constant__ SameParams p, uint32_t* __restrict__ dc0) {
+  __shared__ int wsum;
+  const SameLayout& L = p.layout;
+  const uint32_t* st = p.state32;   // stream 0
+  const int dcl = (int)p.dc_len;
+  if (threadIdx.x == 0) wsum = 0;
+  __syncthreads();
+  int part = 0;
+  for (int i = threadIdx.x; i < dcl; i += blockDim.x) {
+    const uint32_t ff = LANE_ST(st, L, L.dc_ff + i);
+    dc0[i] = ff;
+    dc0[dcl + i] = LANE_ST(st, L, L.dc_fb + i);
+    part += __float2int_rn(__uint_as_float(ff));
+  }
+  atomicAdd(&wsum, part);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    const uint32_t ffsum = LANE_ST(st, L, F_DC_FFSUM);
+    dc0[2 * dcl] = ffsum;
+    dc0[2 * dcl + 1] = LANE_ST(st, L, F_DC_FBSUM);
+    dc0[2 * dcl + 2] = (uint32_t)(__float2int_rn(__uint_as_float(ffsum)) - wsum);
+  }
+}
+
+// ma0[n], n in [0, len): one run of LG_RUN samples per thread, the window sum slid along it
+__global__ void same_long_ma0_kernel(const __grid_constant__ SameParams p, const int16_t* __restrict__ src, const uint32_t len,
+                                     const uint32_t* __restrict__ dc0, float* __restrict__ ma0) {
+  const uint32_t r0 = (blockIdx.x * blockDim.x + threadIdx.x) * LG_RUN;
+  if (r0 >= len) return;
+  const uint32_t r1 = min(r0 + (uint32_t)LG_RUN, len);
+  const int dcl = (int)p.dc_len;
+  const float inv_len = p.dc_inv_len;
+  int s = (int)dc0[2 * dcl + 2];                                    // D + the window x[r0-L .. r0-1]
+  for (int m = (int)r0 - dcl; m < (int)r0; ++m) s += lg_x(src, dc0, dcl, m);
+  for (uint32_t n = r0; n < r1; ++n) {
+    s += (int)src[n] - lg_x(src, dc0, dcl, (int)n - dcl);           // = ffsum[n], exact
+    ma0[n] = FMUL(__int2float_rn(s), inv_len);
+  }
+}
+
+// fbs[n] = ma0[n] - ma0[n - L]: the increments the scan adds
+__global__ void same_long_dfb_kernel(const __grid_constant__ SameParams p, const uint32_t len, const uint32_t* __restrict__ dc0,
+                                     const float* __restrict__ ma0, float* __restrict__ fbs) {
+  const uint32_t n = blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= len) return;
+  const uint32_t dcl = p.dc_len;
+  const float aged = n >= dcl ? ma0[n - dcl] : __uint_as_float(dc0[dcl + n]);   // fb window: ma0[m] at dc0[2L + m]
+  fbs[n] = FSUB(ma0[n], aged);
+}
+
+// In place: fbs[n] = fbsum[n] = fbsum[n-1] + fbs[n], from the state's fbsum.  One warp: lane 0 adds (one shared load
+// per 4 samples, 4 dependent FADDs, one shared store); all lanes stage the next tile with 16-byte asynchronous copies
+// and write the finished one back.  `fbs` is padded by two tiles.
+__global__ void __launch_bounds__(32) same_long_fbscan_kernel(const __grid_constant__ SameParams p, const uint32_t len,
+                                                              const uint32_t* __restrict__ dc0, float* __restrict__ fbs) {
+  __shared__ __align__(16) float tile[2][LS_TILE];
+  const uint32_t lane = threadIdx.x;
+  const auto stage = [&](uint32_t tbase, int buf) {
+    const uint32_t dst = (uint32_t)__cvta_generic_to_shared(&tile[buf][0]);
+#pragma unroll 4
+    for (uint32_t j = lane * 4u; j < LS_TILE; j += 128u)
+      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst + j * 4u), "l"(fbs + tbase + j) : "memory");
+    asm volatile("cp.async.commit_group;" ::: "memory");
+  };
+  float f = __uint_as_float(dc0[2 * p.dc_len + 1]);
+  stage(0u, 0);
+  int buf = 0;
+  for (uint32_t tbase = 0; tbase < len; tbase += LS_TILE, buf ^= 1) {
+    stage(tbase + LS_TILE, buf ^ 1);
+    asm volatile("cp.async.wait_group 1;" ::: "memory");
+    __syncwarp();
+    float4* t4 = reinterpret_cast<float4*>(&tile[buf][0]);
+    const uint32_t n4 = (min((uint32_t)LS_TILE, len - tbase) + 3u) / 4u;
+    if (lane == 0) {
+#pragma unroll 8
+      for (uint32_t j = 0; j < n4; ++j) {
+        float4 v = t4[j];
+        f = FADD(f, v.x); v.x = f;
+        f = FADD(f, v.y); v.y = f;
+        f = FADD(f, v.z); v.z = f;
+        f = FADD(f, v.w); v.w = f;
+        t4[j] = v;
+      }
+    }
+    __syncwarp();
+    float4* g4 = reinterpret_cast<float4*>(fbs + tbase);
+    for (uint32_t j = lane; j < n4; j += 32u) g4[j] = t4[j];
+    __syncwarp();
+  }
+  asm volatile("cp.async.wait_group 0;" ::: "memory");
+}
+
+// d[n] = x[n-L+1] - gate * (fbsum[n] * inv_len)
+__global__ void same_long_dcout_kernel(const __grid_constant__ SameParams p, const int16_t* __restrict__ src, const uint32_t len,
+                                       const uint32_t* __restrict__ dc0, const float* __restrict__ fbs, float* __restrict__ d) {
+  const uint32_t n = blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= len) return;
+  const int dcl = (int)p.dc_len;
+  const int m = (int)n - dcl + 1;
+  const float sig = m >= 0 ? (float)src[m] : __uint_as_float(dc0[m + dcl]);
+  d[n] = FSUB(sig, FMUL(p.dc_gate, FMUL(fbs[n], p.dc_inv_len)));
+}
+
+// The generic-layout DC state after sample pos - 1 of the chunk (1 <= pos <= len): windows x[pos-L .. pos-1] and
+// ma0[pos-L .. pos-1], ffsum = D + their sum, fbsum[pos - 1]
+__global__ void __launch_bounds__(512) same_long_commit_dcg_kernel(const __grid_constant__ SameParams p, const int16_t* __restrict__ src,
+                                                                   const uint32_t pos, const uint32_t* __restrict__ dc0,
+                                                                   const float* __restrict__ ma0, const float* __restrict__ fbs) {
+  __shared__ int wsum;
+  const SameLayout& L = p.layout;
+  uint32_t* st = p.state32;   // stream 0
+  const int dcl = (int)p.dc_len;
+  if (threadIdx.x == 0) wsum = 0;
+  __syncthreads();
+  int part = 0;
+  for (int i = threadIdx.x; i < dcl; i += blockDim.x) {
+    const int m = (int)pos - dcl + i;
+    const int x = lg_x(src, dc0, dcl, m);
+    part += x;
+    LANE_ST(st, L, L.dc_ff + i) = m >= 0 ? __float_as_uint((float)x) : dc0[m + dcl];
+    LANE_ST(st, L, L.dc_fb + i) = m >= 0 ? __float_as_uint(ma0[m]) : dc0[2 * dcl + m];
+  }
+  atomicAdd(&wsum, part);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    LANE_ST(st, L, F_DC_FFSUM) = __float_as_uint(__int2float_rn((int)dc0[2 * dcl + 2] + wsum));
+    LANE_ST(st, L, F_DC_FBSUM) = __float_as_uint(fbs[pos - 1u]);
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------------------- B
-// d: DC-blocked samples of the submit; the range is [pos0, end).  yfull[42 + (n - pos0)] = AGC output of sample n,
-// yfull[0..42) = the demod window before pos0 (copied from the state); gspec[n - pos0] = gain AFTER sample n;
-// g_in[k] = the gain block k > 0 started with after its warm-up.
+// d: DC-blocked samples of the submit; the range is [pos0, end).  yfull[ntaps + (n - pos0)] = AGC output of sample n,
+// yfull[0..ntaps) = the demod window before pos0 (copied from the state); gspec[n - pos0] = gain AFTER sample n;
+// g_in[k] = the gain block k > 0 started with after its warm-up.  NT = ntaps, or 0: p.ntaps (general geometry).  The
+// AGC itself has no geometry: its bandwidth per sample is agc_bandwidth / 520.83 at every rate (receiver.rs:511).
+template <int NT>
 __global__ void same_long_agc_kernel(const __grid_constant__ SameParams p, const float* __restrict__ d, const uint32_t pos0,
                                      const uint32_t end, float* __restrict__ yfull, float* __restrict__ gspec,
                                      float* __restrict__ g_in) {
+  const int ntaps = NT ? NT : (int)p.ntaps;
   const SameLayout& L = p.layout;
   const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
   const unsigned long long sk64 = (unsigned long long)pos0 + (unsigned long long)k * LS_BLOCK;
@@ -103,13 +268,13 @@ __global__ void same_long_agc_kernel(const __grid_constant__ SameParams p, const
   const float g_true = __uint_as_float(LANE_ST(p.state32, L, F_AGC_GAIN));   // gain at pos0
   float g = g_true;
   if (k == 0) {
-    for (int i = 0; i < FAST_NTAPS; ++i) yfull[i] = __uint_as_float(LANE_ST(p.state32, L, L.win + i));
+    for (int i = 0; i < ntaps; ++i) yfull[i] = __uint_as_float(LANE_ST(p.state32, L, L.win + i));
   } else {
     for (uint32_t n = sk - LS_WARM; n < sk; ++n) (void)agc_step(g, d[n], bw, gmin, gmax);   // LS_BLOCK >= LS_WARM: n >= pos0
     g_in[k] = g;
   }
   const uint32_t e = min(sk + (uint32_t)LS_BLOCK, end);
-  float* yo = yfull + FAST_NTAPS - pos0;
+  float* yo = yfull + ntaps - pos0;
   float* go = gspec - pos0;
   for (uint32_t n = sk; n < e; ++n) {
     yo[n] = agc_step(g, d[n], bw, gmin, gmax);
@@ -155,6 +320,36 @@ __global__ void __launch_bounds__(256) same_long_mf_kernel(const __grid_constant
   soft[i] = rclamp(FSUB(hypot_fixed(mr, mi), hypot_fixed(sr, si)), -1.0f, 1.0f);
 }
 
+// The same at any geometry (1..512 taps, SameTapsWide): a shared tile of 256 + ntaps - 1 samples, one output per
+// thread, newest sample first with the exact packed FFMA2 pair of same_rx_wide_kernel.
+__global__ void __launch_bounds__(256) same_long_mf_wide_kernel(const __grid_constant__ SameParams p,
+                                                                const __grid_constant__ SameTapsWide taps,
+                                                                const float* __restrict__ yfull, const uint32_t n_out,
+                                                                float* __restrict__ soft) {
+  __shared__ float wtile[256 + SAME_MAX_TAPS - 1];
+  const uint32_t ntaps = p.ntaps;
+  const uint32_t i0 = blockIdx.x * 256u + 1u;
+  for (uint32_t j = threadIdx.x; j < 256u + ntaps - 1u; j += 256u) {
+    const uint32_t idx = i0 + j;                       // yfull index; valid up to n_out + ntaps - 1
+    wtile[j] = (idx <= n_out + ntaps - 1u) ? yfull[idx] : 0.0f;
+  }
+  __syncthreads();
+  const uint32_t i = i0 + threadIdx.x;
+  if (i > n_out) return;
+  const float2 one2 = make_float2(p.f_one, p.f_one), negz2 = make_float2(p.f_negzero, p.f_negzero);
+  float2 am = make_float2(0.0f, 0.0f), as = make_float2(0.0f, 0.0f);
+  const float* yp = wtile + threadIdx.x + ntaps - 1u;   // newest sample of this output's window
+#pragma unroll 4
+  for (uint32_t j = 0; j < ntaps; ++j) {
+    const float v = yp[-(int)j];
+    const float4 t = taps.t[j];
+    const float2 vv = make_float2(v, v);
+    am = __ffma2_rn(am, one2, __ffma2_rn(vv, make_float2(t.x, t.y), negz2));
+    as = __ffma2_rn(as, one2, __ffma2_rn(vv, make_float2(t.z, t.w), negz2));
+  }
+  soft[i] = rclamp(FSUB(hypot_fixed(am.x, am.y), hypot_fixed(as.x, as.y)), -1.0f, 1.0f);
+}
+
 // ---------------------------------------------------------------------------------------------------------------- D
 // Two warps, one lane each doing sequential work, pipelined:
 //   warp T  the timing loop (A5): picks its soft symbol out of the staged tile (the warp's other lanes stage tiles one
@@ -177,6 +372,9 @@ struct LsRec { uint32_t pos; float zero, sym, until, pavg, pinst, ted0; uint32_t
 #endif
 #define LS_TAIL_BATCH 8u
 
+// NT = ntaps, or 0: p.ntaps (general geometry).  Only the demod window stored at the end depends on it: the timing loop
+// runs the same number of TED rounds per second of audio at every rate.
+template <int NT>
 __global__ void __launch_bounds__(64) same_long_seq_kernel(const __grid_constant__ SameParams p, const float* __restrict__ soft,
                                                            const float* __restrict__ yfull, const float* __restrict__ gspec,
                                                            const uint32_t pos0, uint32_t* __restrict__ ctrl) {
@@ -332,7 +530,8 @@ __global__ void __launch_bounds__(64) same_long_seq_kernel(const __grid_constant
   }
   if (pos > 0u) a.g = gspec[pos - 1u];
   lane_store(a, p, st, a.n0 + pos);
-  for (int i = 0; i < FAST_NTAPS; ++i) LANE_ST(st, L, L.win + i) = __float_as_uint(yfull[pos + i]);
+  const int ntaps = NT ? NT : (int)p.ntaps;
+  for (int i = 0; i < ntaps; ++i) LANE_ST(st, L, L.win + i) = __float_as_uint(yfull[pos + i]);
   ctrl[1] = pos0 + pos;
   ctrl[2] = why;
 }
@@ -354,19 +553,48 @@ extern "C" cudaError_t same_long_launch_commit_dc(const SameParams* p, const uin
   return cudaGetLastError();
 }
 
+// General geometry: dc0 (2 dc_len + 3 words) <- the state's DC words; ma0 and fbsum of the chunk's `len` samples; d
+extern "C" cudaError_t same_long_launch_dc_general(const SameParams* p, const int16_t* d_src, uint32_t len, uint32_t* dc0, float* ma0,
+                                                   float* fbsum, float* d, cudaStream_t stream) {
+  const uint32_t runs = (len + LG_RUN - 1u) / LG_RUN;
+  same_dev::same_long_dc_save_kernel<<<1, 512, 0, stream>>>(*p, dc0);
+  same_dev::same_long_ma0_kernel<<<(runs + 127u) / 128u, 128, 0, stream>>>(*p, d_src, len, dc0, ma0);
+  same_dev::same_long_dfb_kernel<<<(len + 255u) / 256u, 256, 0, stream>>>(*p, len, dc0, ma0, fbsum);
+  same_dev::same_long_fbscan_kernel<<<1, 32, 0, stream>>>(*p, len, dc0, fbsum);
+  same_dev::same_long_dcout_kernel<<<(len + 255u) / 256u, 256, 0, stream>>>(*p, d_src, len, dc0, fbsum, d);
+  return cudaGetLastError();
+}
+
+extern "C" cudaError_t same_long_launch_commit_dc_general(const SameParams* p, const int16_t* d_src, uint32_t pos, const uint32_t* dc0,
+                                                          const float* ma0, const float* fbsum, cudaStream_t stream) {
+  if (pos == 0u) return cudaErrorInvalidValue;
+  same_dev::same_long_commit_dcg_kernel<<<1, 512, 0, stream>>>(*p, d_src, pos, dc0, ma0, fbsum);
+  return cudaGetLastError();
+}
+
 // B + verify + C + D for the range [pos0, end) of the submit; ctrl (device, 4 words) receives {verified end, position
-// reached, reason}.  The caller presets nothing: ctrl[0] is set here.
-extern "C" cudaError_t same_long_launch_speculative(const SameParams* p, const SameTaps2* taps2, const float* d, uint32_t pos0,
-                                                    uint32_t end, float* yfull, float* gspec, float* g_in, float* soft,
-                                                    uint32_t* ctrl, cudaStream_t stream) {
+// reached, reason}.  The caller presets nothing: ctrl[0] is set here.  42 taps: the kernels of the 22050 Hz class
+// (taps2); any other tap count: the general instantiations and the wide matched filter (taps_wide).
+extern "C" cudaError_t same_long_launch_speculative(const SameParams* p, const SameTaps2* taps2, const SameTapsWide* taps_wide,
+                                                    const float* d, uint32_t pos0, uint32_t end, float* yfull, float* gspec,
+                                                    float* g_in, float* soft, uint32_t* ctrl, cudaStream_t stream) {
   const uint32_t n = end - pos0;
   const uint32_t blocks = (n + LS_BLOCK - 1u) / LS_BLOCK;
+  const bool fast = p->ntaps == FAST_NTAPS;
   cudaError_t err = cudaMemcpyAsync(ctrl, &end, sizeof(uint32_t), cudaMemcpyHostToDevice, stream);   // pageable source: staged
   if (err != cudaSuccess) return err;
-  same_dev::same_long_agc_kernel<<<(blocks + 63u) / 64u, 64, 0, stream>>>(*p, d, pos0, end, yfull, gspec, g_in);
+  if (fast)
+    same_dev::same_long_agc_kernel<FAST_NTAPS><<<(blocks + 63u) / 64u, 64, 0, stream>>>(*p, d, pos0, end, yfull, gspec, g_in);
+  else
+    same_dev::same_long_agc_kernel<0><<<(blocks + 63u) / 64u, 64, 0, stream>>>(*p, d, pos0, end, yfull, gspec, g_in);
   if (blocks > 1u)
     same_dev::same_long_verify_kernel<<<(blocks - 1u + 127u) / 128u, 128, 0, stream>>>(gspec, g_in, pos0, end, ctrl);
-  same_dev::same_long_mf_kernel<<<(n + 255u) / 256u, 256, 0, stream>>>(*taps2, yfull, n, soft);
-  same_dev::same_long_seq_kernel<<<1, 64, 0, stream>>>(*p, soft, yfull, gspec, pos0, ctrl);
+  if (fast) {
+    same_dev::same_long_mf_kernel<<<(n + 255u) / 256u, 256, 0, stream>>>(*taps2, yfull, n, soft);
+    same_dev::same_long_seq_kernel<FAST_NTAPS><<<1, 64, 0, stream>>>(*p, soft, yfull, gspec, pos0, ctrl);
+  } else {
+    same_dev::same_long_mf_wide_kernel<<<(n + 255u) / 256u, 256, 0, stream>>>(*p, *taps_wide, yfull, n, soft);
+    same_dev::same_long_seq_kernel<0><<<1, 64, 0, stream>>>(*p, soft, yfull, gspec, pos0, ctrl);
+  }
   return cudaGetLastError();
 }
