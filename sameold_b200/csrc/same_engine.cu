@@ -13,7 +13,6 @@
 #include <cstdlib>
 #include <memory>
 #include <string>
-#include <utility>
 #include <vector>
 
 #include "same_internal.h"
@@ -60,64 +59,6 @@ void rate_range(size_t max_taps, uint32_t* lo, uint32_t* hi) {
   *hi = r;
 }
 
-// ---- owned CUDA resources: released when their owner goes, on the device that is current then ----
-
-// An array of T from Alloc, released with Free.  grow() allocates before it releases: a failed allocation leaves the
-// old array in place and clears the runtime's last error, so that the next launcher does not report it as its own.
-template <class T, cudaError_t (*Alloc)(void**, size_t), cudaError_t (*Free)(void*)>
-class Buf {
- public:
-  Buf() = default;
-  Buf(const Buf&) = delete;
-  Buf& operator=(const Buf&) = delete;
-  ~Buf() { if (p_) Free(p_); }
-  operator T*() const { return p_; }
-  size_t size() const { return n_; }   // elements
-  // room for at least n elements (when it has to grow: n + slack); the contents are not kept
-  cudaError_t grow(size_t n, size_t slack = 0) {
-    if (n <= n_) return cudaSuccess;
-    void* q = nullptr;
-    const cudaError_t err = Alloc(&q, (n + slack) * sizeof(T));
-    if (err != cudaSuccess) { cudaGetLastError(); return err; }
-    if (p_) Free(p_);
-    p_ = static_cast<T*>(q); n_ = n + slack;
-    return cudaSuccess;
-  }
-  void swap(Buf& o) { std::swap(p_, o.p_); std::swap(n_, o.n_); }
-
- private:
-  T* p_ = nullptr;
-  size_t n_ = 0;
-};
-template <class T> using DevBuf = Buf<T, cudaMalloc, cudaFree>;
-template <class T> using PinnedBuf = Buf<T, cudaMallocHost, cudaFreeHost>;
-
-class Event {
- public:
-  Event() = default;
-  Event(const Event&) = delete;
-  Event& operator=(const Event&) = delete;
-  ~Event() { if (ev_) cudaEventDestroy(ev_); }
-  cudaError_t create(unsigned flags = cudaEventDefault) { return cudaEventCreateWithFlags(&ev_, flags); }
-  operator cudaEvent_t() const { return ev_; }
-
- private:
-  cudaEvent_t ev_ = nullptr;
-};
-
-class Stream {
- public:
-  Stream() = default;
-  Stream(const Stream&) = delete;
-  Stream& operator=(const Stream&) = delete;
-  ~Stream() { if (st_) cudaStreamDestroy(st_); }
-  cudaError_t create() { return cudaStreamCreateWithFlags(&st_, cudaStreamNonBlocking); }
-  operator cudaStream_t() const { return st_; }
-
- private:
-  cudaStream_t st_ = nullptr;
-};
-
 struct InputBuf {
   DevBuf<uint8_t> d;                     // device samples (s16 or f32)
   DevBuf<unsigned long long> d_off;
@@ -144,16 +85,8 @@ struct same_engine {
   SameTiles tiles{nullptr, nullptr, 0u, 32u, 1u};
   DevBuf<float> tiles_d;
   DevBuf<uint32_t> tiles_dc_next;
-  // long-stream path (same_long.cu): one stream, long chunks
   int long_stream = 1;            // option "long_stream"
-  DevBuf<float> ls_d, ls_y, ls_g, ls_soft, ls_gin;
-  DevBuf<uint32_t> ls_ctrl;       // {verified end, position reached, reason, span length}
-  DevBuf<unsigned long long> ls_off;   // offset of an unverified span in the chunk (ordinary-kernel launch)
-  DevBuf<uint32_t> ls_dc_at;      // DC-blocker state at the start of an unverified span (34 words, word-major)
-  DevBuf<float> ls_ma0, ls_fbs;   // general geometry: ma0 and fbsum of every sample of the chunk
-  DevBuf<uint32_t> ls_dc0;        // general geometry: the DC words the chunk started with (2 dc_len + 3)
-  PinnedBuf<uint32_t> ls_hctrl;   // mirror + scratch
-  uint64_t ls_spec_launches = 0, ls_fallback_launches = 0;
+  LongPath long_path;             // same_long.cu: one stream, long chunks
   bool saw_f32 = false;           // an f32 submit happened since create / reset(all): DC state may be non-integer -> generic kernel
   uint64_t lost_events = 0, lost_payloads = 0;
   uint64_t rollbacks = 0;          // option "rollbacks"
@@ -212,7 +145,6 @@ void bind(same_engine* e) {
   p.events_cap = (uint32_t)std::min<size_t>(e->d_events.size(), 0xffffffffu);
   p.payload_cap = (uint32_t)std::min<size_t>(e->d_payload.size(), 0xffffffffu);
   p.trace = e->d_trace; p.trace_cap = (uint32_t)(e->d_trace.size() / e->n_streams);
-  e->tiles.d = e->tiles_d; e->tiles.dc_next = e->tiles_dc_next;
 }
 
 // Event arenas of exactly these sizes; the old ones stay in use unless all of the new ones could be allocated
@@ -325,152 +257,11 @@ int ensure_tiles(same_engine* e, uint32_t max_len) {
   const uint32_t n_max = (max_len + 31u) & ~31u;
   CK(e, e->tiles_d.grow((size_t)e->p.layout.n_pad * n_max));
   CK(e, e->tiles_dc_next.grow((size_t)34 * e->p.layout.n_pad));
-  e->tiles.n_max = n_max;
-  bind(e);
+  e->tiles.d = e->tiles_d; e->tiles.dc_next = e->tiles_dc_next; e->tiles.n_max = n_max;
   return SAME_OK;
 }
 
-// ---- long-stream path: see same_long.cu ----
-constexpr uint32_t kLongMinSamples = 65536;     // shorter chunks take the ordinary kernels
-constexpr uint32_t kLongChunk = 1u << 24;       // samples per internal pass (bounds the scratch buffers: 16 B per sample)
-constexpr uint32_t kLongSpan = 8192;            // samples per fallback launch while the AGC is locked (inside a burst)
-constexpr uint32_t kLongSpanMax = 1u << 20;     // longest fallback span after verification stops in a row
-constexpr uint32_t kLongMinPass = 1u << 16;     // shortest range of a speculative pass
-// The three above are samples of the 22050 Hz class.  Any other geometry scales them by ntaps / 42, so that they cover
-// the same audio time (the ordinary spans then cost the same share of a stream, and a pass the same number of TED
-// rounds); the speculative AGC's block and warm-up (same_long.cu) stay in samples, its bandwidth per sample being the
-// same at every rate.
-
-// Any geometry but the 22050 Hz class's (42 taps, DC length 16): the general DC front and the ordinary generic kernel
-bool long_general(const same_engine* e) { return e->p.ntaps != 42 || e->p.dc_len != 16; }
-
-int ensure_long(same_engine* e, size_t n) {
-  CK(e, e->ls_d.grow(n + 64));
-  CK(e, e->ls_y.grow(n + 128 + e->p.ntaps));   // + the demod window before the range
-  if (long_general(e)) {
-    CK(e, e->ls_ma0.grow(n + 64));
-    CK(e, e->ls_fbs.grow(n + 2 * 4096 + 64));  // + two tiles: the scan stages ahead
-    CK(e, e->ls_dc0.grow(2 * (size_t)e->p.dc_len + 3));
-  }
-  CK(e, e->ls_g.grow(n + 64));
-  CK(e, e->ls_soft.grow(n + 2 * 4096 + 64));   // + two tiles: the sequential kernel stages ahead
-  CK(e, e->ls_gin.grow(n / 2048 + 8));
-  CK(e, e->ls_ctrl.grow(4));
-  CK(e, e->ls_hctrl.grow(8));
-  CK(e, e->ls_off.grow(1));
-  CK(e, e->ls_dc_at.grow((size_t)34 * e->p.layout.n_pad));
-  CK(e, e->tiles_dc_next.grow((size_t)34 * e->p.layout.n_pad));
-  bind(e);
-  return SAME_OK;
-}
-
-// One stream, `len` device-resident s16 samples, on the compute stream.  Blocks the host (it steers the passes).
-// A speculative pass covers [pos, pos + window).  Where the speculative AGC's hand-overs verify (loud noise, a gain
-// pinned at a limit) the window doubles after every pass that consumed all of it, so a burst-free chunk takes one pass.
-// Where they do not (quiet noise, DESIGN.md §4) a pass stops at its verified end: the window halves, and the samples
-// after that end go to the ordinary pipelined kernel on the raw samples, in a span that doubles with every stop in a
-// row (the DC-blocker state is first brought to the span's start by kernel A).  So no pass costs more than a constant
-// times what it consumes plus what the pass before it consumed, and input that never verifies runs at the ordinary
-// kernel's speed.  Bursts (AGC locked) go to the tile-fed single-warp kernel on A's output, kLongSpan at a time.
-// Any other geometry (long_general): A is the general DC front, which keeps ma0 and fbsum of every sample, and both
-// kinds of span go to the ordinary generic (or wide) kernel on the raw samples after a DC commit at the span's start.
-int run_long(same_engine* e, const int16_t* d_src, uint32_t len) {
-  const SameLayout& L = e->p.layout;
-  const bool general = long_general(e);
-  const auto scaled = [&](uint32_t v) { return general ? (uint32_t)std::max<uint64_t>(1u, (uint64_t)v * e->p.ntaps / 42u) : v; };
-  const uint32_t span_locked = scaled(kLongSpan), span_max = scaled(kLongSpanMax), min_pass = scaled(kLongMinPass);
-  for (uint32_t base = 0; base < len; base += kLongChunk) {
-    const uint32_t n = std::min(kLongChunk, len - base);
-    int rc = ensure_long(e, n);
-    if (rc) return rc;
-    const int16_t* src = d_src + base;
-    if (general) {
-      CK(e, same_long_launch_dc_general(&e->p, src, n, e->ls_dc0, e->ls_ma0, e->ls_fbs, e->ls_d, e->compute));
-      e->launches += 5;
-    } else {
-      CK(e, same_long_launch_dc(&e->p, src, n, e->ls_d, e->tiles_dc_next, e->compute));
-      e->launches += 1;
-    }
-    // dc_at: the position the resident DC-blocker state belongs to (the state words are committed at the chunk's end)
-    uint32_t pos = 0, window = n, unverified = 0, stops = 0, dc_at = 0;
-    // `span` samples from pos on by the ordinary kernel `k` on the raw samples, the DC state first brought to pos
-    const auto ordinary_span = [&](uint32_t span, Kernel k) -> int {
-      if (dc_at < pos) {
-        if (general) {
-          CK(e, same_long_launch_commit_dc_general(&e->p, src, pos, e->ls_dc0, e->ls_ma0, e->ls_fbs, e->compute));
-          e->launches += 1;
-        } else {
-          CK(e, same_long_launch_dc(&e->p, src + dc_at, pos - dc_at, e->ls_y, e->ls_dc_at, e->compute));
-          CK(e, same_long_launch_commit_dc(&e->p, e->ls_dc_at, e->compute));
-          e->launches += 2;
-        }
-      }
-      e->ls_hctrl[5] = span;
-      *reinterpret_cast<unsigned long long*>(e->ls_hctrl + 6) = pos;
-      CK(e, cudaMemcpyAsync(e->ls_ctrl + 3, e->ls_hctrl + 5, sizeof(uint32_t), cudaMemcpyHostToDevice, e->compute));
-      CK(e, cudaMemcpyAsync(e->ls_off, e->ls_hctrl + 6, sizeof(unsigned long long), cudaMemcpyHostToDevice, e->compute));
-      CK(e, same_launch_rx(&e->p, &e->taps, &e->taps2, &e->taps_wide, k, e->lanes_per_warp, src, 0, e->ls_off, e->ls_ctrl + 3, nullptr,
-                           e->compute));
-      e->launches += 1; e->ls_fallback_launches += 1;
-      pos += span;
-      dc_at = pos;
-      return SAME_OK;
-    };
-    while (pos < n) {
-      if (unverified) {   // the span after a verification stop: the ordinary kernel on the raw samples
-        rc = ordinary_span(std::min(unverified, n - pos), general ? GENERIC : PIPE);
-        if (rc) return rc;
-        unverified = 0;
-        continue;
-      }
-      // is the AGC locked (inside a burst)?  then the samples are the ordinary kernel's, span by span
-      CK(e, cudaMemcpyAsync(e->ls_hctrl + 4, e->d_state + (size_t)F_FLAGS * L.n_pad, sizeof(uint32_t), cudaMemcpyDeviceToHost, e->compute));
-      CK(e, cudaStreamSynchronize(e->compute));
-      if (e->ls_hctrl[4] & FLAG_AGC_LOCKED) {
-        const uint32_t span = std::min(span_locked, n - pos);
-        if (general) {
-          rc = ordinary_span(span, GENERIC);
-          if (rc) return rc;
-          continue;
-        }
-        e->ls_hctrl[5] = span;
-        CK(e, cudaMemcpyAsync(e->ls_ctrl + 3, e->ls_hctrl + 5, sizeof(uint32_t), cudaMemcpyHostToDevice, e->compute));
-        SameTiles t{e->ls_d + pos, e->tiles_dc_next, span, 1u, 0u};
-        CK(e, same_launch_rx_tilefed(&e->p, &e->taps2, e->ls_ctrl + 3, &t, e->compute));
-        e->launches += 1; e->ls_fallback_launches += 1;
-        pos += span;
-        continue;
-      }
-      const uint32_t end = pos + std::min(window, n - pos);
-      CK(e, same_long_launch_speculative(&e->p, &e->taps2, &e->taps_wide, e->ls_d, pos, end, e->ls_y, e->ls_g, e->ls_gin, e->ls_soft,
-                                         e->ls_ctrl, e->compute));
-      e->launches += 4; e->ls_spec_launches += 1;
-      CK(e, cudaMemcpyAsync(e->ls_hctrl, e->ls_ctrl, 3 * sizeof(uint32_t), cudaMemcpyDeviceToHost, e->compute));
-      CK(e, cudaStreamSynchronize(e->compute));
-      const uint32_t reached = e->ls_hctrl[1], why = e->ls_hctrl[2];
-      if (reached < pos || reached > end) return fail(e, SAME_ERR_CUDA, "long-stream pass reported an impossible position");
-      if (reached == pos && why == 0u) return fail(e, SAME_ERR_CUDA, "long-stream pass made no progress");
-      pos = reached;
-      if (why != 0u) continue;    // the symbol stages locked the AGC or reset the timing loop: the next round decides
-      if (reached == end) {       // all of the range verified
-        window = (uint32_t)std::min<uint64_t>(2ull * window, n);
-        stops = 0;
-      } else {                    // verification stop: the hand-over at `reached` did not match
-        window = std::max(min_pass, window / 2u);
-        unverified = std::min(span_max, span_locked << std::min(stops, 7u));
-        stops += 1;
-      }
-    }
-    if (!general) {
-      CK(e, same_long_launch_commit_dc(&e->p, e->tiles_dc_next, e->compute));
-      e->launches += 1;
-    } else if (dc_at < n) {   // (an ordinary span that ended the chunk has left the state at n)
-      CK(e, same_long_launch_commit_dc_general(&e->p, src, n, e->ls_dc0, e->ls_ma0, e->ls_fbs, e->compute));
-      e->launches += 1;
-    }
-  }
-  return SAME_OK;
-}
+constexpr uint32_t kLongMinSamples = 65536;   // shorter chunks take the ordinary kernels, not the long-stream path
 
 // The receiver kernel an s16 submit launches:
 //  * the generic kernel once f32 input reached the state (saw_f32): the DC-blocker state may hold non-integers, and
@@ -566,8 +357,10 @@ int submit_common(same_engine* e, const void* host_samples, const void* dev_samp
   // (the resident state is the same)
   if (kernel == SPLIT && !d_src) kernel = SINGLE;
   if (long_path) {
-    int rc = run_long(e, static_cast<const int16_t*>(d_src) + offsets[0], lengths[0]);
-    if (rc) return rc;
+    std::string error;
+    const int rc = same_long_run(&e->long_path, &e->p, &e->taps, &e->taps2, &e->taps_wide, e->lanes_per_warp,
+                                 static_cast<const int16_t*>(d_src) + offsets[0], lengths[0], e->compute, &error);
+    if (rc) return fail(e, rc, error);
   } else {
     if (kernel == SPLIT) {   // a tile buffer for the longest chunk
       uint32_t max_len = 0;
@@ -787,7 +580,7 @@ void same_engine_destroy(same_engine* e) {
 
 uint32_t same_engine_num_streams(const same_engine* e) { return e ? e->n_streams : 0; }
 uint32_t same_engine_input_rate(const same_engine* e) { return e ? e->cfg.input_rate : 0; }
-uint64_t same_engine_launch_count(const same_engine* e) { return e ? e->launches : 0; }
+uint64_t same_engine_launch_count(const same_engine* e) { return e ? e->launches + e->long_path.launches : 0; }
 void* same_engine_cuda_stream(same_engine* e) { return e ? (void*)e->compute : nullptr; }
 
 int same_engine_sync(same_engine* e) {
@@ -1029,8 +822,8 @@ int same_engine_get_option(same_engine* e, const char* key, int* value) {
   if (strcmp(key, "kernel") == 0 || strcmp(key, "force_generic") == 0) { *value = e->kernel_override; return SAME_OK; }
   if (strcmp(key, "device_sort") == 0) { *value = e->device_sort; return SAME_OK; }
   if (strcmp(key, "long_stream") == 0) { *value = e->long_stream; return SAME_OK; }
-  if (strcmp(key, "long_stream_passes") == 0) { *value = (int)std::min<uint64_t>(e->ls_spec_launches, 0x7fffffff); return SAME_OK; }
-  if (strcmp(key, "long_stream_fallback_spans") == 0) { *value = (int)std::min<uint64_t>(e->ls_fallback_launches, 0x7fffffff); return SAME_OK; }
+  if (strcmp(key, "long_stream_passes") == 0) { *value = (int)std::min<uint64_t>(e->long_path.passes, 0x7fffffff); return SAME_OK; }
+  if (strcmp(key, "long_stream_fallback_spans") == 0) { *value = (int)std::min<uint64_t>(e->long_path.fallback_spans, 0x7fffffff); return SAME_OK; }
   if (strcmp(key, "lanes_per_warp") == 0) { *value = (int)e->lanes_per_warp; return SAME_OK; }
   if (strcmp(key, "state_kernel_us") == 0) { *value = (int)std::min(e->st_kernel_ms * 1000.0f, 2.0e9f); return SAME_OK; }
   if (strcmp(key, "state_copy_us") == 0) { *value = (int)std::min(e->st_copy_ms * 1000.0f, 2.0e9f); return SAME_OK; }

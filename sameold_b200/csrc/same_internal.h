@@ -10,6 +10,7 @@
 
 #include <string>
 
+#include "same_owned.h"
 #include "same_params.h"
 
 // `as usize` of Rust: truncating, saturating, NaN -> 0
@@ -47,18 +48,30 @@ extern "C" cudaError_t same_launch_evsort(const same_event* d_events, uint32_t n
 extern "C" cudaError_t same_launch_init(const SameParams* p, const uint32_t* d_ids, uint32_t n, int after_reset,
                                         cudaStream_t stream);
 
-// ---- launchers: same_long.cu ----
-extern "C" cudaError_t same_long_launch_dc(const SameParams* p, const int16_t* d_src, uint32_t len, float* d, uint32_t* dc_next,
-                                           cudaStream_t stream);
-extern "C" cudaError_t same_long_launch_commit_dc(const SameParams* p, const uint32_t* dc_next, cudaStream_t stream);
-// any other DC geometry (same_long.cu, "A, general"): dc0 holds 2 dc_len + 3 words, ma0 len, fbsum len + 2 * 4096 + 64
-extern "C" cudaError_t same_long_launch_dc_general(const SameParams* p, const int16_t* d_src, uint32_t len, uint32_t* dc0, float* ma0,
-                                                   float* fbsum, float* d, cudaStream_t stream);
-extern "C" cudaError_t same_long_launch_commit_dc_general(const SameParams* p, const int16_t* d_src, uint32_t pos, const uint32_t* dc0,
-                                                          const float* ma0, const float* fbsum, cudaStream_t stream);
-extern "C" cudaError_t same_long_launch_speculative(const SameParams* p, const SameTaps2* taps2, const SameTapsWide* taps_wide,
-                                                    const float* d, uint32_t pos0, uint32_t end, float* yfull, float* gspec,
-                                                    float* g_in, float* soft, uint32_t* ctrl, cudaStream_t stream);
+// ---- the long-stream path, same_long.cu: what it owns (scratch for the longest chunk so far, the control words, its
+// counters) and its entry point ----
+struct LongPath {
+  struct Host {                  // pinned; the fields are named by the device words they travel to or from
+    uint32_t verified_end, reached, why;   // <- ctrl[0..2] after a pass (same_long_seq_kernel)
+    uint32_t flags;              // <- the stream's flags word (FLAG_AGC_LOCKED)
+    uint32_t span;               // -> ctrl[3]: the length of an ordinary span
+    unsigned long long off;      // -> off: its offset in the chunk
+  };
+  DevBuf<float> d, y, g, soft, g_in;   // kernels A-D: DC-blocked samples, AGC output and gains, soft symbols, block gains
+  DevBuf<float> ma0, fbsum;      // general geometry: ma0 and fbsum of every sample of the chunk
+  DevBuf<uint32_t> dc0;          // general geometry: the DC words the chunk started with (2 dc_len + 3)
+  DevBuf<uint32_t> dc_next, dc_at;   // 22050 Hz class: A's DC-blocker state at the chunk's end, at an ordinary span's start
+  DevBuf<uint32_t> ctrl;         // ctrl[0..2]: a pass's result, as in Host; ctrl + 3: the ordinary kernel's length array
+  DevBuf<unsigned long long> off;   // the ordinary kernel's offset array
+  PinnedBuf<Host> host;
+  bool uploading = false;        // a copy from `host` is queued that no synchronisation has retired yet
+  uint64_t passes = 0, fallback_spans = 0, launches = 0;   // speculative passes, ordinary spans, kernel launches
+};
+
+// One stream's `len` device-resident s16 samples through the long-stream path on `stream`, at any geometry; blocks
+// the host (it steers the passes).  SAME_OK, or an error code with the message in *error.
+int same_long_run(LongPath* lp, const SameParams* p, const SameTaps* taps, const SameTaps2* taps2, const SameTapsWide* taps_wide,
+                  uint32_t lanes_per_warp, const int16_t* d_src, uint32_t len, cudaStream_t stream, std::string* error);
 
 // ---- portable stream state, record format and launchers: same_state.cu ----
 extern "C" uint32_t same_state_record_bytes(uint32_t n_words);

@@ -24,7 +24,7 @@
 //                             the AGC is unlocked again; then B-D restart from the true state.
 //   unverified spans          after a pass that stopped at its verified end: the ordinary pipelined kernel on the raw
 //                             samples (DC state brought to the span start by A), in spans that grow while the stops
-//                             repeat; the host also bounds each pass's range (run_long, same_engine.cu).
+//                             repeat; the host also bounds each pass's range (same_long_run, at the end of this file).
 // The speculation in B never decides anything: a block is used only after its hand-over gain was verified, and D's
 // arithmetic is the sequential receiver's (same_lane.cuh), so the events are those of the reference, bit for bit
 // (tests: the full 24 h stream, the 16-minute stream in chunks, every single-stream test above the length threshold).
@@ -40,6 +40,9 @@
 //   bursts and unverified spans   the ordinary generic (or wide) kernel on the raw samples, after a DC commit at the
 //      span's start: the tile-fed and pipelined kernels exist for the 22050 Hz class only.
 #include <cuda_runtime.h>
+
+#include <algorithm>
+#include <cstddef>
 
 #include "same_fast.cuh"
 #include "same_internal.h"
@@ -538,63 +541,191 @@ __global__ void __launch_bounds__(64) same_long_seq_kernel(const __grid_constant
 
 }  // namespace same_dev
 
-// ----------------------------------------------------------------------------------------------------------------
-// Launchers (called from same_engine.cu)
-// ----------------------------------------------------------------------------------------------------------------
-extern "C" cudaError_t same_long_launch_dc(const SameParams* p, const int16_t* d_src, uint32_t len, float* d, uint32_t* dc_next,
-                                           cudaStream_t stream) {
-  const uint32_t runs = (len + LS_RUN - 1u) / LS_RUN;
-  same_dev::same_long_dc_kernel<<<(runs + 127u) / 128u, 128, 0, stream>>>(*p, d_src, len, d, dc_next);
-  return cudaGetLastError();
-}
+// ---------------------------------------------------------------- host: the driver (same_long_run) and its operations
+namespace {
 
-extern "C" cudaError_t same_long_launch_commit_dc(const SameParams* p, const uint32_t* dc_next, cudaStream_t stream) {
-  same_dev::same_long_commit_dc_kernel<<<1, 64, 0, stream>>>(*p, dc_next);
-  return cudaGetLastError();
-}
+constexpr uint32_t kLongChunk = 1u << 24;       // samples per internal pass (bounds the scratch buffers: 16 B per sample)
+constexpr uint32_t kLongSpan = 8192;            // samples per ordinary span while the AGC is locked (inside a burst)
+constexpr uint32_t kLongSpanMax = 1u << 20;     // longest ordinary span after verification stops in a row
+constexpr uint32_t kLongMinPass = 1u << 16;     // shortest range of a speculative pass
+// The three above are samples of the 22050 Hz class; any other tap count scales them by ntaps / 42 to cover the same
+// audio time (an ordinary span then costs the same share of a stream, a pass the same number of TED rounds).  The
+// speculative AGC's block and warm-up stay in samples: its bandwidth per sample is the same at every rate.
 
-// General geometry: dc0 (2 dc_len + 3 words) <- the state's DC words; ma0 and fbsum of the chunk's `len` samples; d
-extern "C" cudaError_t same_long_launch_dc_general(const SameParams* p, const int16_t* d_src, uint32_t len, uint32_t* dc0, float* ma0,
-                                                   float* fbsum, float* d, cudaStream_t stream) {
-  const uint32_t runs = (len + LG_RUN - 1u) / LG_RUN;
-  same_dev::same_long_dc_save_kernel<<<1, 512, 0, stream>>>(*p, dc0);
-  same_dev::same_long_ma0_kernel<<<(runs + 127u) / 128u, 128, 0, stream>>>(*p, d_src, len, dc0, ma0);
-  same_dev::same_long_dfb_kernel<<<(len + 255u) / 256u, 256, 0, stream>>>(*p, len, dc0, ma0, fbsum);
-  same_dev::same_long_fbscan_kernel<<<1, 32, 0, stream>>>(*p, len, dc0, fbsum);
-  same_dev::same_long_dcout_kernel<<<(len + 255u) / 256u, 256, 0, stream>>>(*p, d_src, len, dc0, fbsum, d);
-  return cudaGetLastError();
-}
+#define LS_CU(call) do { const cudaError_t _err = (call); if (_err != cudaSuccess) return _err; } while (0)
 
-extern "C" cudaError_t same_long_launch_commit_dc_general(const SameParams* p, const int16_t* d_src, uint32_t pos, const uint32_t* dc0,
-                                                          const float* ma0, const float* fbsum, cudaStream_t stream) {
-  if (pos == 0u) return cudaErrorInvalidValue;
-  same_dev::same_long_commit_dcg_kernel<<<1, 512, 0, stream>>>(*p, d_src, pos, dc0, ma0, fbsum);
-  return cudaGetLastError();
-}
-
-// B + verify + C + D for the range [pos0, end) of the submit; ctrl (device, 4 words) receives {verified end, position
-// reached, reason}.  The caller presets nothing: ctrl[0] is set here.  42 taps: the kernels of the 22050 Hz class
-// (taps2); any other tap count: the general instantiations and the wide matched filter (taps_wide).
-extern "C" cudaError_t same_long_launch_speculative(const SameParams* p, const SameTaps2* taps2, const SameTapsWide* taps_wide,
-                                                    const float* d, uint32_t pos0, uint32_t end, float* yfull, float* gspec,
-                                                    float* g_in, float* soft, uint32_t* ctrl, cudaStream_t stream) {
-  const uint32_t n = end - pos0;
-  const uint32_t blocks = (n + LS_BLOCK - 1u) / LS_BLOCK;
-  const bool fast = p->ntaps == FAST_NTAPS;
-  cudaError_t err = cudaMemcpyAsync(ctrl, &end, sizeof(uint32_t), cudaMemcpyHostToDevice, stream);   // pageable source: staged
-  if (err != cudaSuccess) return err;
-  if (fast)
-    same_dev::same_long_agc_kernel<FAST_NTAPS><<<(blocks + 63u) / 64u, 64, 0, stream>>>(*p, d, pos0, end, yfull, gspec, g_in);
-  else
-    same_dev::same_long_agc_kernel<0><<<(blocks + 63u) / 64u, 64, 0, stream>>>(*p, d, pos0, end, yfull, gspec, g_in);
-  if (blocks > 1u)
-    same_dev::same_long_verify_kernel<<<(blocks - 1u + 127u) / 128u, 128, 0, stream>>>(gspec, g_in, pos0, end, ctrl);
-  if (fast) {
-    same_dev::same_long_mf_kernel<<<(n + 255u) / 256u, 256, 0, stream>>>(*taps2, yfull, n, soft);
-    same_dev::same_long_seq_kernel<FAST_NTAPS><<<1, 64, 0, stream>>>(*p, soft, yfull, gspec, pos0, ctrl);
-  } else {
-    same_dev::same_long_mf_wide_kernel<<<(n + 255u) / 256u, 256, 0, stream>>>(*p, *taps_wide, yfull, n, soft);
-    same_dev::same_long_seq_kernel<0><<<1, 64, 0, stream>>>(*p, soft, yfull, gspec, pos0, ctrl);
+// One call of the driver: the engine's receiver, the chunk in hand, and the operations on it.  Each operation that
+// differs between the 22050 Hz class and any other geometry tests `general` itself; the driver's loop does not.
+struct Run {
+  LongPath& lp;
+  const SameParams& p;
+  const SameTaps& taps; const SameTaps2& taps2; const SameTapsWide& taps_wide;
+  uint32_t lanes_per_warp;
+  cudaStream_t st;
+  bool general;          // any geometry but the 22050 Hz class's (42 taps, DC length 16)
+  const int16_t* src;    // the chunk's samples
+  uint32_t n, dc_at;     // their number; the position the resident DC-blocker state belongs to
+  // The pinned block lp.host carries the control words.  A read-back lands in it and is waited for.  An upload leaves
+  // it when the stream gets there: the host may write it again only after a synchronisation that follows the copy.
+  // The driver reads a word back before every span, so that holds; upload_span() synchronises first should it not.
+  cudaError_t read_back(void* to, const void* from, size_t bytes) {
+    LS_CU(cudaMemcpyAsync(to, from, bytes, cudaMemcpyDeviceToHost, st));
+    lp.uploading = false;
+    return cudaStreamSynchronize(st);
   }
-  return cudaGetLastError();
+  // an ordinary span's length -> ctrl[3] and, unless off is null, its offset in the chunk -> off
+  cudaError_t upload_span(uint32_t span, const uint32_t* off) {
+    LongPath::Host& h = *lp.host;
+    if (lp.uploading) LS_CU(cudaStreamSynchronize(st));
+    lp.uploading = true;
+    h.span = span;
+    LS_CU(cudaMemcpyAsync(lp.ctrl + 3, &h.span, sizeof h.span, cudaMemcpyHostToDevice, st));
+    if (!off) return cudaSuccess;
+    h.off = *off;
+    return cudaMemcpyAsync(lp.off, &h.off, sizeof h.off, cudaMemcpyHostToDevice, st);
+  }
+  // A on the 22050 Hz class: len samples from `from` on -> d, the DC-blocker state after the last of them -> dc_next
+  cudaError_t launch_dc(uint32_t from, uint32_t len, float* d, uint32_t* dc_next) {
+    same_dev::same_long_dc_kernel<<<((len + LS_RUN - 1u) / LS_RUN + 127u) / 128u, 128, 0, st>>>(p, src + from, len, d, dc_next);
+    lp.launches += 1;
+    return cudaGetLastError();
+  }
+  // the 22050 Hz class's DC-blocker state words <- `words` (A's, 34 per stream, word-major)
+  cudaError_t commit_dc(const uint32_t* words) {
+    same_dev::same_long_commit_dc_kernel<<<1, 64, 0, st>>>(p, words);
+    lp.launches += 1;
+    return cudaGetLastError();
+  }
+  // The chunk's scratch, and A over the chunk: d, and what the DC-blocker state is later taken from (general: dc0, ma0
+  // and fbsum; else dc_next)
+  cudaError_t dc_front() {
+    const uint32_t runs = (n + LG_RUN - 1u) / LG_RUN;
+    LS_CU(lp.d.grow((size_t)n + 64));
+    LS_CU(lp.y.grow((size_t)n + 128 + p.ntaps));        // + the demod window before the range
+    LS_CU(lp.g.grow((size_t)n + 64));
+    LS_CU(lp.soft.grow((size_t)n + 2 * LS_TILE + 64));    // + two tiles: D stages ahead
+    LS_CU(lp.g_in.grow(n / LS_BLOCK + 8));
+    LS_CU(lp.dc_next.grow((size_t)DCW_WORDS * p.layout.n_pad));
+    LS_CU(lp.dc_at.grow((size_t)DCW_WORDS * p.layout.n_pad));
+    LS_CU(lp.ctrl.grow(4));
+    LS_CU(lp.off.grow(1));
+    LS_CU(lp.host.grow(1));
+    if (!general) return launch_dc(0, n, lp.d, lp.dc_next);
+    LS_CU(lp.ma0.grow((size_t)n + 64));
+    LS_CU(lp.fbsum.grow((size_t)n + 2 * LS_TILE + 64));   // + two tiles: the scan stages ahead
+    LS_CU(lp.dc0.grow(2 * (size_t)p.dc_len + 3));
+    same_dev::same_long_dc_save_kernel<<<1, 512, 0, st>>>(p, lp.dc0);
+    same_dev::same_long_ma0_kernel<<<(runs + 127u) / 128u, 128, 0, st>>>(p, src, n, lp.dc0, lp.ma0);
+    same_dev::same_long_dfb_kernel<<<(n + 255u) / 256u, 256, 0, st>>>(p, n, lp.dc0, lp.ma0, lp.fbsum);
+    same_dev::same_long_fbscan_kernel<<<1, 32, 0, st>>>(p, n, lp.dc0, lp.fbsum);
+    same_dev::same_long_dcout_kernel<<<(n + 255u) / 256u, 256, 0, st>>>(p, src, n, lp.dc0, lp.fbsum, lp.d);
+    lp.launches += 5;
+    return cudaGetLastError();
+  }
+  // The resident DC-blocker state brought to pos: general, written from dc0, ma0 and fbsum; else A run again from where
+  // the state is (its samples go to y, unused between passes) and its end state committed
+  cudaError_t dc_to(uint32_t pos) {
+    const uint32_t from = dc_at;
+    if (from >= pos) return cudaSuccess;
+    dc_at = pos;
+    if (!general) {
+      LS_CU(launch_dc(from, pos - from, lp.y, lp.dc_at));
+      return commit_dc(lp.dc_at);
+    }
+    same_dev::same_long_commit_dcg_kernel<<<1, 512, 0, st>>>(p, src, pos, lp.dc0, lp.ma0, lp.fbsum);
+    lp.launches += 1;
+    return cudaGetLastError();
+  }
+  // Up to `span` samples from pos on by an ordinary kernel ("bursts" and "unverified spans" at the top of this file; at
+  // any other geometry both go to the generic or wide kernel); pos advances past them
+  cudaError_t ordinary_span(uint32_t& pos, uint32_t span, bool locked) {
+    const uint32_t at = pos;
+    span = std::min(span, n - at);
+    pos += span;
+    lp.launches += 1; lp.fallback_spans += 1;
+    if (locked && !general) {   // tile-fed on A's output: the DC-blocker state words stay as they are (commit_dc 0)
+      LS_CU(upload_span(span, nullptr));
+      const SameTiles t{lp.d + at, lp.dc_next, span, 1u, 0u};
+      return same_launch_rx_tilefed(&p, &taps2, lp.ctrl + 3, &t, st);
+    }
+    LS_CU(dc_to(at));
+    LS_CU(upload_span(span, &at));
+    dc_at = pos;
+    return same_launch_rx(&p, &taps, &taps2, &taps_wide, general ? GENERIC : PIPE, lanes_per_warp, src, 0, lp.off, lp.ctrl + 3, nullptr, st);
+  }
+  // The DC-blocker state words at the chunk's end: general, written there unless an ordinary span ended the chunk; else
+  // A's end state
+  cudaError_t commit() { return general ? dc_to(n) : commit_dc(lp.dc_next); }
+  // B + verify + C + D over [pos0, end) of the chunk, their result in ctrl[0..2].  42 taps: the kernels of the 22050 Hz
+  // class (taps2); any other tap count: the general instantiations and the wide matched filter (taps_wide).
+  cudaError_t pass(uint32_t pos0, uint32_t end) {
+    const uint32_t len = end - pos0, blocks = (len + LS_BLOCK - 1u) / LS_BLOCK;
+    const bool fast = p.ntaps == FAST_NTAPS;
+    LS_CU(cudaMemcpyAsync(lp.ctrl, &end, sizeof(uint32_t), cudaMemcpyHostToDevice, st));   // pageable source: staged
+    if (fast)
+      same_dev::same_long_agc_kernel<FAST_NTAPS><<<(blocks + 63u) / 64u, 64, 0, st>>>(p, lp.d, pos0, end, lp.y, lp.g, lp.g_in);
+    else
+      same_dev::same_long_agc_kernel<0><<<(blocks + 63u) / 64u, 64, 0, st>>>(p, lp.d, pos0, end, lp.y, lp.g, lp.g_in);
+    if (blocks > 1u)
+      same_dev::same_long_verify_kernel<<<(blocks - 1u + 127u) / 128u, 128, 0, st>>>(lp.g, lp.g_in, pos0, end, lp.ctrl);
+    if (fast) {
+      same_dev::same_long_mf_kernel<<<(len + 255u) / 256u, 256, 0, st>>>(taps2, lp.y, len, lp.soft);
+      same_dev::same_long_seq_kernel<FAST_NTAPS><<<1, 64, 0, st>>>(p, lp.soft, lp.y, lp.g, pos0, lp.ctrl);
+    } else {
+      same_dev::same_long_mf_wide_kernel<<<(len + 255u) / 256u, 256, 0, st>>>(p, taps_wide, lp.y, len, lp.soft);
+      same_dev::same_long_seq_kernel<0><<<1, 64, 0, st>>>(p, lp.soft, lp.y, lp.g, pos0, lp.ctrl);
+    }
+    lp.launches += 4; lp.passes += 1;
+    return cudaGetLastError();
+  }
+};
+static_assert(offsetof(LongPath::Host, why) == 2 * sizeof(uint32_t), "ctrl[0..2] are read back in one copy");
+
+}  // namespace
+
+// The driver.  A pass covers [pos, pos + window) of a chunk: the window doubles after every pass that verified all of
+// it (a burst-free chunk at a level where hand-overs verify takes one pass) and halves after every verification stop,
+// whose unverified span doubles with every stop in a row.  So no pass costs more than a constant times what it
+// consumes plus what the pass before it consumed, and input that never verifies runs at the ordinary kernel's speed.
+#define LS_CK(call) \
+  do { const cudaError_t _err = (call); if (_err != cudaSuccess) return fail(std::string(#call) + ": " + cudaGetErrorString(_err)); } while (0)
+
+int same_long_run(LongPath* lp, const SameParams* p, const SameTaps* taps, const SameTaps2* taps2, const SameTapsWide* taps_wide,
+                  uint32_t lanes_per_warp, const int16_t* d_src, uint32_t len, cudaStream_t stream, std::string* error) {
+  const auto fail = [error](const std::string& msg) { *error = msg; return SAME_ERR_CUDA; };
+  Run r{*lp, *p, *taps, *taps2, *taps_wide, lanes_per_warp, stream, p->ntaps != FAST_NTAPS || p->dc_len != 16, nullptr, 0, 0};
+  const auto scaled = [p](uint32_t v) { return (uint32_t)std::max<uint64_t>(1u, (uint64_t)v * p->ntaps / FAST_NTAPS); };
+  const uint32_t span_locked = scaled(kLongSpan), span_max = scaled(kLongSpanMax), min_pass = scaled(kLongMinPass);
+  for (uint32_t base = 0; base < len; base += kLongChunk) {
+    const uint32_t n = std::min(kLongChunk, len - base);
+    r.src = d_src + base; r.n = n; r.dc_at = 0;
+    LS_CK(r.dc_front());
+    LongPath::Host& h = *lp->host;
+    uint32_t pos = 0, window = n, stops = 0;
+    while (pos < n) {
+      LS_CK(r.read_back(&h.flags, p->state32 + (size_t)F_FLAGS * p->layout.n_pad, sizeof(uint32_t)));   // stream 0
+      if (h.flags & FLAG_AGC_LOCKED) {   // inside a burst: the samples are the ordinary kernel's, span by span
+        LS_CK(r.ordinary_span(pos, span_locked, true));
+        continue;
+      }
+      const uint32_t end = pos + std::min(window, n - pos);
+      LS_CK(r.pass(pos, end));
+      LS_CK(r.read_back(&h.verified_end, lp->ctrl, 3 * sizeof(uint32_t)));
+      if (h.reached < pos || h.reached > end) return fail("long-stream pass reported an impossible position");
+      if (h.reached == pos && h.why == 0u) return fail("long-stream pass made no progress");
+      pos = h.reached;
+      if (h.why != 0u) continue;   // the symbol stages locked the AGC or reset the timing loop: the next round decides
+      if (pos == end) {            // all of the range verified
+        window = (uint32_t)std::min<uint64_t>(2ull * window, n);
+        stops = 0;
+        continue;
+      }
+      // verification stop: the hand-over at pos did not match, and the span after it goes to an ordinary kernel
+      window = std::max(min_pass, window / 2u);
+      LS_CK(r.ordinary_span(pos, std::min(span_max, span_locked << std::min(stops, 7u)), false));
+      stops += 1;
+    }
+    LS_CK(r.commit());
+  }
+  return SAME_OK;
 }
