@@ -136,6 +136,36 @@ impl SameBatchReceiver {
         self.drain()
     }
 
+    /// Interleaved multi-channel PCM: `frames` holds whole frames of `n_channels` samples in `format` (`SAME_FMT_*`;
+    /// s24 is 3-byte packed little-endian).  Sample c of frame n becomes sample n of stream `channel_stream[c]`
+    /// (`None`: stream c; `SAME_CHANNEL_SKIP`: dropped).  Deinterleaved and converted (`sa as f32` for s24 / s32) on
+    /// the GPU; no downmix, no resampling.
+    pub fn process_interleaved(&mut self, frames: &[u8], format: u32, n_channels: u32, channel_stream: Option<&[u32]>)
+                               -> Result<Vec<BatchedEvent>, String> {
+        let bytes = match format {
+            SAME_FMT_S16 => 2,
+            SAME_FMT_S24 => 3,
+            SAME_FMT_S32 | SAME_FMT_F32 => 4,
+            _ => return Err(format!("unknown sample format {}", format)),
+        };
+        let frame = bytes * n_channels as usize;
+        if frame == 0 || frames.len() % frame != 0 {
+            return Err(format!("{} bytes is not a whole number of {}-byte frames", frames.len(), frame));
+        }
+        if let Some(m) = channel_stream {
+            if m.len() != n_channels as usize {
+                return Err(format!("channel_stream has {} entries for {} channels", m.len(), n_channels));
+            }
+        }
+        let map = channel_stream.map_or(ptr::null(), |m| m.as_ptr());
+        unsafe {
+            check(self.multi, same_multi_submit_interleaved(self.multi, frames.as_ptr() as *const _, format, n_channels,
+                                                            (frames.len() / frame) as u64, map))?;
+            check(self.multi, same_multi_sync(self.multi))?;
+        }
+        self.drain()
+    }
+
     /// == `iter_messages` for every stream: `(stream, Message)` in order of occurrence per stream.
     pub fn iter_messages_batched(&mut self, chunks: &[&[i16]]) -> Result<Vec<(u32, Message)>, String> {
         Ok(self

@@ -96,6 +96,14 @@ pub struct same_derived {
     pub ntaps: u32,
 }
 
+/// `enum same_sample_format`: the sample formats of an interleaved submit
+pub const SAME_FMT_S16: u32 = 0;
+pub const SAME_FMT_S24: u32 = 1;
+pub const SAME_FMT_S32: u32 = 2;
+pub const SAME_FMT_F32: u32 = 3;
+/// A `channel_stream` entry that drops its channel
+pub const SAME_CHANNEL_SKIP: u32 = 0xFFFF_FFFF;
+
 extern "C" {
     pub fn same_abi_version() -> u32;
     pub fn same_config_default(cfg: *mut same_config, input_rate: u32);
@@ -116,6 +124,10 @@ extern "C" {
     pub fn same_engine_submit_f32_device(e: *mut same_engine, d_samples: *const f32, total_samples: u64, offsets: *const u64,
                                          lengths: *const u32) -> c_int;
     pub fn same_engine_submit_zeros(e: *mut same_engine, lengths: *const u32) -> c_int;
+    pub fn same_engine_submit_interleaved(e: *mut same_engine, frames: *const c_void, format: u32, n_channels: u32, n_frames: u64,
+                                          channel_stream: *const u32) -> c_int;
+    pub fn same_engine_submit_interleaved_device(e: *mut same_engine, d_frames: *const c_void, format: u32, n_channels: u32,
+                                                 n_frames: u64, channel_stream: *const u32) -> c_int;
     pub fn same_engine_lost_events(e: *mut same_engine, events_lost: *mut u64, payloads_lost: *mut u64) -> c_int;
     pub fn same_engine_sync(e: *mut same_engine) -> c_int;
     pub fn same_engine_pending(e: *mut same_engine, n_events: *mut usize, n_payload: *mut usize) -> c_int;
@@ -165,6 +177,8 @@ extern "C" {
     pub fn same_multi_submit_s16(m: *mut same_multi, samples: *const i16, total_samples: u64, offsets: *const u64, lengths: *const u32) -> c_int;
     pub fn same_multi_submit_f32(m: *mut same_multi, samples: *const f32, total_samples: u64, offsets: *const u64, lengths: *const u32) -> c_int;
     pub fn same_multi_submit_s16_2d(m: *mut same_multi, samples: *const i16, row_stride: u64, col_start: u64, n_cols: u32) -> c_int;
+    pub fn same_multi_submit_interleaved(m: *mut same_multi, frames: *const c_void, format: u32, n_channels: u32, n_frames: u64,
+                                         channel_stream: *const u32) -> c_int;
     pub fn same_multi_submit_zeros(m: *mut same_multi, lengths: *const u32) -> c_int;
     pub fn same_multi_sync(m: *mut same_multi) -> c_int;
     pub fn same_multi_reset(m: *mut same_multi) -> c_int;

@@ -220,6 +220,32 @@ int same_engine_submit_f32(same_engine* e, const float* samples, uint64_t total_
                            const uint32_t* lengths);
 int same_engine_submit_f32_device(same_engine* e, const float* d_samples, uint64_t total_samples,
                                   const uint64_t* offsets, const uint32_t* lengths);
+/* Interleaved multi-channel PCM, as audio interfaces, multi-channel WAV files and SDR channelisers deliver it:
+ * `n_frames` frames of `n_channels` samples each, in one of these formats (native / little endian):
+ *   SAME_FMT_S16  int16                          -> the stream gets the int16 value, exactly as same_engine_submit_s16
+ *   SAME_FMT_S24  3-byte packed little-endian, sign-extended -> `sa as f32`, exact
+ *   SAME_FMT_S32  int32                          -> `sa as f32`: round to nearest, ties to even (2^24 + 1 -> 2^24)
+ *   SAME_FMT_F32  float                          -> the value itself
+ * Sample c of frame n becomes sample n of stream channel_stream[c]: no downmix, no resampling, no scaling.
+ * channel_stream == NULL maps channel c to stream c (n_channels <= n_streams); SAME_CHANNEL_SKIP drops a channel; a
+ * stream no channel feeds gets no samples (as length 0 in same_engine_submit_s16).  S24, S32 and F32 channels take the
+ * f32 path of same_engine_submit_f32 (the engine stays on the rate-generic kernel until same_engine_reset(all)); S16
+ * channels take the s16 path, the long-stream path included.  Chunked submits equal one long submit and equal planar
+ * submits of the same channels, bit for bit.
+ * The frames are deinterleaved on the device: the host variant copies the bytes of the mapped channels' column range
+ * [cmin, cmax] (one flat copy, or one strided cudaMemcpy2DAsync when the range is narrower than a frame) into a staging
+ * buffer and converts them there, on the copy stream, overlapped with the previous submit's receiver kernel.
+ * same_engine_last_timing's h2d_ms covers that copy and the conversion; the conversion counts as one launch.
+ * SAME_ERR_INVALID_ARG, with nothing changed, for an unknown format, n_channels == 0, n_frames > 2^30, a stream id out
+ * of range or named twice (the message names the channel), or a NULL pointer with n_frames > 0. */
+enum same_sample_format { SAME_FMT_S16 = 0, SAME_FMT_S24 = 1, SAME_FMT_S32 = 2, SAME_FMT_F32 = 3 };
+#define SAME_CHANNEL_SKIP 0xFFFFFFFFu
+int same_engine_submit_interleaved(same_engine* e, const void* frames, uint32_t format, uint32_t n_channels,
+                                   uint64_t n_frames, const uint32_t* channel_stream);
+/* Same, but `d_frames` already lives in this device's memory (any alignment): no copy; the conversion runs on the
+ * engine's stream (same_engine_cuda_stream), after whatever the caller queued there. */
+int same_engine_submit_interleaved_device(same_engine* e, const void* d_frames, uint32_t format, uint32_t n_channels,
+                                          uint64_t n_frames, const uint32_t* channel_stream);
 /* Feed lengths[i] zero samples to stream i: the body of SameReceiver::flush (receiver.rs:216-224) without its early
  * return; the host layer applies samedec's repeat-until-quiet rule (app.rs:71-74,118). */
 int same_engine_submit_zeros(same_engine* e, const uint32_t* lengths);
@@ -270,8 +296,9 @@ int same_engine_get_option(same_engine* e, const char* key, int* value);
  * receiver state is not changed. */
 int same_engine_frontend_probe(same_engine* e, const int16_t* d_samples, uint64_t total_samples, const uint64_t* offsets,
                                const uint32_t* lengths, int reps, float* ms_per_launch);
-/* Timing of the last completed submit, measured with CUDA events on the engine's stream: host->device copy and
- * receiver kernel, in milliseconds; kernel launch count since create (for bench.py's gpu_launches). */
+/* Timing of the last completed submit, measured with CUDA events on the engine's stream: host->device copy (for an
+ * interleaved submit: the copy and the conversion to planar rows) and receiver kernel, in milliseconds; kernel launch
+ * count since create (for bench.py's gpu_launches). */
 int same_engine_last_timing(same_engine* e, float* h2d_ms, float* kernel_ms);
 uint64_t same_engine_launch_count(const same_engine* e);
 /* Device-side stopwatch over everything submitted between start and stop (host->device copies, kernels), taken with
@@ -327,6 +354,10 @@ int same_multi_submit_f32(same_multi* m, const float* samples, uint64_t total_sa
 /* HOST matrix samples[n_streams][row_stride]: device i takes its own rows, columns [col_start, col_start + n_cols). */
 int same_multi_submit_s16_2d(same_multi* m, const int16_t* samples, uint64_t row_stride, uint64_t col_start,
                              uint32_t n_cols);
+/* Interleaved frames (same_engine_submit_interleaved) with GLOBAL stream ids in channel_stream: each device copies and
+ * converts only the column range of its own streams' channels. */
+int same_multi_submit_interleaved(same_multi* m, const void* frames, uint32_t format, uint32_t n_channels,
+                                  uint64_t n_frames, const uint32_t* channel_stream);
 int same_multi_submit_zeros(same_multi* m, const uint32_t* lengths);
 int same_multi_sync(same_multi* m);
 int same_multi_reset(same_multi* m);

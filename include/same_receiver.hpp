@@ -19,6 +19,7 @@
 #include <optional>
 #include <stdexcept>
 #include <string>
+#include <type_traits>
 #include <utility>
 #include <vector>
 
@@ -162,6 +163,36 @@ class SameBatchReceiver {
     ck(same_engine_sync(e_));
     return drain_by_stream();
   }
+  // Interleaved multi-channel PCM (same_engine_submit_interleaved): `frames` holds whole frames of n_channels samples
+  // in `format` (SAME_FMT_*); sample c of frame n feeds stream channel_stream[c] (empty: stream c; SAME_CHANNEL_SKIP:
+  // dropped).  Deinterleaved and converted on the GPU.
+  void submit_interleaved(const void* frames, uint32_t format, uint32_t n_channels, uint64_t n_frames,
+                          const std::vector<uint32_t>& channel_stream = {}) {
+    check_map(channel_stream, n_channels);
+    ck(same_engine_submit_interleaved(e_, frames, format, n_channels, n_frames, channel_stream.empty() ? nullptr : channel_stream.data()));
+  }
+  std::vector<std::vector<SameReceiverEvent>> process_interleaved(const void* frames, uint32_t format, uint32_t n_channels,
+                                                                  uint64_t n_frames, const std::vector<uint32_t>& channel_stream = {}) {
+    submit_interleaved(frames, format, n_channels, n_frames, channel_stream);
+    ck(same_engine_sync(e_));
+    return drain_by_stream();
+  }
+  template <class T>   // int16_t, int32_t or float frames: the format follows from the type
+  std::vector<std::vector<SameReceiverEvent>> process_interleaved(const std::vector<T>& frames, uint32_t n_channels,
+                                                                  const std::vector<uint32_t>& channel_stream = {}) {
+    static_assert(std::is_same<T, int16_t>::value || std::is_same<T, int32_t>::value || std::is_same<T, float>::value,
+                  "interleaved frames are int16_t, int32_t or float (s24: the void* overload)");
+    const uint32_t fmt = std::is_same<T, int16_t>::value ? SAME_FMT_S16 : std::is_same<T, int32_t>::value ? SAME_FMT_S32 : SAME_FMT_F32;
+    if (n_channels == 0 || frames.size() % n_channels) throw std::invalid_argument("not a whole number of frames");
+    return process_interleaved(frames.data(), fmt, n_channels, frames.size() / n_channels, channel_stream);
+  }
+  // frames already in this device's memory
+  void submit_interleaved_device(const void* d_frames, uint32_t format, uint32_t n_channels, uint64_t n_frames,
+                                 const std::vector<uint32_t>& channel_stream = {}) {
+    check_map(channel_stream, n_channels);
+    ck(same_engine_submit_interleaved_device(e_, d_frames, format, n_channels, n_frames, channel_stream.empty() ? nullptr : channel_stream.data()));
+  }
+  void sync() { ck(same_engine_sync(e_)); }
   std::vector<std::vector<SameReceiverEvent>> process_zeros(const std::vector<uint32_t>& lengths) {
     ck(same_engine_submit_zeros(e_, lengths.data())); ck(same_engine_sync(e_)); return drain_by_stream();
   }
@@ -232,6 +263,9 @@ class SameBatchReceiver {
 
  private:
   void ck(int rc) { if (rc) throw EngineError(rc, same_engine_last_error(e_)); }
+  static void check_map(const std::vector<uint32_t>& channel_stream, uint32_t n_channels) {
+    if (!channel_stream.empty() && channel_stream.size() != n_channels) throw std::invalid_argument("one channel_stream entry per channel expected");
+  }
   std::vector<std::vector<SameReceiverEvent>> drain_by_stream() {
     size_t nev = 0, npay = 0;
     ck(same_engine_pending(e_, &nev, &npay));

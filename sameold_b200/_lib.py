@@ -83,6 +83,8 @@ API = {
     "same_engine_submit_f32": (C.c_int, [_P, _P, C.c_uint64, _P, _P]),
     "same_engine_submit_f32_device": (C.c_int, [_P, _P, C.c_uint64, _P, _P]),
     "same_engine_submit_zeros": (C.c_int, [_P, _P]),
+    "same_engine_submit_interleaved": (C.c_int, [_P, _P, C.c_uint32, C.c_uint32, C.c_uint64, _P]),
+    "same_engine_submit_interleaved_device": (C.c_int, [_P, _P, C.c_uint32, C.c_uint32, C.c_uint64, _P]),
     "same_engine_lost_events": (C.c_int, [_P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "same_engine_sync": (C.c_int, [_P]),
     "same_engine_pending": (C.c_int, [_P, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
@@ -112,6 +114,7 @@ API = {
     "same_multi_submit_s16": (C.c_int, [_P, _P, C.c_uint64, _P, _P]),
     "same_multi_submit_f32": (C.c_int, [_P, _P, C.c_uint64, _P, _P]),
     "same_multi_submit_s16_2d": (C.c_int, [_P, _P, C.c_uint64, C.c_uint64, C.c_uint32]),
+    "same_multi_submit_interleaved": (C.c_int, [_P, _P, C.c_uint32, C.c_uint32, C.c_uint64, _P]),
     "same_multi_submit_zeros": (C.c_int, [_P, _P]),
     "same_multi_sync": (C.c_int, [_P]),
     "same_multi_reset": (C.c_int, [_P]),

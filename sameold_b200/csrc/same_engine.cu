@@ -61,6 +61,8 @@ void rate_range(size_t max_taps, uint32_t* lo, uint32_t* hi) {
 
 struct InputBuf {
   DevBuf<uint8_t> d;                     // device samples (s16 or f32)
+  DevBuf<uint8_t> raw;                   // interleaved submit: the frames' bytes as copied from the host
+  DevBuf<int32_t> row;                   // interleaved submit: the output row of each copied column, -1 = none
   DevBuf<unsigned long long> d_off;
   DevBuf<uint32_t> d_len;
   Event copied, consumed;
@@ -289,12 +291,47 @@ Kernel rx_kernel(const same_engine* e) {
 
 struct Submit2D { uint64_t row_stride = 0, col_start = 0, dpitch = 0; uint32_t n_cols = 0; bool on = false; };
 
+// Interleaved frames (same_engine_submit_interleaved): host_samples or dev_samples point at frame 0
+struct SubmitInterleaved { uint32_t format = 0, n_channels = 0; uint64_t n_frames = 0; const uint32_t* map = nullptr; bool on = false; };
+
 // sample_fmt: 0 = int16, 1 = float32
 int submit_common(same_engine* e, const void* host_samples, const void* dev_samples, int sample_fmt, uint64_t total,
-                  const uint64_t* offsets, const uint32_t* lengths, bool zeros, Submit2D two_d = Submit2D()) {
+                  const uint64_t* offsets, const uint32_t* lengths, bool zeros, Submit2D two_d = Submit2D(),
+                  SubmitInterleaved il = SubmitInterleaved()) {
   if (!e) return fail(nullptr, SAME_ERR_INVALID_ARG, "null engine");
   std::vector<uint64_t> off2d;
   std::vector<uint32_t> len2d;
+  // interleaved: every mapped channel becomes one row of the device buffer, in channel order, at a pitch of a multiple
+  // of 8 samples (as for the 2-D submit); il_row[c - il_cmin] is the row of channel c, -1 for a skipped one
+  std::vector<int32_t> il_row;
+  uint32_t il_cmin = 0;
+  uint64_t il_dpitch = 0;
+  if (il.on) {
+    std::string why;
+    if (same_check_interleaved(host_samples ? host_samples : dev_samples, il.format, il.n_channels, il.n_frames, il.map,
+                               e->n_streams, &why))
+      return fail(e, SAME_ERR_INVALID_ARG, why);
+    uint32_t cmax = 0;
+    il_cmin = UINT32_MAX;
+    for (uint32_t c = 0; c < il.n_channels; ++c)
+      if ((il.map ? il.map[c] : c) != SAME_CHANNEL_SKIP) { il_cmin = std::min(il_cmin, c); cmax = c; }
+    il_dpitch = (il.n_frames + 7u) & ~(uint64_t)7u;
+    off2d.assign(e->n_streams, 0); len2d.assign(e->n_streams, 0);
+    uint32_t rows = 0;
+    if (il_cmin <= cmax) {
+      il_row.assign(cmax - il_cmin + 1u, -1);
+      for (uint32_t c = il_cmin; c <= cmax; ++c) {
+        const uint32_t s = il.map ? il.map[c] : c;
+        if (s == SAME_CHANNEL_SKIP) continue;
+        il_row[c - il_cmin] = (int32_t)rows;
+        off2d[s] = (uint64_t)rows * il_dpitch; len2d[s] = (uint32_t)il.n_frames;
+        ++rows;
+      }
+    }
+    offsets = off2d.data(); lengths = len2d.data();
+    total = (uint64_t)rows * il_dpitch;
+    sample_fmt = il.format == SAME_FMT_S16 ? 0 : 1;
+  }
   if (two_d.on) {
     if (!host_samples) return fail(e, SAME_ERR_INVALID_ARG, "null argument");
     if (two_d.col_start + two_d.n_cols > two_d.row_stride) return fail(e, SAME_ERR_INVALID_ARG, "column range exceeds row_stride");
@@ -330,7 +367,37 @@ int submit_common(same_engine* e, const void* host_samples, const void* dev_samp
     CK(e, cudaMemcpyAsync(b.d_off, offsets, e->n_streams * sizeof(uint64_t), cudaMemcpyHostToDevice, e->copy));
   }
   CK(e, cudaMemcpyAsync(b.d_len, lengths, e->n_streams * sizeof(uint32_t), cudaMemcpyHostToDevice, e->copy));
-  if (!zeros && host_samples) {
+  // interleaved: the copied frames (host) or the caller's (device) -> planar rows of b.d, one launch on `st`
+  auto ingest = [&](cudaStream_t st, const uint8_t* src, uint64_t pitch) -> int {
+    CK(e, same_launch_ingest(il.format, src, pitch, (uint32_t)il_row.size(), (uint32_t)il.n_frames, b.row, b.d, il_dpitch, st));
+    e->launches += 1;
+    CK(e, cudaEventRecord(e->t_h2d1, st));
+    e->timed_h2d = true;
+    return SAME_OK;
+  };
+  const uint32_t isz = same_format_bytes(il.format);
+  if (il.on && total) {
+    CK(e, b.d.grow(total * ssz, total * ssz / 8 + 8192));
+    CK(e, b.row.grow(il_row.size()));
+    CK(e, cudaMemcpyAsync(b.row, il_row.data(), il_row.size() * sizeof(int32_t), cudaMemcpyHostToDevice, e->copy));
+  }
+  if (il.on && total && host_samples) {
+    // only the bytes of the mapped channels' column range: one flat copy when that is the whole frame, else one
+    // strided copy with a row per frame
+    const uint64_t width = (uint64_t)il_row.size() * isz, fpitch = (uint64_t)il.n_channels * isz;
+    const uint8_t* src = static_cast<const uint8_t*>(host_samples) + (uint64_t)il_cmin * isz;
+    CK(e, b.raw.grow(width * il.n_frames, width * il.n_frames / 8 + 8192));
+    CK(e, cudaEventRecord(e->t_h2d0, e->copy));
+    if (width == fpitch)
+      CK(e, cudaMemcpyAsync(b.raw, src, width * il.n_frames, cudaMemcpyHostToDevice, e->copy));
+    else
+      CK(e, cudaMemcpy2DAsync(b.raw, width, src, fpitch, width, il.n_frames, cudaMemcpyHostToDevice, e->copy));
+    const int rc = ingest(e->copy, b.raw, width);
+    if (rc) return rc;
+    d_src = b.d;
+  } else if (il.on) {
+    d_src = b.d;
+  } else if (!zeros && host_samples) {
     CK(e, b.d.grow(total * ssz, total * ssz / 8 + 8192));
     CK(e, cudaEventRecord(e->t_h2d0, e->copy));
     if (total && two_d.on)
@@ -347,6 +414,12 @@ int submit_common(same_engine* e, const void* host_samples, const void* dev_samp
   }
   CK(e, cudaEventRecord(b.copied, e->copy));
   CK(e, cudaStreamWaitEvent(e->compute, b.copied, 0));
+  if (il.on && total && dev_samples) {   // ordered after the caller's work on the engine's stream
+    CK(e, cudaEventRecord(e->t_h2d0, e->compute));
+    const int rc = ingest(e->compute, static_cast<const uint8_t*>(dev_samples) + (uint64_t)il_cmin * isz,
+                          (uint64_t)il.n_channels * isz);
+    if (rc) return rc;
+  }
   CK(e, cudaEventRecord(e->t_k0, e->compute));
   Kernel kernel = rx_kernel(e);
   // one stream, a long chunk: the long-stream path (time-parallel DC / AGC / matched filters, sequential timing loop), at
@@ -382,6 +455,31 @@ int submit_common(same_engine* e, const void* host_samples, const void* dev_samp
 }
 
 }  // namespace
+
+int same_check_interleaved(const void* frames, uint32_t format, uint32_t n_channels, uint64_t n_frames,
+                           const uint32_t* channel_stream, uint32_t n_streams, std::string* why) {
+  auto bad = [why](const std::string& msg) { *why = msg; return (int)SAME_ERR_INVALID_ARG; };
+  if (!same_format_bytes(format)) return bad("unknown sample format " + std::to_string(format));
+  if (n_channels == 0) return bad("n_channels is 0");
+  if (n_frames > (1u << 30)) return bad("chunk longer than 2^30 samples");
+  if (!frames && n_frames) return bad("null argument");
+  if (!channel_stream) {
+    if (n_channels > n_streams)
+      return bad("channel " + std::to_string(n_streams) + ": no stream " + std::to_string(n_streams) + " (channel_stream == NULL maps channel c to stream c, and there are " +
+                 std::to_string(n_streams) + " streams)");
+    return SAME_OK;
+  }
+  std::vector<uint32_t> fed_by(n_streams, SAME_CHANNEL_SKIP);
+  for (uint32_t c = 0; c < n_channels; ++c) {
+    const uint32_t s = channel_stream[c];
+    if (s == SAME_CHANNEL_SKIP) continue;
+    if (s >= n_streams) return bad("channel " + std::to_string(c) + ": stream id " + std::to_string(s) + " out of range");
+    if (fed_by[s] != SAME_CHANNEL_SKIP)
+      return bad("channel " + std::to_string(c) + ": stream " + std::to_string(s) + " is already fed by channel " + std::to_string(fed_by[s]));
+    fed_by[s] = c;
+  }
+  return SAME_OK;
+}
 
 extern "C" {
 
@@ -718,6 +816,18 @@ int same_engine_submit_s16_device(same_engine* e, const int16_t* d_samples, uint
 
 int same_engine_submit_zeros(same_engine* e, const uint32_t* lengths) {
   return submit_common(e, nullptr, nullptr, 0, 0, nullptr, lengths, true);
+}
+
+int same_engine_submit_interleaved(same_engine* e, const void* frames, uint32_t format, uint32_t n_channels,
+                                   uint64_t n_frames, const uint32_t* channel_stream) {
+  SubmitInterleaved il; il.format = format; il.n_channels = n_channels; il.n_frames = n_frames; il.map = channel_stream; il.on = true;
+  return submit_common(e, frames, nullptr, 0, 0, nullptr, nullptr, false, Submit2D(), il);
+}
+
+int same_engine_submit_interleaved_device(same_engine* e, const void* d_frames, uint32_t format, uint32_t n_channels,
+                                          uint64_t n_frames, const uint32_t* channel_stream) {
+  SubmitInterleaved il; il.format = format; il.n_channels = n_channels; il.n_frames = n_frames; il.map = channel_stream; il.on = true;
+  return submit_common(e, nullptr, d_frames, 0, 0, nullptr, nullptr, false, Submit2D(), il);
 }
 
 int same_engine_pending(same_engine* e, size_t* n_events, size_t* n_payload_bytes) {

@@ -48,6 +48,22 @@ extern "C" cudaError_t same_launch_evsort(const same_event* d_events, uint32_t n
 extern "C" cudaError_t same_launch_init(const SameParams* p, const uint32_t* d_ids, uint32_t n, int after_reset,
                                         cudaStream_t stream);
 
+// ---- interleaved ingest: same_ingest.cu ----
+// n_frames frames of `format` (enum same_sample_format), frame_pitch_bytes apart, columns 0..n_cols-1 from `src` on:
+// column c -> row d_row[c] of `dst` (-1: none; rows dpitch samples apart, dpitch a multiple of 8), int16 rows for
+// SAME_FMT_S16, f32 rows otherwise.  One launch.
+extern "C" cudaError_t same_launch_ingest(uint32_t format, const void* src, uint64_t frame_pitch_bytes, uint32_t n_cols,
+                                          uint32_t n_frames, const int32_t* d_row, void* dst, uint64_t dpitch,
+                                          cudaStream_t stream);
+// Bytes per sample of `format`, 0 for an unknown format
+inline uint32_t same_format_bytes(uint32_t format) {
+  return format == SAME_FMT_S16 ? 2u : format == SAME_FMT_S24 ? 3u : format == SAME_FMT_S32 || format == SAME_FMT_F32 ? 4u : 0u;
+}
+// The argument checks of an interleaved submit (same_engine.cu) against n_streams streams: SAME_OK, or
+// SAME_ERR_INVALID_ARG with the reason (naming the channel) in *why
+int same_check_interleaved(const void* frames, uint32_t format, uint32_t n_channels, uint64_t n_frames,
+                           const uint32_t* channel_stream, uint32_t n_streams, std::string* why);
+
 // ---- the long-stream path, same_long.cu: what it owns (scratch for the longest chunk so far, the control words, its
 // counters) and its entry point ----
 struct LongPath {

@@ -33,6 +33,7 @@ struct Shard {
   int rc = 0;
   // scratch reused across submits
   std::vector<uint64_t> off;
+  std::vector<uint32_t> map;   // interleaved submit: this shard's stream of each channel
   size_t pend_ev = 0, pend_pay = 0;
   // stream-state export / import: this shard's share of a call
   std::vector<uint32_t> st_ids, st_pos;
@@ -205,6 +206,24 @@ int same_multi_submit_s16_2d(same_multi* m, const int16_t* samples, uint64_t row
   if (!m || !samples) return mfail(m, SAME_ERR_INVALID_ARG, "null argument");
   return run_all(m, [=](Shard& s) {
     return same_engine_submit_s16_2d(s.eng, samples + (uint64_t)s.first * row_stride, row_stride, col_start, n_cols);
+  });
+}
+
+// Every shard sees the whole frames with a map of its own streams only, so its engine copies and converts just the
+// column range of its own channels.
+int same_multi_submit_interleaved(same_multi* m, const void* frames, uint32_t format, uint32_t n_channels,
+                                  uint64_t n_frames, const uint32_t* channel_stream) {
+  if (!m) return mfail(nullptr, SAME_ERR_INVALID_ARG, "null handle");
+  std::string why;
+  if (same_check_interleaved(frames, format, n_channels, n_frames, channel_stream, m->n_streams, &why))
+    return mfail(m, SAME_ERR_INVALID_ARG, why);
+  return run_all(m, [=](Shard& s) {
+    s.map.resize(n_channels);
+    for (uint32_t c = 0; c < n_channels; ++c) {
+      const uint32_t g = channel_stream ? channel_stream[c] : c;
+      s.map[c] = g != SAME_CHANNEL_SKIP && g >= s.first && g - s.first < s.count ? g - s.first : SAME_CHANNEL_SKIP;
+    }
+    return same_engine_submit_interleaved(s.eng, frames, format, n_channels, n_frames, s.map.data());
   });
 }
 

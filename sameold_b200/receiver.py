@@ -39,6 +39,56 @@ _KIND_NAMES = {
 }
 
 
+# Interleaved PCM (same_engine_submit_interleaved): sample formats and the "drop this channel" stream id
+FMT_S16, FMT_S24, FMT_S32, FMT_F32 = 0, 1, 2, 3
+CHANNEL_SKIP = 0xFFFFFFFF
+_FMT_NAMES = {"s16": FMT_S16, "s24": FMT_S24, "s32": FMT_S32, "f32": FMT_F32}
+_FMT_BYTES = {FMT_S16: 2, FMT_S24: 3, FMT_S32: 4, FMT_F32: 4}
+_FMT_OF_DTYPE = {np.dtype(np.int16): FMT_S16, np.dtype(np.int32): FMT_S32, np.dtype(np.float32): FMT_F32}
+
+
+def _fmt_code(fmt) -> int:
+    if isinstance(fmt, str):
+        if fmt not in _FMT_NAMES:
+            raise ValueError(f"unknown sample format {fmt!r}: one of {sorted(_FMT_NAMES)}")
+        return _FMT_NAMES[fmt]
+    return int(fmt)
+
+
+def _channel_map(channel_streams, n_channels):
+    """None -> None (channel c feeds stream c); else uint32[n_channels], None or a negative id = CHANNEL_SKIP."""
+    if channel_streams is None:
+        return None
+    ids = [CHANNEL_SKIP if c is None or int(c) < 0 else int(c) for c in channel_streams]
+    if len(ids) != n_channels:
+        raise ValueError(f"channel_streams has {len(ids)} entries for {n_channels} channels")
+    return np.array(ids, dtype=np.uint32)
+
+
+def _interleaved(frames, channel_streams, fmt, n_channels):
+    """-> (buffer kept alive during the submit, its address, format code, n_channels, n_frames, map or None).
+    `frames`: a 2-D [n_frames, n_channels] int16 / int32 / float32 array, or a bytes-like of packed frames with `fmt`
+    and `n_channels` (the only way to pass s24)."""
+    if isinstance(frames, np.ndarray) and frames.ndim == 2:
+        if frames.dtype not in _FMT_OF_DTYPE:
+            raise ValueError(f"interleaved frames of dtype {frames.dtype}: int16, int32 or float32 (s24: a bytes-like)")
+        code = _FMT_OF_DTYPE[frames.dtype]
+        if fmt is not None and _fmt_code(fmt) != code:
+            raise ValueError(f"fmt {fmt!r} does not match frames of dtype {frames.dtype}")
+        buf = np.ascontiguousarray(frames)
+        n_frames, n_channels = buf.shape
+    else:
+        if fmt is None or n_channels is None:
+            raise ValueError("a bytes-like of interleaved frames needs fmt and n_channels")
+        code, n_channels = _fmt_code(fmt), int(n_channels)
+        buf = np.frombuffer(frames, dtype=np.uint8) if not isinstance(frames, np.ndarray) else frames.reshape(-1).view(np.uint8)
+        frame_bytes = _FMT_BYTES.get(code, 1) * max(n_channels, 1)
+        if buf.size % frame_bytes:
+            raise ValueError(f"{buf.size} bytes is not a whole number of {frame_bytes}-byte frames")
+        n_frames = buf.size // frame_bytes
+    return buf, (buf.ctypes.data if buf.size else None), code, n_channels, n_frames, _channel_map(channel_streams, n_channels)
+
+
 class SameEngineError(RuntimeError):
     """A non-zero status from the C ABI (resource/engine errors; decode errors are event values, never exceptions)."""
 
@@ -397,6 +447,34 @@ class SameBatchReceiver:
         self._keep = (lengths,)
         self._ck(self._lib.same_engine_submit_zeros(self._h, lengths.ctypes.data))
 
+    def submit_interleaved(self, frames, channel_streams: Optional[Sequence[int]] = None, fmt=None,
+                           n_channels: Optional[int] = None):
+        """Interleaved multi-channel PCM: `frames` is a 2-D [n_frames, n_channels] int16 / int32 / float32 array (s16,
+        s32, f32), or a bytes-like of packed frames with fmt ("s16", "s24", "s32", "f32") and n_channels.  Sample c of
+        frame n becomes sample n of stream channel_streams[c] (None: stream c; None or -1 in the list: channel
+        dropped).  Deinterleaved and converted (`sa as f32` for s24 / s32) on the GPU; s16 channels take the s16 path,
+        the others the f32 path of submit_f32."""
+        buf, ptr, code, nc, nf, cmap = _interleaved(frames, channel_streams, fmt, n_channels)
+        self._keep = (buf, cmap)
+        self._ck(self._lib.same_engine_submit_interleaved(self._h, ptr, code, nc, nf,
+                                                          None if cmap is None else cmap.ctypes.data))
+
+    def process_interleaved(self, frames, channel_streams: Optional[Sequence[int]] = None, fmt=None,
+                            n_channels: Optional[int] = None) -> List[List[SameReceiverEvent]]:
+        """submit_interleaved + sync; returns the events per stream."""
+        self.submit_interleaved(frames, channel_streams, fmt, n_channels)
+        self.sync()
+        return self.drain_by_stream()
+
+    def submit_interleaved_device(self, d_ptr: int, fmt, n_channels: int, n_frames: int,
+                                  channel_streams: Optional[Sequence[int]] = None):
+        """Interleaved frames already in this device's memory (raw device pointer, any alignment), converted on the
+        engine's stream after whatever the caller queued there."""
+        cmap = _channel_map(channel_streams, int(n_channels))
+        self._keep = (cmap,)
+        self._ck(self._lib.same_engine_submit_interleaved_device(self._h, C.c_void_p(d_ptr), _fmt_code(fmt), int(n_channels),
+                                                                 int(n_frames), None if cmap is None else cmap.ctypes.data))
+
     def sync(self):
         self._ck(self._lib.same_engine_sync(self._h))
         self._keep = None
@@ -689,6 +767,15 @@ class SameMultiReceiver:
             raise ValueError(f"expected {self.n_streams} chunks, got {lengths.size}")
         self._keep = (flat, offsets, lengths)
         self._ck(self._lib.same_multi_submit_s16(self._h, flat.ctypes.data, flat.size, offsets.ctypes.data, lengths.ctypes.data))
+
+    def submit_interleaved(self, frames, channel_streams: Optional[Sequence[int]] = None, fmt=None,
+                           n_channels: Optional[int] = None):
+        """SameBatchReceiver.submit_interleaved with GLOBAL stream ids: each device copies and converts only the columns
+        of its own streams."""
+        buf, ptr, code, nc, nf, cmap = _interleaved(frames, channel_streams, fmt, n_channels)
+        self._keep = (buf, cmap)
+        self._ck(self._lib.same_multi_submit_interleaved(self._h, ptr, code, nc, nf,
+                                                         None if cmap is None else cmap.ctypes.data))
 
     def submit_2d(self, host_ptr: int, row_stride: int, col_start: int, n_cols: int):
         self._ck(self._lib.same_multi_submit_s16_2d(self._h, C.c_void_p(host_ptr), int(row_stride), int(col_start), int(n_cols)))
